@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: .et encode + decode throughput (uncompressed GB/s) against the HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A step = one encode (histogram -> host codebook -> pack) followed by one decode (dictionary parse
 -> self-synchronising decode) of the workload, both through the C ABI (include/entreepy_b200.h).
@@ -230,6 +230,10 @@ class OneGpu:
         got = self.codec.decode_dev(self.enc.data_ptr() + 4, self.size - 4, self.dec.data_ptr(), self.n, self.flags, self.stream)
         return got, 0
 
+    def outputs(self, got, offset):
+        """What the callers of et_encode_dev / et_decode_dev received in the last step."""
+        return {"encoded": self.enc[: self.size], "decoded": self.dec[:got]}, [self.size, got]
+
     def e2e_buffers(self):
         c = self.codec
         return c.pinned(self.n), c.pinned(self.n + 16384), c.pinned(self.n)
@@ -282,6 +286,16 @@ class ManyGpus:
         d = self.coder.decode(self.res.header[4:], self.res.body_bytes, self.range, self.dec)
         self.rounds = d.rounds
         return d.n_local, d.offset
+
+    def outputs(self, got, offset):
+        """What this rank's caller received in the last step: the .et header, the body bytes [own_lo, own_hi) it
+        holds, and the text it decoded, which starts at `offset` of the original."""
+        import torch
+
+        res = self.res
+        header = torch.frombuffer(bytearray(res.header), dtype=torch.uint8)
+        body = self.body[res.own_lo - res.first_byte : res.own_hi - res.first_byte]
+        return {"header": header, "encoded": body, "decoded": self.dec[:got]}, [res.own_lo, res.own_hi, offset, got]
 
     def e2e_buffers(self):
         import torch
@@ -413,6 +427,36 @@ def run_other_configs(codec, stream, peak, steps=3):
     return out
 
 
+DUMP_VALUES = 12 << 20  # float32 values --dump-outputs writes, all ranks together (48 MB of the 64 MB it may write)
+DUMP_BLOCK = 1 << 20    # bytes per block sum of an output written as a sample
+
+
+def dump_outputs(path, outputs, sizes, rank, world):
+    """--dump-outputs: the byte arrays the timed path returned in its last step, as .npy files, so that two builds
+    can be compared output for output.  <name>.npy holds the bytes as float32: the whole array when it is short,
+    otherwise the bytes at positions numpy.random.default_rng(0).integers(0, len, k), sorted, plus <name>_block_sums.npy
+    (float64), the sum of every DUMP_BLOCK bytes, so that a change anywhere shows.  sizes.npy (float64) holds the
+    counts the calls returned.  With N > 1 every rank writes its own files, suffixed _rank<r>."""
+    import torch
+
+    os.makedirs(path, exist_ok=True)
+    tag = f"_rank{rank}" if world > 1 else ""
+    k = DUMP_VALUES // (len(outputs) * world)
+    for name, t in outputs.items():
+        n = t.numel()
+        vals = t
+        if n > k:
+            idx = np.sort(np.random.default_rng(0).integers(0, n, k))
+            vals = t[torch.from_numpy(idx).to(t.device)]
+            whole = n // DUMP_BLOCK * DUMP_BLOCK
+            sums = [t[:whole].view(-1, DUMP_BLOCK).sum(dim=1, dtype=torch.int64).cpu()]
+            if whole < n:
+                sums.append(t[whole:].sum(dtype=torch.int64).view(1).cpu())
+            np.save(os.path.join(path, f"{name}_block_sums{tag}.npy"), torch.cat(sums).numpy().astype(np.float64))
+        np.save(os.path.join(path, f"{name}{tag}.npy"), vals.float().cpu().numpy())
+    np.save(os.path.join(path, f"sizes{tag}.npy"), np.array(sizes, dtype=np.float64))
+
+
 def run_ours(args, rank, world):
     import torch
 
@@ -518,9 +562,11 @@ def run_ours(args, rank, world):
         t_end = torch.cuda.Event(enable_timing=True)
         t_begin.record()
         for ev in step_events:
-            step(stats, ev)
+            c_local, got, offset = step(stats, ev)
         t_end.record()
         barrier()
+    if args.dump_outputs:  # before the end-to-end leg, which reuses the N > 1 arm's buffers
+        dump_outputs(args.dump_outputs, *arm.outputs(got, offset), rank, world)
     total_ms = t_begin.elapsed_time(t_end)
     launches = codec.kernel_launches - launches0
     enc_ms = statistics.mean(s[0].elapsed_time(s[1]) for s in stats)
@@ -656,7 +702,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--py-exchange", action="store_true", help="N>1: the exchanges in Python over torch.distributed instead of inside the library")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block (text-5M, adversarial, text-4G)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU path returned; --impl reference times a host sample")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.workload is None:

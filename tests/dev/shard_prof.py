@@ -1,5 +1,6 @@
 import os, sys, time, json
-sys.path.insert(0, os.environ.get("GRAFT_REPO_ROOT", "/root/repo"))
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT)
 import torch, torch.distributed as dist
 import entreepy_b200 as et
 from entreepy_b200 import sharded, synth
@@ -9,7 +10,7 @@ rank, world = dist.get_rank(), dist.get_world_size()
 codec = et.Codec(local)
 n_total = (1 << 32) - 16
 plan = sharded.ShardPlan(n_total, world, rank)
-man = json.load(open(os.path.join(os.environ.get("GRAFT_REPO_ROOT", "/root/repo"), "tests/golden/manifest.json")))
+man = json.load(open(os.path.join(ROOT, "tests/golden/manifest.json")))
 thr = synth.thresholds_from_weights(synth.text_weights(man["midsummer_histogram"]))
 inp = torch.empty(plan.n_local + 16, dtype=torch.uint8, device="cuda")
 stream = torch.cuda.current_stream().cuda_stream

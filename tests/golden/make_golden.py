@@ -1,12 +1,12 @@
-"""Regenerates tests/golden/ from the reference's own fixtures (run in the build container only).
+"""Regenerates tests/golden/ from the reference's own fixtures.
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <typio/entreepy checkout>/res
 
-Inputs : /root/reference/res/*.txt  (the files test.zig:35-72 round-trips; public-domain text).
+Inputs : res/*.txt of typio/entreepy (the files test.zig:35-72 round-trips; public-domain text).
 Outputs: <name>            the input bytes (test DATA, not reference source code)
          <name>.et         .et file produced by the CPU oracle (oracle/entreepy_oracle.c)
          manifest.json     sizes, sha256s, header lengths, code-length summary, Midsummer histogram
-The GPU box has no /root/reference, so the inputs travel with the repo.
+The tests need no copy of the reference: the inputs are committed here.
 """
 import hashlib
 import json
@@ -18,7 +18,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import oracle  # noqa: E402
 
-RES = "/root/reference/res"
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+RES = sys.argv[1]
 NAMES = ["test.txt", "nice.shakespeare.txt", "a_midsummer_nights_dream.txt"]
 
 # SURVEY.md §8c — derived by an independent restatement during the survey.
