@@ -17,6 +17,21 @@
 
 using namespace et;
 
+constexpr size_t kMaxHeaderBytes = 4096;
+
+// The small fixed block of a context; the device copy and its pinned host mirror share this layout.
+struct SmallBlock {
+    alignas(128) unsigned long long counts[256];
+    alignas(128) uint8_t pack_tables[2048 + 256];      // narrow: 256 x {code, len} u32 | wide: 256 x u64 codes, 256 x u8 lengths
+    alignas(128) uint32_t lut[2 * kLutSize];            // clut | wlut
+    alignas(128) uint32_t nodes[kMaxTrieNodes];         // the dictionary's trie
+    alignas(128) uint16_t slots[kLutSize + (kMaxSubTables << kSubBits)];  // slot of a marker window | second-level tables
+    alignas(128) uint32_t thresholds[256];              // et_synth_dev
+    alignas(128) DecodeStatus status;                   // host copy: what the last decode read back
+    alignas(128) uint32_t table_work[32];               // slot counter + slot windows of launch_build_tables
+    alignas(128) uint8_t header[kMaxHeaderBytes];       // header staging
+};
+
 struct ncclUniqueIdBytes {  // layout of ncclUniqueId (nccl.h): passed by value to ncclCommInitRank
     char b[ET_COMM_ID_BYTES];
 };
@@ -31,8 +46,8 @@ struct et_ctx {
     // device scratch, grown on demand
     void *d_scratch = nullptr;
     size_t scratch_cap = 0;
-    uint8_t *d_small = nullptr;  // fixed block: counts, tables, LUT, trie, thresholds
-    uint8_t *h_small = nullptr;  // pinned mirror of d_small + header staging
+    SmallBlock *d_small = nullptr;  // fixed block: counts, tables, LUT, trie, thresholds
+    SmallBlock *h_small = nullptr;  // pinned mirror of d_small: staging of the header, counts and decode status
     // bulk staging for the host-buffer entry points
     uint8_t *d_in = nullptr, *d_out = nullptr;
     size_t d_in_cap = 0, d_out_cap = 0;
@@ -47,19 +62,6 @@ struct et_ctx {
 };
 
 namespace {
-
-// layout of the small fixed block (device and pinned host copies share it)
-constexpr size_t kOffCounts = 0;                                    // 256 x u64
-constexpr size_t kOffPackTables = 2048;                             // narrow 2 KiB | wide 2304 B
-constexpr size_t kOffLut = 8192;                                    // clut | wlut: 2 x 4096 x u32
-constexpr size_t kOffNodes = kOffLut + 2 * kLutSize * 4;            // kMaxTrieNodes x u32
-constexpr size_t kOffSlots = kOffNodes + kMaxTrieNodes * 4;         // kLutSize x u16 slot of a marker window | sub-tables
-constexpr size_t kOffThresholds = kOffSlots + kLutSize * 2 + (kMaxSubTables << kSubBits) * 2;  // 256 x u32
-constexpr size_t kOffFlags = kOffThresholds + 1024;                 // error flags + total (16 B)
-constexpr size_t kOffTableWork = kOffFlags + 64;                    // slot counter + slot windows of launch_build_tables (128 B)
-constexpr size_t kOffHeader = kOffTableWork + 128;                  // 4 KiB header staging
-constexpr size_t kSmallBytes = kOffHeader + 4096;
-constexpr size_t kMaxHeaderBytes = 4096;
 
 int fail(et_ctx *ctx, int status, const char *fmt, ...) {
     if (ctx) {
@@ -155,13 +157,13 @@ struct StageTimer {
 
 // Histogram of a device buffer into host counts (blocks until the counts are on the host).
 int histogram_dev(et_ctx *ctx, const void *d_in, size_t n, uint64_t counts[256], cudaStream_t s) {
-    unsigned long long *d_counts = reinterpret_cast<unsigned long long *>(ctx->d_small + kOffCounts);
+    unsigned long long *d_counts = ctx->d_small->counts;
     ET_CUDA(ctx, cudaMemsetAsync(d_counts, 0, 2048, s));
     ET_CUDA(ctx, launch_histogram(static_cast<const uint8_t *>(d_in), n, d_counts, ctx->num_sms, s));
     if (n) ctx->launches += 1;
-    ET_CUDA(ctx, cudaMemcpyAsync(ctx->h_small + kOffCounts, d_counts, 2048, cudaMemcpyDeviceToHost, s));
+    ET_CUDA(ctx, cudaMemcpyAsync(ctx->h_small->counts, d_counts, sizeof ctx->h_small->counts, cudaMemcpyDeviceToHost, s));
     ET_CUDA(ctx, cudaStreamSynchronize(s));
-    std::memcpy(counts, ctx->h_small + kOffCounts, 2048);
+    std::memcpy(counts, ctx->h_small->counts, sizeof ctx->h_small->counts);
     return ET_OK;
 }
 
@@ -170,7 +172,7 @@ int upload_pack_tables(et_ctx *ctx, const et_codebook &cb, bool *wide, cudaStrea
     PackTables t;
     const int rc = make_pack_tables(cb, &t);
     if (rc != ET_OK) return fail(ctx, rc, "code length %u cannot be emitted", cb.max_length);
-    uint8_t *h = ctx->h_small + kOffPackTables;
+    uint8_t *h = ctx->h_small->pack_tables;
     size_t bytes;
     if (t.narrow_ok) {
         std::memcpy(h, t.narrow, 2048);
@@ -181,7 +183,7 @@ int upload_pack_tables(et_ctx *ctx, const et_codebook &cb, bool *wide, cudaStrea
         bytes = 2304;
     }
     *wide = !t.narrow_ok;
-    ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small + kOffPackTables, h, bytes, cudaMemcpyHostToDevice, s));
+    ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small->pack_tables, h, bytes, cudaMemcpyHostToDevice, s));
     return ET_OK;
 }
 
@@ -191,13 +193,11 @@ int pack_dev(et_ctx *ctx, const void *d_in, size_t n, const et_codebook &cb, uin
     int rc = upload_pack_tables(ctx, cb, &wide, s);
     if (rc != ET_OK) return rc;
     const PackGeometry g = pack_geometry(d_in, n);
-    const size_t sb = pack_scratch_bytes(g.num_tiles);
-    rc = ensure_scratch(ctx, sb);
+    rc = ensure_scratch(ctx, pack_scratch_bytes(g));
     if (rc != ET_OK) return rc;
-    const PackScratch ps = pack_scratch_carve(ctx->d_scratch, g.num_tiles);
     int launches = 0;
-    ET_CUDA(ctx, launch_pack(g, ctx->d_small + kOffPackTables, wide, cb.max_length, d_body, bit_phase, ps, ctx->d_scratch, sb,
-                             ctx->num_sms, s, &launches, ctx->tune.pack_single_pass != 0, ctx->tune.pack_bits_ctas));
+    ET_CUDA(ctx, launch_pack(g, ctx->d_small->pack_tables, wide, cb.max_length, d_body, bit_phase, ctx->d_scratch, ctx->num_sms, s,
+                             &launches, ctx->tune.pack_single_pass != 0, ctx->tune.pack_bits_ctas));
     ctx->launches += (uint64_t)launches;
     return ET_OK;
 }
@@ -263,8 +263,8 @@ extern "C" int et_ctx_create(int device, et_ctx **out) {
     ok = ok && cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking) == cudaSuccess;
     ok = ok && cudaStreamCreateWithFlags(&ctx->copy_stream2, cudaStreamNonBlocking) == cudaSuccess;
     for (auto &e : ctx->ev) ok = ok && cudaEventCreate(&e) == cudaSuccess;
-    ok = ok && cudaMalloc(reinterpret_cast<void **>(&ctx->d_small), kSmallBytes) == cudaSuccess;
-    ok = ok && cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_small), kSmallBytes, cudaHostAllocDefault) == cudaSuccess;
+    ok = ok && cudaMalloc(reinterpret_cast<void **>(&ctx->d_small), sizeof(SmallBlock)) == cudaSuccess;
+    ok = ok && cudaHostAlloc(reinterpret_cast<void **>(&ctx->h_small), sizeof(SmallBlock), cudaHostAllocDefault) == cudaSuccess;
     ok = ok && unpack_init_device(device, &ctx->tune) == cudaSuccess;
     ok = ok && pack_init_device(ctx->tune.max_smem, &ctx->tune.pack_bits_ctas) == cudaSuccess;
     ctx->trie = new (std::nothrow) UnpackTrie;
@@ -386,7 +386,7 @@ extern "C" int et_encode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_ou
     if (rc != ET_OK) return rc;
     if (flags & ET_FLAG_DEBUG) print_dictionary(ctx->out_fd, plan.cb);
     if (write_out) {
-        uint8_t *h_header = ctx->h_small + kOffHeader;
+        uint8_t *h_header = ctx->h_small->header;
         size_t hl = 0;
         rc = et_write_header(&plan.cb, n, h_header, kMaxHeaderBytes, &hl);  // E5
         if (rc != ET_OK) return fail(ctx, rc, "header");
@@ -424,7 +424,7 @@ extern "C" int et_encode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
 
     // E1 overlapped with the upload: the input goes up in slices on copy_stream; the
     // histogram of slice k runs on `s` while slice k+1 is still in flight.
-    unsigned long long *d_counts = reinterpret_cast<unsigned long long *>(ctx->d_small + kOffCounts);
+    unsigned long long *d_counts = ctx->d_small->counts;
     ET_CUDA(ctx, cudaMemsetAsync(d_counts, 0, 2048, s));
     const size_t slice = (size_t)64 << 20;
     for (size_t off = 0; off < n; off += slice) {
@@ -435,10 +435,10 @@ extern "C" int et_encode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
         ET_CUDA(ctx, launch_histogram(ctx->d_in + off, len, d_counts, ctx->num_sms, s));
         ctx->launches += 1;
     }
-    ET_CUDA(ctx, cudaMemcpyAsync(ctx->h_small + kOffCounts, d_counts, 2048, cudaMemcpyDeviceToHost, s));
+    ET_CUDA(ctx, cudaMemcpyAsync(ctx->h_small->counts, d_counts, sizeof ctx->h_small->counts, cudaMemcpyDeviceToHost, s));
     ET_CUDA(ctx, cudaStreamSynchronize(s));
     uint64_t counts[256];
-    std::memcpy(counts, ctx->h_small + kOffCounts, 2048);
+    std::memcpy(counts, ctx->h_small->counts, sizeof ctx->h_small->counts);
 
     EncodePlan plan;
     rc = plan_encode(ctx, counts, n, cap, flags, &plan);
@@ -505,50 +505,38 @@ int upload_unpack_tables(et_ctx *ctx, const et_dictionary &dict, cudaStream_t s,
                                                      : "dictionary is not a prefix code");
     }
     ctx->fixed_len = (t->complete && t->prefix_free && dict.min_length == dict.max_length) ? dict.max_length : 0u;
-    std::memcpy(ctx->h_small + kOffNodes, t->nodes, (size_t)t->n_nodes * 4);
-    ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small + kOffNodes, ctx->h_small + kOffNodes, (size_t)t->n_nodes * 4, cudaMemcpyHostToDevice, s));
+    std::memcpy(ctx->h_small->nodes, t->nodes, (size_t)t->n_nodes * 4);
+    ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small->nodes, ctx->h_small->nodes, (size_t)t->n_nodes * 4, cudaMemcpyHostToDevice, s));
     int launches = 0;
-    ET_CUDA(ctx, launch_build_tables(reinterpret_cast<const uint32_t *>(ctx->d_small + kOffNodes), reinterpret_cast<uint32_t *>(ctx->d_small + kOffLut),
-                                     reinterpret_cast<uint16_t *>(ctx->d_small + kOffSlots), reinterpret_cast<uint32_t *>(ctx->d_small + kOffTableWork), s,
-                                     &launches));
+    ET_CUDA(ctx, launch_build_tables(ctx->d_small->nodes, ctx->d_small->lut, ctx->d_small->slots, ctx->d_small->table_work, s, &launches));
     ctx->launches += (uint64_t)launches;
     return ET_OK;
 }
 
-// Decode the part of a device-resident body that `g` describes.  *n_symbols = symbols found, capped at
-// max_symbols.  tables_ready: upload_unpack_tables() was already called for this dictionary (the
-// pipelined host path does it before it queues the bulk uploads, which would otherwise delay it).
+// Decode the part of a device-resident body that `g` describes: min(symbols found, max_symbols) bytes to d_out.
+// *st = the status words it ended with (symbols found, entry, exit).  tables_ready: upload_unpack_tables() was
+// already called for this dictionary (the pipelined host path does it before it queues the bulk uploads, which
+// would otherwise delay it).
 int unpack_dev(et_ctx *ctx, const UnpackGeometry &g, const et_dictionary &dict, uint8_t *d_out, uint64_t max_symbols,
-               uint64_t *n_symbols, cudaStream_t s, StageTimer *tm = nullptr, uint32_t *entry_exit = nullptr,
-               bool tables_ready = false, bool validate = false, uint64_t *found = nullptr) {
+               cudaStream_t s, DecodeStatus *st, StageTimer *tm = nullptr, bool tables_ready = false, bool validate = false) {
     int rc = tables_ready ? ET_OK : upload_unpack_tables(ctx, dict, s, validate);
     if (rc != ET_OK) return rc;
     if (tm) tm->mark(2);
 
     const uint32_t chunk_bytes = unpack_chunk_bytes(g, ctx->tune, dict.min_length, dict.max_length);
-    rc = ensure_scratch(ctx, unpack_scratch_bytes(g, chunk_bytes));
+    const uint32_t transfer_states = (dict.max_length - dict.min_length <= 2 && dict.max_length <= 16) ? dict.max_length : 0u;
+    rc = ensure_scratch(ctx, unpack_scratch_bytes(g, chunk_bytes, transfer_states));
     if (rc != ET_OK) return rc;
-    const uint32_t *d_clut = reinterpret_cast<const uint32_t *>(ctx->d_small + kOffLut);
+    const uint32_t *d_clut = ctx->d_small->lut;
     const uint32_t *d_wlut = d_clut + kLutSize;
-    const uint32_t *d_nodes = reinterpret_cast<const uint32_t *>(ctx->d_small + kOffNodes);
     int launches = 0;
     uint32_t rounds = 0;
-    const uint16_t *d_slots = reinterpret_cast<const uint16_t *>(ctx->d_small + kOffSlots);
-    ET_CUDA(ctx, launch_unpack(g, chunk_bytes, d_clut, d_wlut, d_nodes, d_slots, d_out, max_symbols, ctx->d_scratch,
-                               ctx->h_small + kOffFlags, s, ctx->tune, ctx->fixed_len,
-                               (dict.max_length - dict.min_length <= 2 && dict.max_length <= 16) ? dict.max_length : 0u, &launches, &rounds));
+    ET_CUDA(ctx, launch_unpack(g, chunk_bytes, d_clut, d_wlut, ctx->d_small->nodes, ctx->d_small->slots, d_out, max_symbols,
+                               ctx->d_scratch, &ctx->h_small->status, s, ctx->tune, ctx->fixed_len, transfer_states, &launches, &rounds));
     ctx->launches += (uint64_t)launches;
     ctx->last_decode_rounds = rounds;
-    // launch_unpack left the stream idle and a copy of the scratch header in the pinned block:
-    // pad(4) | error flags(4) | symbols found(8) | changed(4) | largest region(4) | entry, exit (4+4)
-    uint32_t flags = 0;
-    unsigned long long total = 0;
-    std::memcpy(&flags, ctx->h_small + kOffFlags + 4, 4);
-    std::memcpy(&total, ctx->h_small + kOffFlags + 8, 8);
-    if (entry_exit) std::memcpy(entry_exit, ctx->h_small + kOffFlags + 24, 8);
-    if (flags & kErrInvalidCode) return fail(ctx, ET_ERR_CORRUPT, "body contains a bit pattern that is not a code");
-    *n_symbols = std::min<uint64_t>(total, max_symbols);
-    if (found) *found = total;
+    *st = ctx->h_small->status;  // launch_unpack left the stream idle
+    if (st->error_flags & kErrInvalidCode) return fail(ctx, ET_ERR_CORRUPT, "body contains a bit pattern that is not a code");
     return ET_OK;
 }
 
@@ -583,7 +571,7 @@ extern "C" int et_decode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_ou
     tm.mark(0);
     // D1+D2: the dictionary is parsed on the host from the first bytes of the stream
     const size_t head = std::min(n, kMaxHeaderBytes);
-    uint8_t *h_header = ctx->h_small + kOffHeader;
+    uint8_t *h_header = ctx->h_small->header;
     ET_CUDA(ctx, cudaMemcpyAsync(h_header, d_in, head, cudaMemcpyDeviceToHost, s));
     ET_CUDA(ctx, cudaStreamSynchronize(s));
     et_dictionary dict;
@@ -594,11 +582,12 @@ extern "C" int et_decode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_ou
     tm.mark(1);
     if (!(flags & ET_FLAG_WRITE_OUTPUT) || empty) return ET_OK;  // dry run: bytes_written stays 0 (decode.zig:185-188)
     if (!d_out && cap) return ET_ERR_INVALID_ARG;
-    uint64_t produced = 0;
     const uint64_t want = std::min<uint64_t>(dict.body_len, cap);
+    DecodeStatus st;
     rc = unpack_dev(ctx, unpack_geometry(static_cast<const uint8_t *>(d_in) + dict.body_offset, n - dict.body_offset), dict,
-                    static_cast<uint8_t *>(d_out), want, &produced, s, &tm, nullptr, false, (flags & ET_FLAG_VALIDATE) != 0);  // D3
+                    static_cast<uint8_t *>(d_out), want, s, &st, &tm, false, (flags & ET_FLAG_VALIDATE) != 0);  // D3
     if (rc != ET_OK) return rc;
+    const uint64_t produced = std::min<uint64_t>(st.total, want);
     tm.mark(3);
     ET_CUDA(ctx, cudaEventSynchronize(ctx->ev[3]));
     tm.finish(4);
@@ -643,8 +632,10 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
         if (n_slices == 1) {
             if (body_bytes)
                 ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_in, in + dict.body_offset, body_bytes, cudaMemcpyHostToDevice, s));
-            rc = unpack_dev(ctx, unpack_geometry(ctx->d_in, body_bytes), dict, ctx->d_out, want, &produced, s, nullptr, nullptr, false, validate);
+            DecodeStatus st;
+            rc = unpack_dev(ctx, unpack_geometry(ctx->d_in, body_bytes), dict, ctx->d_out, want, s, &st, nullptr, false, validate);
             if (rc != ET_OK) return rc;
+            produced = std::min<uint64_t>(st.total, want);
             if (write_out) {
                 if (produced == cap && dict.body_len > cap)
                     return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %u symbols, capacity %zu", dict.body_len, cap);
@@ -677,16 +668,16 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
                 const size_t own_lo = k ? k * kSlice - 64 : 0, own_hi = last ? body_bytes : (k + 1) * kSlice - 64;
                 const size_t avail = std::min(body_bytes, (k + 1) * kSlice);
                 cudaStreamWaitEvent(s, up[k], 0);
-                uint32_t ee[2] = {0, 0};
-                uint64_t got = 0;
+                DecodeStatus st;
                 rc = unpack_dev(ctx, unpack_geometry_shard(ctx->d_in, avail, own_lo, own_hi, (long long)head_bit), dict,
-                                ctx->d_out + produced, want - produced, &got, s, nullptr, ee, true);
+                                ctx->d_out + produced, want - produced, s, &st, nullptr, true);
                 if (rc != ET_OK) {
                     cudaStreamSynchronize(ctx->copy_stream);
                     cleanup();
                     return rc;
                 }
-                head_bit = (uint64_t)own_hi * 8 + ee[1];
+                head_bit = (uint64_t)own_hi * 8 + st.exit;
+                const uint64_t got = std::min<uint64_t>(st.total, want - produced);
                 if (write_out && got)  // unpack_dev returned after its kernels finished: the text is ready to go down
                     cudaMemcpyAsync(out + produced, ctx->d_out + produced, got, cudaMemcpyDeviceToHost, ctx->copy_stream2);
                 produced += got;
@@ -739,18 +730,18 @@ extern "C" int et_unpack_shard_dev(et_ctx *ctx, const void *d_range, size_t rang
     tm.mark(0);
     tm.mark(1);
     const UnpackGeometry g = unpack_geometry_shard(d_range, range_bytes, own_begin_byte, own_end_byte, (long long)head_bit);
-    uint64_t produced = 0, found = 0;
-    uint32_t ee[2] = {0, 0};
-    const int rc = unpack_dev(ctx, g, *dict, static_cast<uint8_t *>(d_out), cap, &produced, s, &tm, ee, false, false, &found);
+    DecodeStatus st;
+    const int rc = unpack_dev(ctx, g, *dict, static_cast<uint8_t *>(d_out), cap, s, &st, &tm);
     if (rc != ET_OK) return rc;
+    const uint64_t found = st.total;
     tm.mark(3);
     ET_CUDA(ctx, cudaEventSynchronize(ctx->ev[3]));
     tm.finish(4);
     *n_symbols = found;  // the caller's text offsets are sums of these: never a clipped count
     if (found > cap) return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: the shard holds %llu symbols, capacity %zu", (unsigned long long)found, cap);
     // entry: bits past the first bit of the 32-byte sector grid the chunks are cut on (= own_begin: it is 32-byte aligned)
-    if (entry_bit) *entry_bit = (uint64_t)own_begin_byte * 8 + ee[0];
-    if (exit_bit) *exit_bit = (uint64_t)own_end_byte * 8 + ee[1];
+    if (entry_bit) *entry_bit = (uint64_t)own_begin_byte * 8 + st.entry;
+    if (exit_bit) *exit_bit = (uint64_t)own_end_byte * 8 + st.exit;
     return ET_OK;
 }
 
@@ -760,10 +751,10 @@ extern "C" int et_synth_dev(et_ctx *ctx, void *d_out, size_t n, uint64_t seed, u
     if (!ctx || (!d_out && n) || !thresholds) return ET_ERR_INVALID_ARG;
     ET_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = stream ? static_cast<cudaStream_t>(stream) : ctx->stream;
-    std::memcpy(ctx->h_small + kOffThresholds, thresholds, 1024);
-    ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small + kOffThresholds, ctx->h_small + kOffThresholds, 1024, cudaMemcpyHostToDevice, s));
+    std::memcpy(ctx->h_small->thresholds, thresholds, sizeof ctx->h_small->thresholds);
+    ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small->thresholds, ctx->h_small->thresholds, sizeof ctx->h_small->thresholds, cudaMemcpyHostToDevice, s));
     ET_CUDA(ctx, launch_synth(static_cast<uint8_t *>(d_out), n, seed, first_index,
-                              reinterpret_cast<const uint32_t *>(ctx->d_small + kOffThresholds), s));
+                              ctx->d_small->thresholds, s));
     ET_CUDA(ctx, cudaStreamSynchronize(s));
     return ET_OK;
 }

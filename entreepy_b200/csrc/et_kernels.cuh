@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include "et_internal.h"
+#include "et_scratch.h"
 
 namespace et {
 
@@ -25,25 +26,14 @@ struct PackGeometry {
 };
 PackGeometry pack_geometry(const void *d_in, size_t n);
 
-// Device scratch the pack kernels need for `num_tiles` tiles (4096 symbols each).  The wide kernel (codes of
-// 33..64 bits) works on those tiles; the lane-run path (codes <= 32 bits) carves the same block for its regions
-// of 2048 symbols (two per tile) and its u16 run totals: pack_scratch_bytes() covers both.
-struct PackScratch {
-    unsigned long long *tile_state;   // [num_tiles] last bit + 1 of each tile (wide kernel: look-back descriptors)
-    unsigned long long *group_prefix; // [ceil(num_tiles / 256)] bits before each group of tiles
-    uint32_t *tile_bits;              // [num_tiles]
-    uint8_t *seam_head;               // [num_tiles]
-    uint8_t *seam_tail;               // [num_tiles]
-    uint32_t *ticket;                 // [1] (wide kernel)
-};
-size_t pack_scratch_bytes(uint32_t num_tiles);
-PackScratch pack_scratch_carve(void *base, uint32_t num_tiles);
+// Device scratch the pack kernels need (pack_layout(), et_scratch.h).
+size_t pack_scratch_bytes(const PackGeometry &g);
 
 // d_tables: narrow -> 256 x {code, len} (u32 pairs); wide -> 256 x u64 codes followed by 256 x u8 lengths.
 // max_len: longest code (sizes the bit image of a warp on the narrow path).
 // bits_ctas_per_sm: from pack_init_device() (0: ask the runtime at every call).
 cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, uint32_t max_len, uint8_t *d_out, uint32_t bit_phase,
-                        const PackScratch &s, void *scratch_base, size_t scratch_bytes, int num_sms,
+                        void *scratch_base, int num_sms,
                         cudaStream_t stream, int *launches, bool single_pass = false, int bits_ctas_per_sm = 0);
 // Once per context: lets the pack kernels use all of an SM's shared memory and reads how many CTAs of pass A fit an SM
 // (both used to be asked of the runtime at every call, a few microseconds each with the GPU waiting).
@@ -51,7 +41,6 @@ cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm);
 
 // ---------------------------------------------------------------- K3-K5 (chunked self-synchronising decoder)
 constexpr int kSubseqBits = 128;    // a piece: the unit the stream is read in (one 16-byte load)
-constexpr int kChunkThreads = 256;  // chunks per CTA
 
 // Where the stream sits relative to the 16-byte grid the pieces are cut on.  All bit
 // positions are relative to body_aligned.
@@ -90,13 +79,12 @@ struct UnpackTuning {
 cudaError_t unpack_init_device(int device, UnpackTuning *tune);
 void unpack_free_device(UnpackTuning *tune);
 
-// Chunk size for this stream (bytes per thread) and the device scratch the decoder needs.
+// Chunk size for this stream (bytes per thread) and the device scratch the decoder needs (decode_layout(), et_scratch.h).
 uint32_t unpack_chunk_bytes(const UnpackGeometry &g, const UnpackTuning &tune, uint32_t min_length, uint32_t max_length);
-size_t unpack_scratch_bytes(const UnpackGeometry &g, uint32_t chunk_bytes);
-// Scratch header after the call: [4] error flags (u32), [8] symbols found (u64), [24] entry used
-// by the first chunk, [28] exit of the last chunk (u32 bits).  Writes min(total, max_symbols)
-// bytes to d_out.  Blocks on the stream between check rounds; on return the stream is idle and
-// h_hdr (pinned host memory, 64 bytes) holds a copy of the first 32 bytes of the scratch header.
+size_t unpack_scratch_bytes(const UnpackGeometry &g, uint32_t chunk_bytes, uint32_t transfer_states);
+// Writes min(total, max_symbols) bytes to d_out.  Blocks on the stream between check rounds; on return the
+// stream is idle and h_status (pinned host memory) holds the status words the decode ended with (DecodeStatus:
+// error flags, symbols found, entry used by the first chunk, exit of the last chunk).
 // d_slots: slot of every marker window (kLutSize x u16) followed by the second-level tables (launch_build_tables).
 // *rounds_out = passes over the chunk entries it took (2 = the guesses plus one repair round sufficed).
 // fixed_len: the dictionary is a complete code whose codes all have this many bits (0: it is not) — such a
@@ -106,7 +94,7 @@ size_t unpack_scratch_bytes(const UnpackGeometry &g, uint32_t chunk_bytes);
 // transfer function and scans instead of running repair rounds.
 cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const uint32_t *d_clut, const uint32_t *d_wlut,
                           const uint32_t *d_nodes, const uint16_t *d_slots, uint8_t *d_out, uint64_t max_symbols, void *scratch_base,
-                          uint8_t *h_hdr, cudaStream_t stream, const UnpackTuning &tune, uint32_t fixed_len, uint32_t transfer_states,
+                          DecodeStatus *h_status, cudaStream_t stream, const UnpackTuning &tune, uint32_t fixed_len, uint32_t transfer_states,
                           int *launches, uint32_t *rounds_out);
 
 // The decoder's first-level tables (et_internal.h) from the uploaded trie, on the device.

@@ -883,25 +883,7 @@ PackGeometry pack_geometry(const void *d_in, size_t n) {
     return g;
 }
 
-// The lane-run path cuts the input into regions of 2048 symbols (two per tile) and keeps a u16 per run of 64.
-size_t pack_scratch_bytes(uint32_t num_tiles) {
-    // [ticket + pad : 16][tile_state : 8*T][group_prefix : 8*G][tile_bits : 4*T][seam_head : T][seam_tail : T][run_bits : 64*T]
-    const size_t t = (size_t)num_tiles * 2 + 2;
-    const size_t groups = (t + 7) / 8;
-    return 16 + t * 14 + groups * 8 + 16 + t * 64 + 64;
-}
-PackScratch pack_scratch_carve(void *base, uint32_t num_tiles) {
-    PackScratch s;
-    const size_t groups = ((size_t)num_tiles + 7) / 8;
-    uint8_t *p = static_cast<uint8_t *>(base);
-    s.ticket = reinterpret_cast<uint32_t *>(p);
-    s.tile_state = reinterpret_cast<unsigned long long *>(p + 16);
-    s.group_prefix = s.tile_state + num_tiles;
-    s.tile_bits = reinterpret_cast<uint32_t *>(s.group_prefix + groups);
-    s.seam_head = reinterpret_cast<uint8_t *>(s.tile_bits + num_tiles);
-    s.seam_tail = s.seam_head + num_tiles;
-    return s;
-}
+size_t pack_scratch_bytes(const PackGeometry &g) { return pack_layout(nullptr, g.num_tiles).bytes; }
 
 cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm) {
     cudaError_t err = cudaFuncSetAttribute(pack_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
@@ -914,9 +896,10 @@ cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm) {
 }
 
 cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, uint32_t max_len, uint8_t *d_out, uint32_t bit_phase,
-                        const PackScratch &s, void *scratch_base, size_t scratch_bytes, int num_sms,
-                        cudaStream_t stream, int *launches, bool single_pass, int bits_ctas_per_sm) {
+                        void *scratch_base, int num_sms, cudaStream_t stream, int *launches, bool single_pass,
+                        int bits_ctas_per_sm) {
     if (g.num_tiles == 0) return cudaSuccess;
+    const PackLayout s = pack_layout(scratch_base, g.num_tiles);
     cudaError_t err = cudaSuccess;
     PackArgs a;
     a.in_aligned = g.in_aligned;
@@ -930,7 +913,7 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
     a.seam_head = s.seam_head;
     a.seam_tail = s.seam_tail;
     a.ticket = s.ticket;
-    a.tile_desc = nullptr;
+    a.tile_desc = s.tile_desc;
     a.tile_bits = s.tile_bits;
     a.group_prefix = s.group_prefix;
     a.group_tiles = 1;
@@ -941,7 +924,7 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
 
     if (wide) {
         // look-back descriptors and the ticket start from zero
-        err = cudaMemsetAsync(scratch_base, 0, 16 + (size_t)g.num_tiles * 8, stream);
+        err = cudaMemsetAsync(s.ticket, 0, reinterpret_cast<uint8_t *>(s.tile_state + g.num_tiles) - reinterpret_cast<uint8_t *>(s.ticket), stream);
         if (err != cudaSuccess) return err;
         const int smem = StageWords<true>::value * 4 + PackCfg<true>::kTableBytes;
         err = cudaFuncSetAttribute(pack_wide_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
@@ -954,18 +937,9 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
         pack_wide_kernel<true><<<grid, kPackThreads, smem, stream>>>(a);
         if (launches) *launches += 1;
     } else {
-        (void)scratch_bytes;
-        // lane-run path: regions of 2048 symbols, carved from the same scratch block
+        // lane-run path: regions of 2048 symbols, in the slots of the same layout
         const uint32_t n_regions = (uint32_t)((g.v_end + kRegionSyms - 1) / kRegionSyms);
-        const uint32_t r_alloc = 2 * g.num_tiles + 2;  // regions the slabs of pass A may touch
-        const PackScratch rs = pack_scratch_carve(scratch_base, r_alloc);
-        a.tile_state = rs.tile_state;
-        a.seam_head = rs.seam_head;
-        a.seam_tail = rs.seam_tail;
-        a.tile_bits = rs.tile_bits;
-        a.group_prefix = rs.group_prefix;
-        a.run_bits = reinterpret_cast<uint16_t *>(
-            (reinterpret_cast<uintptr_t>(rs.seam_tail + r_alloc) + 15) & ~(uintptr_t)15);
+        a.run_bits = s.run_bits;
         a.n_regions = n_regions;
         a.num_tiles = n_regions;
         a.interior_lo = g.misalign ? 1u : 0u;
@@ -974,7 +948,7 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
         a.image_words = (uint32_t)(kStageGuard + (kRegionSyms * max_len + 31) / 32 + 16 + 3) & ~3u;
         if (a.image_words < kStageGuard + kRegionSyms / 4) a.image_words = kStageGuard + kRegionSyms / 4;  // the image also stages the region's text
         if (single_pass) {
-            // single pass: tiles of `warps` regions, look-back descriptors where the two-pass path keeps its run totals
+            // single pass: tiles of `warps` regions, each with a look-back descriptor
             const uint32_t priv_stride = (2u * max_len + 1u) | 1u;  // words of a lane's private string (64 codes), odd: lanes never share a bank at equal depth
             const uint32_t warp_bytes = (32u * priv_stride + a.image_words) * 4u + 32u;
             int max_smem = 0, dev = 0;
@@ -985,14 +959,12 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
             if (warps > 4) warps &= ~3u;
             if (warps >= 1) {
                 const uint32_t n_tiles = (n_regions + warps - 1) / warps;
-                a.tile_desc = reinterpret_cast<unsigned long long *>(a.run_bits);  // [n_tiles] <= 8 B per region: inside the run-total area (64 B per region)
-                if ((err = cudaMemsetAsync(rs.ticket, 0, 16, stream)) != cudaSuccess) return err;
+                if ((err = cudaMemsetAsync(s.ticket, 0, 16, stream)) != cudaSuccess) return err;
                 if ((err = cudaMemsetAsync(a.tile_desc, 0, (size_t)n_tiles * 8, stream)) != cudaSuccess) return err;
                 const int smem = kTableBytes + (int)(warps * warp_bytes);
                 if ((err = cudaFuncSetAttribute(pack_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return err;
                 unsigned grid = (unsigned)num_sms * (2u * (unsigned)smem + 2048u <= (unsigned)max_smem ? 2u : 1u);
                 if (grid > n_tiles) grid = n_tiles;
-                a.ticket = rs.ticket;
                 pack_tiles_kernel<<<grid, warps * 32, smem, stream>>>(a, warps, priv_stride, n_tiles);
                 if (launches) *launches += 1;
                 if ((err = cudaGetLastError()) != cudaSuccess) return err;

@@ -39,19 +39,6 @@ namespace et {
 
 namespace {
 
-// Parts of a chunk that the lane write walk decodes side by side (et_lanes.inc).  MEASURED (r2, text-1G, all else equal):
-// two parts 0.996 ms per decode, four parts 1.012 ms - the write walk gains (wait stalls down, issue slots 59 -> 68 %) what
-// the count walk loses to recording three boundaries per chunk instead of one (four reconvergence points per chunk).
-#ifndef ET_WRITE_CHAINS
-#define ET_WRITE_CHAINS 2
-#endif
-// What the count walk records for the write walk per chunk: 18 bits per boundary.
-#if ET_WRITE_CHAINS == 2
-typedef uint32_t mid_t;
-#else
-typedef uint64_t mid_t;
-#endif
-
 constexpr uint32_t kPosMask = 0x1ffu;  // position field of a packed walk state (bit 8 = marker)
 
 struct DecArgs {
@@ -531,7 +518,6 @@ __global__ void __launch_bounds__(kChunkThreads, 6) chunk_sync_kernel(const DecA
 // function from at most max_len entries to (exit, symbols).  One thread per (chunk, entry) tabulates it; composing the
 // functions left to right is associative, so the true entry of every chunk comes out of a scan - no rounds, no luck.
 // The cost is max_len count walks instead of one (8 for byte-uniform data), all of them parallel.
-constexpr uint32_t kMaxStates = 16;
 __global__ void __launch_bounds__(kChunkThreads, 6) chunk_transfer_kernel(const DecArgs a, uint32_t s_log2, uint32_t n_states) {
     __shared__ __align__(16) uint32_t clut_sh[kLutSize];
     for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) clut_sh[i] = a.clut[i];
@@ -566,7 +552,6 @@ __global__ void __launch_bounds__(kChunkThreads, 6) chunk_transfer_kernel(const 
 //   compose_blocks    one block scans the block totals;
 //   compose_apply     every thread enters its segment with the true entry in hand and writes what the repair rounds
 //                     would have settled on: start_off, exit_off, count.
-constexpr uint32_t kSegChunks = 16, kSegThreads = 256;
 constexpr unsigned long long kIdentMap = 0xFEDCBA9876543210ull;
 __device__ __forceinline__ unsigned long long map_then(unsigned long long first, unsigned long long second, uint32_t n_states) {
     unsigned long long out = 0;
@@ -983,23 +968,16 @@ uint32_t unpack_chunk_bytes(const UnpackGeometry &g, const UnpackTuning &tune, u
     return cb;
 }
 
-size_t unpack_scratch_bytes(const UnpackGeometry &g, uint32_t chunk_bytes) {
-    const uint64_t n = chunk_count(g, chunk_bytes);
-    const uint64_t per = chunk_bytes == kLaneBytes ? 32 : kChunkThreads;  // chunks per scanned sum
-    const uint64_t nb = (n + per - 1) / per;
-    const uint64_t ng = (nb + kGroupRegions - 1) / kGroupRegions;
-    // exit (u8) and symbols (u16) per (chunk, entry); a map per segment of chunks and per block of segments
-    const size_t transfer = chunk_bytes == kLaneBytes ? 0 : (size_t)n * kMaxStates * 3 + 64 + ((size_t)n / kSegChunks + 2 * kSegThreads + 64) * 8;
-    return 64 + (size_t)nb * 8 + (size_t)n * (4 + 2 + 2 + sizeof(mid_t)) + 64 + (size_t)ng * 8 + 64 + (size_t)nb * (4 + 4 + 4 + 1) + 320 + transfer;
+size_t unpack_scratch_bytes(const UnpackGeometry &g, uint32_t chunk_bytes, uint32_t transfer_states) {
+    return decode_layout(nullptr, chunk_count(g, chunk_bytes), chunk_bytes == kLaneBytes, transfer_states).bytes;
 }
 
 // Lane-interleaved decoder: the same protocol as below with regions of 32 chunks per warp.  One extra
 // look at the scratch header after the scan: the largest region sizes the text stage of a warp.
-static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, const void *d_header, uint8_t *h_hdr, cudaStream_t stream,
+static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, const DecodeStatus *d_status, DecodeStatus *h_status, cudaStream_t stream,
                                        const UnpackTuning &tune, int *launches, uint32_t *rounds_out) {
     cudaError_t err;
     const int max_smem = tune.max_smem, num_sms = tune.num_sms;
-    const uint32_t *h_changed = reinterpret_cast<const uint32_t *>(h_hdr + 16);
     // count walk: one CTA per SM, as many warps as images fit beside the tables
     uint32_t sync_warps = ((uint32_t)max_smem - kSyncTableBytes) / kImgBytes;
     if (sync_warps > kMaxLaneWarps) sync_warps = kMaxLaneWarps;
@@ -1040,7 +1018,7 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
     edge_check_kernel<<<(n_regions + 255) / 256, 256, 0, stream>>>(a, n_regions);
     region_sync_kernel<<<sync_grid, sync_warps * 32, sync_smem, stream>>>(a, n_regions, 1, sync_warps);
     if (launches) *launches += 3;
-    if ((err = cudaMemsetAsync(a.changed, 0, 8, stream)) != cudaSuccess) return err;  // changed and max_sum
+    if ((err = cudaMemsetAsync(a.changed, 0, 2 * sizeof(uint32_t), stream)) != cudaSuccess) return err;  // changed and max_sum
     uint32_t rounds = 2;
     for (;;) {
         const uint32_t n_groups = (n_regions + kGroupRegions - 1) / kGroupRegions;
@@ -1053,7 +1031,7 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
             a, n_regions, (uint32_t)max_smem, write_warps);
         if (launches) *launches += 4;
         // one look at the scratch header: error flags, symbols found, "an entry was wrong", entry and exit of the shard
-        if ((err = cudaMemcpyAsync(h_hdr, d_header, 32, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return err;
+        if ((err = cudaMemcpyAsync(h_status, d_status, kDecodeStatusReadBack, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return err;
         if ((err = cudaStreamSynchronize(stream)) != cudaSuccess) return err;
         if ((tune.debug & 1) && d_dbg) {
             static unsigned long long h[2 * 256 * 35];
@@ -1081,21 +1059,21 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
         }
         if (tune.debug & 1)
             fprintf(stderr, "[lanes] regions=%u chunks=%u max_sum=%u rounds=%u changed=%u\n", n_regions, a.n_chunks,
-                    *reinterpret_cast<const uint32_t *>(h_hdr + 20), rounds, *h_changed);
-        if (*h_changed == 0) break;  // every entry was the true one: what the write walk produced stands
+                    h_status->max_sum, rounds, h_status->changed);
+        if (h_status->changed == 0) break;  // every entry was the true one: what the write walk produced stands
         // entries still moving: fixpoint rounds, four per host visit; a check that lists nothing is the proof
         for (;;) {
             for (int i = 0; i < 4; ++i)
                 if ((err = repair((int)rounds + i)) != cudaSuccess) return err;
             rounds += 4;
-            if ((err = cudaMemsetAsync(a.changed, 0, 8, stream)) != cudaSuccess) return err;
+            if ((err = cudaMemsetAsync(a.changed, 0, 2 * sizeof(uint32_t), stream)) != cudaSuccess) return err;
             if ((err = cudaMemsetAsync(a.work_count, 0, 4, stream)) != cudaSuccess) return err;
             region_check_kernel<<<check_grid, 256, 0, stream>>>(a, n_regions);
             if (launches) *launches += 1;
-            if ((err = cudaMemcpyAsync(h_hdr, d_header, 32, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return err;
+            if ((err = cudaMemcpyAsync(h_status, d_status, kDecodeStatusReadBack, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return err;
             if ((err = cudaStreamSynchronize(stream)) != cudaSuccess) return err;
-            if (tune.debug & 1) fprintf(stderr, "[lanes] repair rounds=%u changed=%u\n", rounds, *h_changed);
-            if (*h_changed == 0) break;
+            if (tune.debug & 1) fprintf(stderr, "[lanes] repair rounds=%u changed=%u\n", rounds, h_status->changed);
+            if (h_status->changed == 0) break;
             if (rounds > a.n_chunks + 8u) return cudaErrorUnknown;  // cannot happen: each round settles one more chunk
         }
         if ((err = cudaMemsetAsync(a.error_flags, 0, 4, stream)) != cudaSuccess) return err;  // raised by a wrong parse
@@ -1107,21 +1085,20 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
 
 cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const uint32_t *d_clut, const uint32_t *d_wlut,
                           const uint32_t *d_nodes, const uint16_t *d_slots, uint8_t *d_out, uint64_t max_symbols, void *scratch_base,
-                          uint8_t *h_hdr, cudaStream_t stream, const UnpackTuning &tune, uint32_t fixed_len, uint32_t transfer_states,
+                          DecodeStatus *h_status, cudaStream_t stream, const UnpackTuning &tune, uint32_t fixed_len, uint32_t transfer_states,
                           int *launches, uint32_t *rounds_out) {
-    uint32_t *h_flag = reinterpret_cast<uint32_t *>(h_hdr + 32);  // a word for the check rounds
     const uint64_t n64 = chunk_count(g, chunk_bytes);
-    uint8_t *p = static_cast<uint8_t *>(scratch_base);
-    cudaError_t err = cudaMemsetAsync(p, 0, 64, stream);
+    const bool lanes = chunk_bytes == kLaneBytes;
+    const DecodeLayout L = decode_layout(scratch_base, n64, lanes, transfer_states);
+    cudaError_t err = cudaMemsetAsync(L.status, 0, sizeof(DecodeStatus), stream);
     if (err != cudaSuccess) return err;
     if (rounds_out) *rounds_out = 0;
-    if (n64 == 0) {  // nothing to decode: an all-zero header
-        for (int i = 0; i < 32; ++i) h_hdr[i] = 0;
+    if (n64 == 0) {  // nothing to decode: all-zero status
+        *h_status = DecodeStatus{};
         return cudaStreamSynchronize(stream);
     }
     const uint32_t n = (uint32_t)n64;
-    const bool lanes = chunk_bytes == kLaneBytes;
-    const uint32_t nb = lanes ? (n + 31u) / 32u : (n + kChunkThreads - 1) / kChunkThreads;
+    const uint32_t nb = (uint32_t)L.n_blocks;
     DecArgs a;
     a.body_aligned = g.body_aligned;
     a.grid_bit = g.own_begin_bit / 256 * 256;  // chunks are whole 32-byte sectors
@@ -1141,30 +1118,29 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
     a.t_count = reinterpret_cast<const uint16_t *>(tune.d_lane_tables);
     a.t_write = reinterpret_cast<const uint32_t *>(static_cast<const uint8_t *>(tune.d_lane_tables) + kCountTableBytes);
     a.t_single = static_cast<const uint8_t *>(tune.d_lane_tables) + kCountTableBytes + kWriteTableBytes;
-    // [pad(4) | error flags(4) | total(8) | changed(4) | pad(4) | entry/exit(8)] then the arrays
-    a.error_flags = reinterpret_cast<uint32_t *>(p + 4);
-    a.total = reinterpret_cast<unsigned long long *>(p + 8);
-    a.changed = reinterpret_cast<uint32_t *>(p + 16);
-    a.max_sum = reinterpret_cast<uint32_t *>(p + 20);
-    a.entry_exit = reinterpret_cast<uint32_t *>(p + 24);
-    a.block_prefix = reinterpret_cast<unsigned long long *>(p + 64);
-    a.count = reinterpret_cast<uint32_t *>(p + 64 + (size_t)nb * 8);
-    a.start_off = reinterpret_cast<uint16_t *>(p + 64 + (size_t)nb * 8 + (size_t)n * 4);
-    a.exit_off = reinterpret_cast<uint16_t *>(p + 64 + (size_t)nb * 8 + (size_t)n * 6);
-    a.mid = reinterpret_cast<mid_t *>(p + 64 + (size_t)nb * 8 + (size_t)n * 8);
-    a.group_prefix = reinterpret_cast<unsigned long long *>(p + ((64 + (size_t)nb * 8 + (size_t)n * (8 + sizeof(mid_t)) + 63) & ~(size_t)63));
-    a.work = reinterpret_cast<uint32_t *>(a.group_prefix + (nb + 1023) / 1024 + 1);
-    a.work_count = reinterpret_cast<uint32_t *>(p + 32);
-    a.edge = a.work + nb + 8;
-    a.rsum = a.edge + nb + 8;
-    a.self_listed = reinterpret_cast<uint8_t *>(a.rsum + nb + 8);
-    a.tr_exit = reinterpret_cast<uint8_t *>(a.work) + (((size_t)nb * 13 + 256 + 63) & ~(size_t)63);
-    a.tr_cnt = reinterpret_cast<uint16_t *>(a.tr_exit + (size_t)n * kMaxStates);
+    a.error_flags = &L.status->error_flags;
+    a.total = &L.status->total;
+    a.changed = &L.status->changed;
+    a.max_sum = &L.status->max_sum;
+    a.entry_exit = &L.status->entry;
+    a.work_count = &L.status->work_count;
+    a.block_prefix = L.block_prefix;
+    a.count = L.count;
+    a.start_off = L.start_off;
+    a.exit_off = L.exit_off;
+    a.mid = L.mid;
+    a.group_prefix = L.group_prefix;
+    a.work = L.work;
+    a.edge = L.edge;
+    a.rsum = L.rsum;
+    a.self_listed = L.self_listed;
+    a.tr_exit = L.tr_exit;
+    a.tr_cnt = L.tr_cnt;
     a.out = d_out;
     a.max_symbols = max_symbols;
     a.dbg = nullptr;
 
-    if (lanes) return launch_unpack_lanes(a, nb, p, h_hdr, stream, tune, launches, rounds_out);
+    if (lanes) return launch_unpack_lanes(a, nb, L.status, h_status, stream, tune, launches, rounds_out);
 
     // Common case (codes that re-synchronise quickly): one walk from the guesses, one repair
     // round for the few chunks whose run-up was too short (text: 0.1 % of them; their exits do
@@ -1172,12 +1148,11 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
     // chunk), the final check fused into the block sums, the write walk — and a single look at
     // the flag at the very end.  Only when that check failed (slowly synchronising codes) do
     // the fixpoint rounds run, and the sums and the write walk are repeated.
-    const bool transfer = transfer_states >= 2 && transfer_states <= kMaxStates && !fixed_len && n > 1 && !tune.no_transfer;
+    const bool transfer = L.tr_log2 != 0 && !fixed_len && n > 1 && !tune.no_transfer;
     uint32_t rounds = 2;
     if (transfer) {
         // slowly synchronising codes: the chunks' transfer functions and a scan instead of repair rounds
-        uint32_t s_log2 = 1;
-        while ((1u << s_log2) < transfer_states) ++s_log2;
+        const uint32_t s_log2 = L.tr_log2;
         const uint64_t threads = (uint64_t)n << s_log2;
         if (tune.d_lane_tables && threads >= (uint64_t)tune.num_sms * kTransfer16Threads * 4 &&
             (size_t)tune.max_smem >= kCount16TableBytes + kLutSize * 4u) {
@@ -1187,13 +1162,10 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
             if (launches) *launches += 1;
         } else
             chunk_transfer_kernel<<<(unsigned)((threads + kChunkThreads - 1) / kChunkThreads), kChunkThreads, 0, stream>>>(a, s_log2, transfer_states);
-        const uint32_t seg_blocks = (n + kSegChunks * kSegThreads - 1) / (kSegChunks * kSegThreads);
-        unsigned long long *seg_prefix = reinterpret_cast<unsigned long long *>(a.tr_cnt + ((size_t)n << s_log2)) ;
-        seg_prefix = reinterpret_cast<unsigned long long *>((reinterpret_cast<uintptr_t>(seg_prefix) + 7) & ~(uintptr_t)7);
-        unsigned long long *block_map = seg_prefix + (size_t)seg_blocks * kSegThreads;
-        compose_segments_kernel<<<seg_blocks, kSegThreads, 0, stream>>>(a, s_log2, transfer_states, seg_prefix, block_map);
-        compose_blocks_kernel<<<1, 1024, 0, stream>>>(seg_blocks, transfer_states, block_map);
-        compose_apply_kernel<<<seg_blocks, kSegThreads, 0, stream>>>(a, s_log2, transfer_states, seg_prefix, block_map);
+        const uint32_t seg_blocks = (uint32_t)L.seg_blocks;
+        compose_segments_kernel<<<seg_blocks, kSegThreads, 0, stream>>>(a, s_log2, transfer_states, L.seg_prefix, L.block_map);
+        compose_blocks_kernel<<<1, 1024, 0, stream>>>(seg_blocks, transfer_states, L.block_map);
+        compose_apply_kernel<<<seg_blocks, kSegThreads, 0, stream>>>(a, s_log2, transfer_states, L.seg_prefix, L.block_map);
         if (launches) *launches += 4;
         rounds = 1;
     } else {
@@ -1213,11 +1185,11 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
             chunk_sync_kernel<<<nb, kChunkThreads, 0, stream>>>(a, (int)rounds + 3);
             rounds += 4;
             if (launches) *launches += 4;
-            e = cudaMemcpyAsync(h_flag, a.changed, 4, cudaMemcpyDeviceToHost, stream);
+            e = cudaMemcpyAsync(&h_status->changed, a.changed, 4, cudaMemcpyDeviceToHost, stream);
             if (e != cudaSuccess) return e;
             e = cudaStreamSynchronize(stream);
             if (e != cudaSuccess) return e;
-            if (*h_flag == 0) return cudaSuccess;
+            if (h_status->changed == 0) return cudaSuccess;
             if (rounds > n + 8u) return cudaErrorUnknown;  // cannot happen: each round settles one more chunk
         }
     };
@@ -1232,11 +1204,11 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
         chunk_scan_kernel<<<1, 1024, 0, stream>>>(a, a.block_prefix, nb);
         chunk_write_kernel<<<nb, kChunkThreads, 0, stream>>>(a);
         if (launches) *launches += 3;
-        err = cudaMemcpyAsync(h_hdr, p, 32, cudaMemcpyDeviceToHost, stream);  // the whole scratch header, for the caller as well
+        err = cudaMemcpyAsync(h_status, L.status, kDecodeStatusReadBack, cudaMemcpyDeviceToHost, stream);  // for the caller as well
         if (err != cudaSuccess) return err;
         err = cudaStreamSynchronize(stream);
         if (err != cudaSuccess) return err;
-        if (*reinterpret_cast<const uint32_t *>(h_hdr + 16) == 0) break;  // every entry was the true one: what the write walk produced stands
+        if (h_status->changed == 0) break;  // every entry was the true one: what the write walk produced stands
         err = settle();
         if (err != cudaSuccess) return err;
         // the error flags the first write walk may have raised came from a wrong parse
