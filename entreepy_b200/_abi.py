@@ -4,7 +4,7 @@ import ctypes
 import os
 
 PKG = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("ET_LIB") or os.path.join(PKG, "lib", "libentreepy_b200.so")  # ET_LIB: a tuning variant (build.build_variant)
+LIB_PATH = os.environ.get("ET_LIB") or os.path.join(PKG, "lib", "libentreepy_b200.so")  # ET_LIB: another build of the library, to compare two builds run for run
 
 OK = 0
 ERR_QUEUE_EMPTY, ERR_NO_SPACE, ERR_OUT_OF_MEMORY, ERR_CUDA, ERR_NO_DEVICE = 1, 2, 3, 4, 5
@@ -12,7 +12,7 @@ ERR_CORRUPT, ERR_TOO_LARGE, ERR_UNSUPPORTED, ERR_INVALID_ARG = 6, 7, 8, 9
 
 FLAG_WRITE_OUTPUT, FLAG_PRINT_OUTPUT, FLAG_DEBUG = 0x1, 0x2, 0x4
 FLAG_QUIET, FLAG_NO_SCRATCH_LIMIT, FLAG_VALIDATE, FLAG_TIMING = 0x100, 0x200, 0x400, 0x800
-TUNE_LANE_MIN_BYTES, TUNE_DEBUG, TUNE_SYNC_WARPS, TUNE_PACK_SINGLE_PASS, TUNE_NO_TRANSFER, TUNE_WRITE_WARPS = 1, 2, 3, 4, 5, 6
+TUNE_LANE_MIN_BYTES, TUNE_DEBUG, TUNE_NO_TRANSFER = 1, 2, 5  # 3, 4 and 6 are retired
 
 # every symbol include/entreepy_b200.h declares
 SYMBOLS = [

@@ -40,20 +40,6 @@ def _stale(target, deps):
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_variant(tag, defines):
-    """A tuning variant of the library (tools/variants.py): lib/libentreepy_b200_<tag>.so built with -D flags;
-    ET_LIB=<path> makes entreepy_b200._abi load it instead of the product library."""
-    os.makedirs(LIBDIR, exist_ok=True)
-    out = os.path.join(LIBDIR, f"libentreepy_b200_{tag}.so")
-    srcs = [os.path.join(CSRC, s) for s in SOURCES]
-    cmd = [nvcc(), *NVCC_FLAGS, *[f"-D{d}" for d in defines], "-shared", "-o", out, *srcs]
-    res = subprocess.run(cmd, capture_output=True, text=True)
-    if res.returncode != 0:
-        sys.stderr.write(res.stdout + res.stderr)
-        raise RuntimeError(f"nvcc failed building variant {tag}")
-    return out
-
-
 def build(force=False, verbose=False):
     os.makedirs(LIBDIR, exist_ok=True)
     os.makedirs(os.path.dirname(CLI), exist_ok=True)

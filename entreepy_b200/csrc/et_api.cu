@@ -197,7 +197,7 @@ int pack_dev(et_ctx *ctx, const void *d_in, size_t n, const et_codebook &cb, uin
     if (rc != ET_OK) return rc;
     int launches = 0;
     ET_CUDA(ctx, launch_pack(g, ctx->d_small->pack_tables, wide, cb.max_length, d_body, bit_phase, ctx->d_scratch, ctx->num_sms, s,
-                             &launches, ctx->tune.pack_single_pass != 0, ctx->tune.pack_bits_ctas));
+                             &launches, ctx->tune.pack_bits_ctas));
     ctx->launches += (uint64_t)launches;
     return ET_OK;
 }
@@ -318,10 +318,7 @@ extern "C" int et_ctx_set_tuning(et_ctx *ctx, int key, long long value) {
     switch (key) {
         case ET_TUNE_LANE_MIN_BYTES: ctx->tune.lane_min_bytes = value; return ET_OK;
         case ET_TUNE_DEBUG: ctx->tune.debug = (int)value; return ET_OK;  // bit 0: lane decoder timings, bit 1: phases of the sharded calls
-        case ET_TUNE_SYNC_WARPS: ctx->tune.sync_warps = (int)value; return ET_OK;
-        case ET_TUNE_WRITE_WARPS: ctx->tune.write_warps = (int)value; return ET_OK;
         case ET_TUNE_NO_TRANSFER: ctx->tune.no_transfer = value != 0; return ET_OK;
-        case ET_TUNE_PACK_SINGLE_PASS: ctx->tune.pack_single_pass = value != 0; return ET_OK;
     }
     return fail(ctx, ET_ERR_INVALID_ARG, "unknown tuning key %d", key);
 }

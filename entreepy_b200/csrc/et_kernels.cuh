@@ -34,7 +34,7 @@ size_t pack_scratch_bytes(const PackGeometry &g);
 // bits_ctas_per_sm: from pack_init_device() (0: ask the runtime at every call).
 cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, uint32_t max_len, uint8_t *d_out, uint32_t bit_phase,
                         void *scratch_base, int num_sms,
-                        cudaStream_t stream, int *launches, bool single_pass = false, int bits_ctas_per_sm = 0);
+                        cudaStream_t stream, int *launches, int bits_ctas_per_sm = 0);
 // Once per context: lets the pack kernels use all of an SM's shared memory and reads how many CTAs of pass A fit an SM
 // (both used to be asked of the runtime at every call, a few microseconds each with the GPU waiting).
 cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm);
@@ -69,10 +69,7 @@ struct UnpackTuning {
     int debug = 0;
     int max_smem = 0;  // cudaDevAttrMaxSharedMemoryPerBlockOptin
     int num_sms = 0;
-    int sync_warps = 0;             // > 0: warps per CTA of the count walk (default: as many as fit)
-    int write_warps = 0;            // > 0: warps per CTA of the write walk (default: as many as fit)
     int no_transfer = 0;            // non-zero: slowly synchronising codes take the repair rounds instead of transfer functions
-    int pack_single_pass = 0;       // non-zero: the encoder packs in ONE pass with a decoupled look-back (measured slower, see et_pack.cu)
     int pack_bits_ctas = 0;         // CTAs of pack pass A per SM (pack_init_device)
     void *d_lane_tables = nullptr;  // device-built tables of the lane-interleaved decoder
 };

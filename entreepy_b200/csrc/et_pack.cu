@@ -15,11 +15,12 @@
 //                             time); adjacent symbols are fused into pairs when they fit 32
 //                             bits; everything goes through one 64-bit accumulator whose whole
 //                             words are ORed straight into their place in the warp's shared bit
-//                             image; the image is funnel-shifted to the region's final bit
-//                             position, byte-swapped to stream order (big-endian bit packing)
-//                             and stored as aligned 16-byte vectors.
-// A single-pass decoupled look-back was built first and measured: the chain of descriptors could
-// not retire more than ~64 tiles/us.  With the offsets known from pass A every region is independent.
+//                             image, which is assembled at the region's final bit position inside
+//                             its 16-byte output blocks; the image is byte-swapped to stream order
+//                             (big-endian bit packing) and stored as aligned 16-byte vectors.
+// A single pass with a decoupled look-back over tiles of 16 regions was built and measured (r2, text-1G: 1.93 ms
+// against 0.93 ms for the two passes): the CTA-wide lockstep it needs bounds it (stall_barrier 4.6 per issued
+// instruction).  With the offsets known from pass A every region is independent.
 // Codes longer than 32 bits (where the reference itself emits truncated paths, SURVEY §0.4) use
 // the wide kernel further down (4096-symbol tiles, look-back).
 //
@@ -38,19 +39,6 @@ namespace et {
 namespace {
 
 constexpr int kWarps = kPackThreads / 32;
-
-template <bool WIDE>
-struct PackCfg;
-template <>
-struct PackCfg<true> {
-    static constexpr int kMaxLen = 64;
-    static constexpr int kTableBytes = 256 * 8 + 256;  // codes + lengths, not replicated
-};
-// worst-case tile bits + up to 127 bits of alignment slack + one spare word, in uint4 units
-template <bool WIDE>
-struct StageWords {
-    static constexpr int value = (((kPackTileSyms * PackCfg<WIDE>::kMaxLen + 128 + 32) + 127) / 128) * 4;
-};
 
 struct PackArgs {
     const uint8_t *in_aligned;
@@ -72,7 +60,6 @@ struct PackArgs {
     uint16_t *run_bits;                // [32 * regions] lane-run pack: bits of every run of 64 symbols
     uint32_t n_regions;                // lane-run pack: regions of 2048 symbols (one warp each)
     uint32_t image_words;              // lane-run pack: words of a warp's bit image (guard included)
-    unsigned long long *tile_desc;     // single-pass pack: look-back descriptors, one per tile of `warps` regions
 };
 
 __device__ __forceinline__ uint32_t warp_inclusive_scan(uint32_t v, uint32_t lane) {
@@ -149,9 +136,9 @@ __global__ void __launch_bounds__(1024) group_scan_kernel(const PackArgs a, uint
 //   pass B  pack_runs_kernel: persistent warps.  A lane owns one run: four 16-byte loads, its
 //           bit offset inside the region from a warp scan of the run totals, then the 64
 //           symbols go through one 64-bit accumulator straight to their place in the warp's
-//           shared bit image.  The image is shifted to the region's bit position, swapped to
-//           stream order and stored as aligned 16-byte vectors; the two bytes a region may
-//           share with its neighbours take the seam arrays, as above.
+//           shared bit image, at the region's bit position in its output blocks.  The image is
+//           swapped to stream order and stored as aligned 16-byte vectors; the two bytes a
+//           region may share with its neighbours take the seam arrays, as above.
 constexpr int kRunSyms = 64;
 constexpr int kRegionSyms = 32 * kRunSyms;  // 2048
 constexpr int kRunWarps = 16;
@@ -375,17 +362,14 @@ __device__ __forceinline__ void pack_run_symbols(BitAcc &acc, const uint4 (&raw)
     }
 }
 
-// The finished bit image of region r (region bit b in word kStageGuard + (b >> 5), MSB first) goes to its place in the
-// output: shifted to the region's final bit position, swapped to stream order, stored as aligned 16-byte vectors; the
-// (at most two) bytes it shares with its neighbours go to the seam arrays.
-// Frame: the 16-byte blocks of the output that the region touches; frame bit of region bit 0 (< 128):
+// The finished bit image of region r goes to its place in the output: swapped to stream order, stored as aligned 16-byte
+// vectors; the (at most two) bytes it shares with its neighbours go to the seam arrays.  The image is assembled at frame
+// positions (frame: the 16-byte blocks of the output that the region touches; frame word f is image word kStageGuard + f,
+// MSB first: pack_runs_kernel knows where the region goes before it packs), so a block of the output is four image words
+// as they stand.  Frame bit of region bit 0 (< 128):
 __device__ __forceinline__ uint32_t region_frame_shift(const PackArgs &a, unsigned long long bit_begin) {
     return (uint32_t)(reinterpret_cast<uintptr_t>(a.out + (bit_begin >> 3)) & 15u) * 8u + (uint32_t)(bit_begin & 7);
 }
-// IN_FRAME: the image was assembled at frame positions already (image bit = frame bit: pack_runs_kernel knows where the
-// region goes before it packs), so a block of the output is four image words as they stand; else the image starts at
-// region bit 0 and is funnel-shifted here.
-template <bool IN_FRAME = false>
 __device__ __forceinline__ void region_copy_out(const PackArgs &a, uint32_t r, const uint32_t *stage, uint8_t *edge,
                                                 unsigned long long bit_begin, uint32_t region_bits, uint32_t lane) {
     const unsigned long long bit_end = bit_begin + region_bits;
@@ -395,74 +379,43 @@ __device__ __forceinline__ void region_copy_out(const PackArgs &a, uint32_t r, c
     const uint32_t shift = align * 8 + (uint32_t)(bit_begin & 7);  // frame bit of region bit 0 (< 128)
     const uint32_t used_bits = shift + region_bits;
     const uint32_t n_chunks = (used_bits + 127u) >> 7;
-    {
-        const unsigned long long byte0 = bit_begin >> 3;
-        const unsigned long long full_lo = (bit_begin + 7) >> 3, full_hi = bit_end >> 3;  // owned bytes [lo,hi)
-        const uint32_t s_lo = (uint32_t)(full_lo - byte0) + align;                       // frame coordinates
-        const uint32_t s_hi = full_hi >= full_lo ? (uint32_t)(full_hi - byte0) + align : s_lo;
-        const bool has_head = (bit_begin & 7) != 0;
-        const bool has_tail = (bit_end & 7) != 0 && full_hi >= full_lo;
-        const uint32_t s_head = align;
-        const uint32_t s_tail = (uint32_t)(full_hi - byte0) + align;  // only meaningful when has_tail
-        if (lane == 0) {
-            if (!has_head) a.seam_head[r] = 0;
-            if (!has_tail) a.seam_tail[r] = 0;
-        }
-        // frame word f holds region bits [32f - shift, 32f - shift + 32): image word f - ws shifted right by bs
-        // bits, its top bits coming from the word before.  Two aligned 16-byte shared loads per chunk (the four
-        // image words of the chunk and the four before them: conflict-free), then a warp-uniform choice of which
-        // of the eight words feed which frame word.
-        const uint32_t bs = shift & 31u, ws = shift >> 5;
-        for (uint32_t c = lane; c < n_chunks; c += 32) {
-            const uint4 *src = reinterpret_cast<const uint4 *>(stage + kStageGuard) + c;
-            const uint4 q = src[0];
-            uint4 p = q;
-            if (!IN_FRAME) p = src[-1];
-            uint32_t f0, f1, f2, f3;
-            if (IN_FRAME) {
-                f0 = q.x; f1 = q.y; f2 = q.z; f3 = q.w;
-            } else switch (ws) {
-                case 0:
-                    f0 = __funnelshift_r(q.x, p.w, bs); f1 = __funnelshift_r(q.y, q.x, bs);
-                    f2 = __funnelshift_r(q.z, q.y, bs); f3 = __funnelshift_r(q.w, q.z, bs);
-                    break;
-                case 1:
-                    f0 = __funnelshift_r(p.w, p.z, bs); f1 = __funnelshift_r(q.x, p.w, bs);
-                    f2 = __funnelshift_r(q.y, q.x, bs); f3 = __funnelshift_r(q.z, q.y, bs);
-                    break;
-                case 2:
-                    f0 = __funnelshift_r(p.z, p.y, bs); f1 = __funnelshift_r(p.w, p.z, bs);
-                    f2 = __funnelshift_r(q.x, p.w, bs); f3 = __funnelshift_r(q.y, q.x, bs);
-                    break;
-                default:
-                    f0 = __funnelshift_r(p.y, p.x, bs); f1 = __funnelshift_r(p.z, p.y, bs);
-                    f2 = __funnelshift_r(p.w, p.z, bs); f3 = __funnelshift_r(q.x, p.w, bs);
-                    break;
-            }
-            const uint4 v = make_uint4(bswap32(f0), bswap32(f1), bswap32(f2), bswap32(f3));
-            const uint32_t k0 = c * 16;
-            if (k0 >= s_lo && k0 + 16 <= s_hi) {
-                st_stream_v4(gbase + k0, v);
-            } else {
-                // a block at the ragged start (slot 0) or end (slot 1) of the region: parked, the warp stores its bytes below
-                *reinterpret_cast<uint4 *>(edge + (c == 0 ? 0 : 16)) = v;
-            }
-        }
-        // The two ragged blocks, one byte per lane (lanes 0-15: the first block, 16-31: the last one): a single lane
-        // walking their bytes one at a time cost the warp ~200 instructions per region with 31 lanes idle.
-        __syncwarp();
-        if (n_chunks) {
-            const uint32_t blk = lane < 16 ? 0u : n_chunks - 1u, k0 = blk * 16u, k = k0 + (lane & 15u);
-            const bool ragged = !(k0 >= s_lo && k0 + 16u <= s_hi) && (lane < 16 || n_chunks > 1);
-            if (ragged) {
-                const uint32_t byte = edge[(lane < 16 ? 0u : 16u) + (lane & 15u)];
-                if (k >= s_lo && k < s_hi) gbase[k] = (uint8_t)byte;
-                if (has_head && k == s_head) a.seam_head[r] = (uint8_t)byte;
-                if (has_tail && k == s_tail) a.seam_tail[r] = (uint8_t)byte;
-            }
-        }
-        __syncwarp();  // the slots are free again
+    const unsigned long long byte0 = bit_begin >> 3;
+    const unsigned long long full_lo = (bit_begin + 7) >> 3, full_hi = bit_end >> 3;  // owned bytes [lo,hi)
+    const uint32_t s_lo = (uint32_t)(full_lo - byte0) + align;                       // frame coordinates
+    const uint32_t s_hi = full_hi >= full_lo ? (uint32_t)(full_hi - byte0) + align : s_lo;
+    const bool has_head = (bit_begin & 7) != 0;
+    const bool has_tail = (bit_end & 7) != 0 && full_hi >= full_lo;
+    const uint32_t s_head = align;
+    const uint32_t s_tail = (uint32_t)(full_hi - byte0) + align;  // only meaningful when has_tail
+    if (lane == 0) {
+        if (!has_head) a.seam_head[r] = 0;
+        if (!has_tail) a.seam_tail[r] = 0;
     }
+    for (uint32_t c = lane; c < n_chunks; c += 32) {
+        const uint4 q = reinterpret_cast<const uint4 *>(stage + kStageGuard)[c];
+        const uint4 v = make_uint4(bswap32(q.x), bswap32(q.y), bswap32(q.z), bswap32(q.w));
+        const uint32_t k0 = c * 16;
+        if (k0 >= s_lo && k0 + 16 <= s_hi) {
+            st_stream_v4(gbase + k0, v);
+        } else {
+            // a block at the ragged start (slot 0) or end (slot 1) of the region: parked, the warp stores its bytes below
+            *reinterpret_cast<uint4 *>(edge + (c == 0 ? 0 : 16)) = v;
+        }
+    }
+    // The two ragged blocks, one byte per lane (lanes 0-15: the first block, 16-31: the last one): a single lane
+    // walking their bytes one at a time cost the warp ~200 instructions per region with 31 lanes idle.
+    __syncwarp();
+    if (n_chunks) {
+        const uint32_t blk = lane < 16 ? 0u : n_chunks - 1u, k0 = blk * 16u, k = k0 + (lane & 15u);
+        const bool ragged = !(k0 >= s_lo && k0 + 16u <= s_hi) && (lane < 16 || n_chunks > 1);
+        if (ragged) {
+            const uint32_t byte = edge[(lane < 16 ? 0u : 16u) + (lane & 15u)];
+            if (k >= s_lo && k < s_hi) gbase[k] = (uint8_t)byte;
+            if (has_head && k == s_head) a.seam_head[r] = (uint8_t)byte;
+            if (has_tail && k == s_tail) a.seam_tail[r] = (uint8_t)byte;
+        }
+    }
+    __syncwarp();  // the slots are free again
 }
 
 // Pass B.  Dynamic shared memory: table (32 KiB, 16-lane replicated) | per warp: bit image | per warp: 32 edge bytes.
@@ -546,150 +499,23 @@ __global__ void __launch_bounds__(kRunWarps * 32, 2) pack_runs_kernel(const Pack
             if (acc.pos & 31u) atomicOr(stage + kStageGuard + ((shift + my_off + my_bits) >> 5), acc.lo << (32u - (acc.pos & 31u)));
         }
         __syncwarp();  // image complete
-        region_copy_out<true>(a, r, stage, edge, bit_begin, region_bits, lane);
+        region_copy_out(a, r, stage, edge, bit_begin, region_bits, lane);
         __syncwarp();  // everyone has read the image
         if (r_next >= a.n_regions) break;
         r = r_next;
     }
 }
 
-// ------------------------------------------------------------------ single-pass pack (codes <= 32 bits)
-// ONE pass over the text: the offsets come from a decoupled look-back instead of a first pass.
-// A CTA works on a TILE of `warps` consecutive regions (one warp each), tiles are handed out in order by a ticket:
-//   1. a lane packs the 64 symbols of its run into a PRIVATE bit string in shared memory, from bit 0 of its own
-//      words (no offset needed yet); its length is the run's bit count;
-//   2. warp scan of the run lengths: the lane's bit offset inside the region, the region's bits;
-//   3. the region totals of the tile meet in shared memory (named barrier: the other warps only arrive); warp 0 scans
-//      them, publishes the tile's bit count in its look-back descriptor and walks back over the descriptors of the
-//      tiles before it (aggregates until the first inclusive prefix) - while the other warps do step 4;
-//   4. every lane shifts its private string to its offset inside the warp's region image (funnel shift per word;
-//      whole words are stored, the two words it shares with its neighbours are ORed into zeroed words);
-//   5. barrier; the region's final bit position is the tile's base plus the totals of the warps before: the image goes
-//      out exactly as in the two-pass kernel (region_copy_out).
-// What the look-back costs: one 8-byte descriptor per 32 Ki symbols (16 warps) and, in the steady state, one or two L2
-// round trips per tile, hidden behind step 4.  (The first attempt at this, with 4 Ki-symbol tiles, was limited by the
-// descriptor chain - ~64 tiles/us - to 4 ms/GiB; at CTA-sized tiles the chain needs 33 K steps per GiB instead of 262 K.)
-// MEASURED (r2, text-1G, profiles/r2_kernels.md): 1.93 ms against 0.29 + 0.77 ms for the two passes.  The chain is no
-// longer the limit; the CTA-wide lockstep is (stall_barrier 4.6 per issued instruction, 0.34 IPC per scheduler), and the
-// private strings double a warp's shared memory, which halves the warps per SM.  The two-pass pack therefore stays the
-// default and this kernel is selectable (ET_TUNE_PACK_SINGLE_PASS) - it reads the text once (DRAM 1.09 + 0.58 GB vs
-// 2.17 + 0.63 GB) and would win on a part where HBM, not instruction issue, bounds this path.
-constexpr int kTileMaxWarps = 16;
-struct TileShared {
-    uint32_t region_bits[kTileMaxWarps];
-    unsigned long long tile_base;
-    uint32_t next_tile;
-};
-__device__ __forceinline__ void named_bar_sync(int id, int threads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
-__device__ __forceinline__ void named_bar_arrive(int id, int threads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
-
-// Dynamic shared memory: table (32 KiB) | per warp: private strings (32 lanes x priv_stride words) | bit image | 32 edge bytes.
-__global__ void __launch_bounds__(kTileMaxWarps * 32, 1) pack_tiles_kernel(const PackArgs a, uint32_t warps, uint32_t priv_stride, uint32_t n_tiles) {
-    extern __shared__ __align__(16) uint8_t smem[];
-    __shared__ TileShared sh;
-    uint8_t *table = smem;
-    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, threads = warps * 32;
-    const uint32_t warp_words = 32u * priv_stride + a.image_words;
-    uint32_t *priv = reinterpret_cast<uint32_t *>(smem + kTableBytes) + (size_t)warp * warp_words + lane * priv_stride;
-    uint32_t *stage = reinterpret_cast<uint32_t *>(smem + kTableBytes) + (size_t)warp * warp_words + 32u * priv_stride;
-    uint8_t *edge = smem + kTableBytes + (size_t)warps * warp_words * 4 + warp * 32;
-    {
-        const uint2 *src = static_cast<const uint2 *>(a.tables);
-        uint2 *dst = reinterpret_cast<uint2 *>(table);
-        for (uint32_t i = tid; i < 256 * kTableLanes; i += threads) dst[i] = src[i / kTableLanes];
-        for (uint32_t i = lane; i < a.image_words; i += 32) stage[i] = 0;
-        if (tid == 0) sh.next_tile = atomicAdd(a.ticket, 1u);
-    }
-    __syncthreads();
-    const uint8_t *table_lane = table + (lane & (kTableLanes - 1)) * 8;
-    const uint32_t r128 = opaque_128(a);
-    const uint32_t priv_bit0 = (uint32_t)__cvta_generic_to_shared(priv) * 8u;
-
-    for (;;) {
-        const uint32_t tile = sh.next_tile;
-        if (tile >= n_tiles) break;
-        const uint32_t r = tile * warps + warp;
-        const bool live = r < a.n_regions;
-        // ---- 1. the run into the lane's private string
-        uint32_t my_bits = 0;
-        if (live) {
-            const bool interior = region_is_interior(a, r);
-            uint4 raw[4];
-            unsigned long long valid;
-            load_run(a, r, lane, interior, raw, &valid);
-            BitAcc acc;
-            open_acc(acc, priv_bit0);
-            pack_run_symbols(acc, raw, valid, interior, table_lane, r128);
-            my_bits = acc.pos - priv_bit0;
-            if (my_bits & 31u) priv[my_bits >> 5] = acc.lo << (32u - (my_bits & 31u));  // the unfinished last word, zero padded
-        }
-        // ---- 2. offsets inside the region
-        const uint32_t incl = warp_inclusive_scan(my_bits, lane);
-        const uint32_t region_bits = __shfl_sync(0xffffffffu, incl, 31);
-        const uint32_t my_off = incl - my_bits;
-        if (lane == 0) sh.region_bits[warp] = region_bits;
-        // ---- 3. the tile's bit count meets the tiles before it (warp 0), the others go on
-        if (warp != 0) {
-            named_bar_arrive(1, (int)threads);
-        } else {
-            named_bar_sync(1, (int)threads);
-            uint32_t mine = lane < warps ? sh.region_bits[lane] : 0u;
-            const uint32_t tile_bits = __reduce_add_sync(0xffffffffu, mine);
-            unsigned long long start;
-            if (tile == 0) {
-                start = a.bit_phase;
-            } else {
-                if (lane == 0) st_relaxed_u64(a.tile_desc + tile, kStatusAggregate | tile_bits);
-                start = lookback_exclusive(a.tile_desc, tile, lane);
-            }
-            if (lane == 0) {
-                st_relaxed_u64(a.tile_desc + tile, kStatusPrefix | (start + tile_bits));
-                sh.tile_base = start;
-                sh.next_tile = atomicAdd(a.ticket, 1u);  // every warp has read the current one: it arrived at barrier 1
-            }
-        }
-        // ---- 4. private strings to their place in the region image
-        if (live) {
-            const uint32_t w0 = my_off >> 5, s = my_off & 31u, n_w = (my_bits + 31u) >> 5;
-            const uint32_t w_last = (my_off + my_bits) >> 5;  // the word after the lane's last bit may be this one too
-            uint32_t *img = stage + kStageGuard;
-            // words shared with the neighbours (and the two after the region's end, which the copy-out reads) start from zero
-            if (my_bits) {
-                img[w0] = 0;
-                img[w_last] = 0;
-            }
-            if (lane < 2) img[(region_bits >> 5) + lane] = 0;
-            __syncwarp();
-            uint32_t prev = 0;
-            for (uint32_t j = 0; j <= n_w && my_bits; ++j) {
-                const uint32_t cur = j < n_w ? priv[j] : 0u;
-                const uint32_t v = __funnelshift_r(cur, prev, s);  // (prev:cur) >> s: the low s bits of prev on top of cur's high bits
-                prev = cur;
-                if (j == 0 || w0 + j >= w_last) {
-                    if (v) atomicOr(img + w0 + j, v);
-                } else {
-                    img[w0 + j] = v;
-                }
-            }
-        }
-        // ---- 5. the tile's base is known: out it goes
-        named_bar_sync(2, (int)threads);
-        if (live) {
-            unsigned long long bit_begin = sh.tile_base;
-            for (uint32_t q = 0; q < warp; ++q) bit_begin += sh.region_bits[q];
-            if (lane == 0) a.tile_state[r] = bit_begin + region_bits;  // for the seam fix-up
-            region_copy_out(a, r, stage, edge, bit_begin, region_bits, lane);
-        }
-        named_bar_sync(3, (int)threads);  // sh.region_bits and sh.tile_base may be overwritten; next_tile is settled
-    }
-}
-
 // ------------------------------------------------------------------ wide kernel (codes of 33..64 bits)
-template <bool WIDE>
+constexpr int kWideMaxLen = 64;
+constexpr int kWideTableBytes = 256 * 8 + 256;  // codes + lengths, not replicated
+// worst-case tile bits + up to 127 bits of alignment slack + one spare word, in uint4 units
+constexpr int kWideStageWords = (((kPackTileSyms * kWideMaxLen + 128 + 32) + 127) / 128) * 4;
+
 __global__ void __launch_bounds__(kPackThreads) pack_wide_kernel(const PackArgs a) {
     extern __shared__ __align__(16) uint8_t smem[];
     uint32_t *stage = reinterpret_cast<uint32_t *>(smem);
-    uint8_t *table = smem + StageWords<WIDE>::value * 4;
+    uint8_t *table = smem + kWideStageWords * 4;
     __shared__ uint32_t warp_sum[kWarps];
     __shared__ unsigned long long tile_base_sh;
     __shared__ uint32_t tile_sh;
@@ -697,10 +523,10 @@ __global__ void __launch_bounds__(kPackThreads) pack_wide_kernel(const PackArgs 
 
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
-    for (int i = tid; i < StageWords<WIDE>::value; i += kPackThreads) stage[i] = 0;
+    for (int i = tid; i < kWideStageWords; i += kPackThreads) stage[i] = 0;
     {
         const uint8_t *src = static_cast<const uint8_t *>(a.tables);
-        for (int i = tid; i < PackCfg<true>::kTableBytes; i += kPackThreads) table[i] = src[i];
+        for (int i = tid; i < kWideTableBytes; i += kPackThreads) table[i] = src[i];
     }
     const unsigned long long *wide_code = reinterpret_cast<const unsigned long long *>(table);
     const uint8_t *wide_len = table + 256 * 8;
@@ -896,8 +722,7 @@ cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm) {
 }
 
 cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, uint32_t max_len, uint8_t *d_out, uint32_t bit_phase,
-                        void *scratch_base, int num_sms, cudaStream_t stream, int *launches, bool single_pass,
-                        int bits_ctas_per_sm) {
+                        void *scratch_base, int num_sms, cudaStream_t stream, int *launches, int bits_ctas_per_sm) {
     if (g.num_tiles == 0) return cudaSuccess;
     const PackLayout s = pack_layout(scratch_base, g.num_tiles);
     cudaError_t err = cudaSuccess;
@@ -913,7 +738,6 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
     a.seam_head = s.seam_head;
     a.seam_tail = s.seam_tail;
     a.ticket = s.ticket;
-    a.tile_desc = s.tile_desc;
     a.tile_bits = s.tile_bits;
     a.group_prefix = s.group_prefix;
     a.group_tiles = 1;
@@ -926,15 +750,15 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
         // look-back descriptors and the ticket start from zero
         err = cudaMemsetAsync(s.ticket, 0, reinterpret_cast<uint8_t *>(s.tile_state + g.num_tiles) - reinterpret_cast<uint8_t *>(s.ticket), stream);
         if (err != cudaSuccess) return err;
-        const int smem = StageWords<true>::value * 4 + PackCfg<true>::kTableBytes;
-        err = cudaFuncSetAttribute(pack_wide_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        const int smem = kWideStageWords * 4 + kWideTableBytes;
+        err = cudaFuncSetAttribute(pack_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
         if (err != cudaSuccess) return err;
         int per_sm = (227 * 1024) / (smem + 1024);
         if (per_sm > 2048 / kPackThreads) per_sm = 2048 / kPackThreads;
         if (per_sm < 1) per_sm = 1;
         unsigned grid = (unsigned)num_sms * (unsigned)per_sm;
         if (grid > g.num_tiles) grid = g.num_tiles;
-        pack_wide_kernel<true><<<grid, kPackThreads, smem, stream>>>(a);
+        pack_wide_kernel<<<grid, kPackThreads, smem, stream>>>(a);
         if (launches) *launches += 1;
     } else {
         // lane-run path: regions of 2048 symbols, in the slots of the same layout
@@ -947,32 +771,6 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
         if (a.interior_hi < a.interior_lo) a.interior_hi = a.interior_lo;
         a.image_words = (uint32_t)(kStageGuard + (kRegionSyms * max_len + 31) / 32 + 16 + 3) & ~3u;
         if (a.image_words < kStageGuard + kRegionSyms / 4) a.image_words = kStageGuard + kRegionSyms / 4;  // the image also stages the region's text
-        if (single_pass) {
-            // single pass: tiles of `warps` regions, each with a look-back descriptor
-            const uint32_t priv_stride = (2u * max_len + 1u) | 1u;  // words of a lane's private string (64 codes), odd: lanes never share a bank at equal depth
-            const uint32_t warp_bytes = (32u * priv_stride + a.image_words) * 4u + 32u;
-            int max_smem = 0, dev = 0;
-            if ((err = cudaGetDevice(&dev)) != cudaSuccess) return err;
-            if ((err = cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return err;
-            uint32_t warps = ((uint32_t)max_smem - (uint32_t)kTableBytes - 1024u) / warp_bytes;
-            if (warps > (uint32_t)kTileMaxWarps) warps = kTileMaxWarps;
-            if (warps > 4) warps &= ~3u;
-            if (warps >= 1) {
-                const uint32_t n_tiles = (n_regions + warps - 1) / warps;
-                if ((err = cudaMemsetAsync(s.ticket, 0, 16, stream)) != cudaSuccess) return err;
-                if ((err = cudaMemsetAsync(a.tile_desc, 0, (size_t)n_tiles * 8, stream)) != cudaSuccess) return err;
-                const int smem = kTableBytes + (int)(warps * warp_bytes);
-                if ((err = cudaFuncSetAttribute(pack_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)) != cudaSuccess) return err;
-                unsigned grid = (unsigned)num_sms * (2u * (unsigned)smem + 2048u <= (unsigned)max_smem ? 2u : 1u);
-                if (grid > n_tiles) grid = n_tiles;
-                pack_tiles_kernel<<<grid, warps * 32, smem, stream>>>(a, warps, priv_stride, n_tiles);
-                if (launches) *launches += 1;
-                if ((err = cudaGetLastError()) != cudaSuccess) return err;
-                seam_fixup_kernel<<<(n_regions + 255) / 256, 256, 0, stream>>>(a.tile_state, a.seam_head, a.seam_tail, n_regions, bit_phase, d_out);
-                if (launches) *launches += 1;
-                return cudaGetLastError();
-            }
-        }
         // pass A: run and region totals (a warp per region), prefixes inside groups of 1024 regions, prefixes of the groups
         // (a region holds at most 2048 x 32 bits, a group 2^26: the prefix inside a group fits 32 bits)
         a.group_tiles = kPrefixGroup;

@@ -9,18 +9,8 @@ namespace et {
 
 constexpr int kChunkThreads = 256;  // chunks per CTA of the per-thread decoder
 
-// Parts of a chunk that the lane write walk decodes side by side (et_lanes.inc).  MEASURED (r2, text-1G, all else equal):
-// two parts 0.996 ms per decode, four parts 1.012 ms - the write walk gains (wait stalls down, issue slots 59 -> 68 %) what
-// the count walk loses to recording three boundaries per chunk instead of one (four reconvergence points per chunk).
-#ifndef ET_WRITE_CHAINS
-#define ET_WRITE_CHAINS 2
-#endif
-// What the count walk records for the write walk per chunk: 18 bits per boundary.
-#if ET_WRITE_CHAINS == 2
+// What the count walk records for the write walk per chunk: where its second part begins (18 bits, et_lanes.inc).
 typedef uint32_t mid_t;
-#else
-typedef uint64_t mid_t;
-#endif
 
 constexpr uint32_t kMaxStates = 16;                  // most entries of a chunk's transfer function (longest code of such a dictionary)
 constexpr uint32_t kSegChunks = 16, kSegThreads = 256;  // transfer functions: chunks per composing thread, threads per block
@@ -121,8 +111,7 @@ inline DecodeLayout decode_layout(void *base, uint64_t n, bool lanes, uint32_t t
 }
 
 // The pack's scratch for num_tiles tiles of 4096 symbols.  The wide kernel uses one slot per tile; the lane-run path
-// one per region of 2048 symbols (two per tile, and pass A's slabs may touch two more).  The single pass keeps its
-// look-back descriptors where the two-pass path keeps run_bits: neither uses the other's.  The arrays follow each other at
+// one per region of 2048 symbols (two per tile, and pass A's slabs may touch two more).  The arrays follow each other at
 // their elements' alignment (16 bytes for ticket, tile_state and run_bits): MEASURED (text-1G, B200 at 1000 W), putting
 // every array on a 128-byte boundary made the pack 2 % slower (0.809 -> 0.826 ms) with the same kernels.
 struct PackLayout {
@@ -133,7 +122,6 @@ struct PackLayout {
     uint32_t *tile_bits = nullptr;               // [slots] two passes: bits of the earlier regions of the same group
     unsigned long long *group_prefix = nullptr;  // [(slots + 7) / 8] two passes: bits before each group
     uint16_t *run_bits = nullptr;                // [32 * slots] two passes: bits of every run of 64 symbols
-    unsigned long long *tile_desc = nullptr;     // [slots] single pass: look-back descriptors
     size_t bytes = 0;
 };
 
@@ -147,10 +135,8 @@ inline PackLayout pack_layout(void *base, uint32_t num_tiles) {
     L.tile_bits = c.take<uint32_t>(slots, 4);
     L.seam_head = c.take<uint8_t>(slots, 1);
     L.seam_tail = c.take<uint8_t>(slots, 1);
-    Carve single = c;
-    L.tile_desc = single.take<unsigned long long>(slots, 16);
     L.run_bits = c.take<uint16_t>(slots * 32, 16);
-    L.bytes = c.bytes > single.bytes ? c.bytes : single.bytes;
+    L.bytes = c.bytes;
     return L;
 }
 

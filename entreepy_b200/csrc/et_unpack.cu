@@ -981,7 +981,6 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
     // count walk: one CTA per SM, as many warps as images fit beside the tables
     uint32_t sync_warps = ((uint32_t)max_smem - kSyncTableBytes) / kImgBytes;
     if (sync_warps > kMaxLaneWarps) sync_warps = kMaxLaneWarps;
-    if (tune.sync_warps > 0 && (uint32_t)tune.sync_warps < sync_warps) sync_warps = (uint32_t)tune.sync_warps;
     if (sync_warps > 4) sync_warps &= ~3u;  // the same number of warps on each of the SM's four schedulers: they share the regions evenly
     // a stream with fewer regions than the GPU has warps for: a few warps on every SM rather than full CTAs on a few SMs
     auto spread = [&](uint32_t warps_max) {
@@ -1025,7 +1024,7 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
         region_sum_kernel<<<n_groups, 1024, 0, stream>>>(a, n_regions);
         chunk_scan_kernel<<<1, 1024, 0, stream>>>(a, a.group_prefix, n_groups);
         region_apply_kernel<<<n_groups, 1024, 0, stream>>>(a, n_regions);
-        const uint32_t write_warps = spread(tune.write_warps > 0 ? (uint32_t)tune.write_warps : 16u);
+        const uint32_t write_warps = spread(16u);
         const uint32_t write_blocks = (n_regions + write_warps - 1) / write_warps;
         region_write_kernel<<<write_blocks < (uint32_t)num_sms ? write_blocks : (uint32_t)num_sms, 512, max_smem, stream>>>(
             a, n_regions, (uint32_t)max_smem, write_warps);

@@ -116,12 +116,9 @@ ET_API uint32_t et_ctx_last_decode_rounds(const et_ctx *ctx);
  * variables ET_LANE_MIN_BYTES and ET_DEBUG_LANES seed the first two when the context is created. */
 #define ET_TUNE_LANE_MIN_BYTES 1 /* bodies of at least this many bytes take the lane-interleaved decoder; -1 = default */
 #define ET_TUNE_DEBUG 2          /* bit 0: lane decoder timings per decode on stderr; bit 1: host time of the phases of a sharded call (rank 0) */
-#define ET_TUNE_SYNC_WARPS 3     /* warps per CTA of the decoder's count walk; 0 = as many as fit */
 #define ET_TUNE_NO_TRANSFER 5     /* non-zero: slowly synchronising codes are decoded with repair rounds (round 1's way) instead of
                                      the scan of per-chunk transfer functions */
-#define ET_TUNE_WRITE_WARPS 6     /* warps per CTA of the decoder's write walk; 0 = as many as fit */
-#define ET_TUNE_PACK_SINGLE_PASS 4 /* non-zero: the encoder packs in one pass over the text (decoupled look-back over tile
-                                     descriptors) instead of two (run totals, then pack); measured slower on B200, kept selectable */
+/* Keys 3, 4 and 6 are retired (they selected measured-and-rejected kernel variants) and must not be reused. */
 ET_API int et_ctx_set_tuning(et_ctx *ctx, int key, long long value);
 
 /* Pinned host memory for full-rate host<->device copies in et_encode/et_decode. */

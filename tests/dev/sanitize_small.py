@@ -31,16 +31,9 @@ with et.Codec(0) as c:
     assert enc.tobytes() == want
     k, dec = c.decode(enc[4:m])
     assert dec.tobytes() == oracle.decode(want[4:], data.size).tobytes()
-    # slowly synchronising code (transfer functions), single-pass pack, a shard with an unknown head
-    from entreepy_b200 import _abi
-
+    # slowly synchronising code (transfer functions)
     data = rng.integers(1, 256, 150001, dtype=np.uint8)
     m, enc = c.encode(data, et.EncodeFlags(write_output=True, no_scratch_limit=True))
     k, dec = c.decode(enc[4:m])
     assert k == data.size and dec.tobytes() == data.tobytes()
-    c.set_tuning(_abi.TUNE_PACK_SINGLE_PASS, 1)
-    data = host[:100003]
-    m, enc = c.encode(data, et.EncodeFlags(write_output=True, no_scratch_limit=True))
-    assert enc.tobytes() == oracle.encode(data, cap=9000 + 5 * data.size).tobytes()
-    c.set_tuning(_abi.TUNE_PACK_SINGLE_PASS, 0)
 print("sanitize_small ok")

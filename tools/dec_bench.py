@@ -27,14 +27,8 @@ else:
     w = [0] + [1] * 255
 thr = synth.thresholds_from_weights(w)
 c = et.Codec(0)
-if os.environ.get("ET_WRITE_WARPS"):
-    c.set_tuning(et._abi.TUNE_WRITE_WARPS, int(os.environ["ET_WRITE_WARPS"]))
-if os.environ.get("ET_SYNC_WARPS"):
-    c.set_tuning(et._abi.TUNE_SYNC_WARPS, int(os.environ["ET_SYNC_WARPS"]))
 if os.environ.get("ET_LANE_MIN_BYTES"):
     c.set_tuning(et._abi.TUNE_LANE_MIN_BYTES, int(os.environ["ET_LANE_MIN_BYTES"]))
-if os.environ.get("ET_PACK_SINGLE_PASS"):
-    c.set_tuning(et._abi.TUNE_PACK_SINGLE_PASS, 1)
 dev = torch.empty(n, dtype=torch.uint8, device="cuda")
 c.synth_dev(dev.data_ptr(), n, synth.SEED, 0, thr)
 enc = torch.empty(n + n // 8 + 16384, dtype=torch.uint8, device="cuda")
