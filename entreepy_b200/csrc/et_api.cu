@@ -57,6 +57,8 @@ struct et_ctx {
     uint32_t last_decode_rounds = 0;  // passes over the chunk entries in the last decode (2 = guesses + one repair round sufficed)
     UnpackTuning tune;                // device properties + et_ctx_set_tuning() knobs
     UnpackTrie *trie = nullptr;       // host scratch of the dictionary parser (80 KB: not on the stack)
+    uint8_t *h_batch = nullptr;       // pinned mirror of a batch group's scratch (et_batch.inc), grown on demand
+    size_t h_batch_cap = 0;
     uint32_t fixed_len = 0;           // the uploaded decoder tables are a complete code whose codes all have this length (0: not so)
     char err[512] = {0};
 };
@@ -288,6 +290,7 @@ extern "C" void et_ctx_destroy(et_ctx *ctx) {
     if (ctx->d_scratch) cudaFree(ctx->d_scratch);
     if (ctx->d_small) cudaFree(ctx->d_small);
     if (ctx->h_small) cudaFreeHost(ctx->h_small);
+    if (ctx->h_batch) cudaFreeHost(ctx->h_batch);
     if (ctx->d_in) cudaFree(ctx->d_in);
     if (ctx->d_out) cudaFree(ctx->d_out);
     for (auto &e : ctx->ev)
@@ -488,9 +491,9 @@ extern "C" int et_pack_shard_dev(et_ctx *ctx, const void *d_in, size_t n, const 
 // ====================================================================== decode
 namespace {
 
-// The dictionary's trie goes up; the decoder's tables are derived from it on the device (launch_build_tables).
-// validate: ET_FLAG_VALIDATE was passed.
-int upload_unpack_tables(et_ctx *ctx, const et_dictionary &dict, cudaStream_t s, bool validate = false) {
+// The dictionary's trie into ctx->trie, with ET_FLAG_VALIDATE's checks when validate.  *fixed_len (on success): the length of
+// every code when they form a complete code of one length, else 0.
+int make_trie(et_ctx *ctx, const et_dictionary &dict, bool validate, uint32_t *fixed_len) {
     UnpackTrie *t = ctx->trie;
     int rc = make_unpack_trie(dict, t);
     if (rc == ET_OK && validate && !t->prefix_free) rc = ET_ERR_CORRUPT;
@@ -501,13 +504,27 @@ int upload_unpack_tables(et_ctx *ctx, const et_dictionary &dict, cudaStream_t s,
                              : why_incomplete        ? "dictionary is not a complete code (Kraft sum != 1)"
                                                      : "dictionary is not a prefix code");
     }
-    ctx->fixed_len = (t->complete && t->prefix_free && dict.min_length == dict.max_length) ? dict.max_length : 0u;
+    *fixed_len = (t->complete && t->prefix_free && dict.min_length == dict.max_length) ? dict.max_length : 0u;
+    return ET_OK;
+}
+
+// The dictionary's trie goes up; the decoder's tables are derived from it on the device (launch_build_tables).
+// validate: ET_FLAG_VALIDATE was passed.
+int upload_unpack_tables(et_ctx *ctx, const et_dictionary &dict, cudaStream_t s, bool validate = false) {
+    const int rc = make_trie(ctx, dict, validate, &ctx->fixed_len);
+    if (rc != ET_OK) return rc;
+    UnpackTrie *t = ctx->trie;
     std::memcpy(ctx->h_small->nodes, t->nodes, (size_t)t->n_nodes * 4);
     ET_CUDA(ctx, cudaMemcpyAsync(ctx->d_small->nodes, ctx->h_small->nodes, (size_t)t->n_nodes * 4, cudaMemcpyHostToDevice, s));
     int launches = 0;
     ET_CUDA(ctx, launch_build_tables(ctx->d_small->nodes, ctx->d_small->lut, ctx->d_small->slots, ctx->d_small->table_work, s, &launches));
     ctx->launches += (uint64_t)launches;
     return ET_OK;
+}
+
+// Bit offsets at which a chunk can be entered, for codes that synchronise slowly (lengths within 2 bits of each other); else 0.
+uint32_t transfer_states_of(const et_dictionary &dict) {
+    return (dict.max_length - dict.min_length <= 2 && dict.max_length <= 16) ? dict.max_length : 0u;
 }
 
 // Decode the part of a device-resident body that `g` describes: min(symbols found, max_symbols) bytes to d_out.
@@ -521,7 +538,7 @@ int unpack_dev(et_ctx *ctx, const UnpackGeometry &g, const et_dictionary &dict, 
     if (tm) tm->mark(2);
 
     const uint32_t chunk_bytes = unpack_chunk_bytes(g, ctx->tune, dict.min_length, dict.max_length);
-    const uint32_t transfer_states = (dict.max_length - dict.min_length <= 2 && dict.max_length <= 16) ? dict.max_length : 0u;
+    const uint32_t transfer_states = transfer_states_of(dict);
     rc = ensure_scratch(ctx, unpack_scratch_bytes(g, chunk_bytes, transfer_states));
     if (rc != ET_OK) return rc;
     const uint32_t *d_clut = ctx->d_small->lut;
@@ -757,3 +774,4 @@ extern "C" int et_synth_dev(et_ctx *ctx, void *d_out, size_t n, uint64_t seed, u
 }
 
 #include "et_shard.inc"
+#include "et_batch.inc"

@@ -98,6 +98,34 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
 cudaError_t launch_build_tables(const uint32_t *d_nodes, uint32_t *d_clut, uint16_t *d_slots, uint32_t *d_work, cudaStream_t stream,
                                 int *launches);
 
+// ---------------------------------------------------------------- batched decode (et_batch.inc)
+// Whether launch_unpack decodes this stream with the per-thread chunk kernels and no transfer functions, the only path
+// the batch kernels implement; *n_chunks = its chunks.
+bool batch_takes(const UnpackGeometry &g, uint32_t chunk_bytes, uint32_t transfer_states, uint32_t fixed_len, const UnpackTuning &tune,
+                 uint32_t *n_chunks);
+// One stream of a batch group on that path: its place in the group's scratch (BatchLayout L, device addresses).
+struct BatchStream {
+    UnpackGeometry g;
+    uint32_t n_chunks, chunk_bytes, fixed_len;
+    uint32_t node_off;      // its trie: L.nodes + node_off
+    uint64_t first_chunk;   // its chunks in L.count / start_off / exit_off
+    uint32_t first_tile;    // its tiles in L.tiles and L.tile_sums
+    uint8_t *out;
+    uint64_t max_symbols;
+};
+size_t batch_args_bytes();
+// Writes the decoder's arguments for stream j of the group to dst (host memory, batch_args_bytes() bytes).
+void batch_fill_args(void *dst, const BatchLayout &L, uint32_t j, const BatchStream &s);
+// Copies the first min(n, kBatchHeadBytes) bytes of every L.sources[i] to L.heads + i * kBatchHeadBytes.
+cudaError_t launch_batch_heads(const BatchLayout &L, uint32_t items, cudaStream_t stream, int *launches);
+// Every stream's clut | wlut and slots from its trie (one launch of each table kernel; L.work cleared by the caller).
+cudaError_t launch_batch_tables(const BatchLayout &L, uint32_t items, cudaStream_t stream, int *launches);
+// Decodes the group (args and tiles uploaded, tables built, status cleared) as launch_unpack's per-thread path decodes
+// one stream.  Blocks on the stream; on return *h_status (pinned) holds status .. item_status (BatchLayout::status_bytes).
+// settle_first: a stream with long chunks synchronises slowly, so the entries are settled before the first write walk.
+cudaError_t launch_unpack_batch(const BatchLayout &L, uint32_t items, uint32_t n_tiles, uint64_t n_chunks, bool settle_first,
+                                BatchStatus *h_status, cudaStream_t stream, int *launches, uint32_t *rounds_out);
+
 // ---------------------------------------------------------------- synthetic input generator
 cudaError_t launch_synth(uint8_t *d_out, size_t n, uint64_t seed, uint64_t first_index, const uint32_t *d_thresholds,
                          cudaStream_t stream);

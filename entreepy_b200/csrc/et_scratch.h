@@ -5,6 +5,8 @@
 #include <cstddef>
 #include <cstdint>
 
+#include "et_internal.h"
+
 namespace et {
 
 constexpr int kChunkThreads = 256;  // chunks per CTA of the per-thread decoder
@@ -136,6 +138,83 @@ inline PackLayout pack_layout(void *base, uint32_t num_tiles) {
     L.seam_head = c.take<uint8_t>(slots, 1);
     L.seam_tail = c.take<uint8_t>(slots, 1);
     L.run_bits = c.take<uint16_t>(slots * 32, 16);
+    L.bytes = c.bytes;
+    return L;
+}
+
+// ---------------------------------------------------------------- batched decode (et_decode_batch_dev)
+// A batch is decoded in groups of streams; a group's tables and chunk arrays share one scratch block.
+constexpr uint32_t kBatchGroupItems = 512;           // streams per group: bounds the per-stream tables (48 KB each)
+constexpr uint64_t kBatchGroupBytes = 256ull << 20;  // stream bytes per group (a longer stream is a group of its own): bounds the chunk arrays
+constexpr size_t kBatchHeadBytes = 4096;             // front of a stream the host parses the dictionary from, as et_decode_dev does
+constexpr uint32_t kBatchWorkWords = 32;             // per stream: slot counter and slot windows of the table build
+constexpr size_t kBatchSlots = kLutSize + (kMaxSubTables << kSubBits);  // per stream: marker-window slots, second-level tables
+
+struct BatchSource {  // the front of a stream: p[0, min(n, kBatchHeadBytes)) is gathered for the host
+    const uint8_t *p;
+    uint64_t n;
+};
+struct BatchTile {  // kChunkThreads chunks of one stream, from its chunk `first`
+    uint32_t item, first;
+};
+struct BatchItemStatus {
+    unsigned long long total;  // symbols found
+    uint32_t error_flags;      // kErrInvalidCode
+    uint32_t changed;          // the final check found a chunk whose entry was not its left neighbour's exit
+};
+struct BatchStatus {
+    uint32_t changed;        // some stream's entries moved (the sync rounds, the final check)
+    uint32_t entry_exit[2];  // written by the scan, not used
+    uint32_t pad;
+};
+
+// The scratch of one group: `items` streams on the per-thread chunk path with `tiles` tiles, `chunks` chunks and
+// `node_words` words of tries in all.  The arrays come in four runs: cleared before the group (status .. work), the
+// heads (sources, heads), uploaded with one copy (args .. nodes), device only.  A pinned host buffer of host_bytes
+// carved the same way mirrors the first three; the host reads back status .. item_status with one copy.
+struct BatchLayout {
+    BatchStatus *status = nullptr;           // [1]
+    BatchItemStatus *item_status = nullptr;  // [items]
+    uint32_t *work = nullptr;                // [items * kBatchWorkWords]
+    BatchSource *sources = nullptr;          // [items]
+    uint8_t *heads = nullptr;                // [items * kBatchHeadBytes]
+    uint8_t *args = nullptr;                 // [items * args_bytes] the decoder's arguments per stream
+    BatchTile *tiles = nullptr;              // [tiles]
+    uint32_t *nodes = nullptr;               // [node_words] every stream's trie
+    uint32_t *lut = nullptr;                 // [items * 2 * kLutSize] clut | wlut per stream
+    uint16_t *slots = nullptr;               // [items * kBatchSlots]
+    unsigned long long *tile_sums = nullptr; // [tiles + 1] symbols per tile, scanned in place; [tiles] = the group's total
+    uint32_t *count = nullptr;               // [chunks]
+    uint16_t *start_off = nullptr;           // [chunks]
+    uint16_t *exit_off = nullptr;            // [chunks]
+    size_t clear_bytes = 0;                  // status .. work, from the start of the block
+    size_t status_bytes = 0;                 // status .. item_status
+    size_t upload_begin = 0, upload_end = 0; // args .. nodes
+    size_t host_bytes = 0;                   // status .. nodes
+    size_t bytes = 0;
+};
+
+inline BatchLayout batch_layout(void *base, uint32_t items, size_t args_bytes, uint64_t tiles, uint64_t node_words, uint64_t chunks) {
+    BatchLayout L;
+    Carve c{static_cast<uint8_t *>(base)};
+    L.status = c.take<BatchStatus>(1);
+    L.item_status = c.take<BatchItemStatus>(items);
+    L.status_bytes = c.bytes;
+    L.work = c.take<uint32_t>((size_t)items * kBatchWorkWords);
+    L.clear_bytes = c.bytes;
+    L.sources = c.take<BatchSource>(items);
+    L.heads = c.take<uint8_t>((size_t)items * kBatchHeadBytes);
+    L.args = c.take<uint8_t>((size_t)items * args_bytes);
+    L.upload_begin = c.bytes - (size_t)items * args_bytes;
+    L.tiles = c.take<BatchTile>(tiles);
+    L.nodes = c.take<uint32_t>(node_words);
+    L.upload_end = L.host_bytes = c.bytes;
+    L.lut = c.take<uint32_t>((size_t)items * 2 * kLutSize);
+    L.slots = c.take<uint16_t>((size_t)items * kBatchSlots);
+    L.tile_sums = c.take<unsigned long long>(tiles + 1);
+    L.count = c.take<uint32_t>(chunks);
+    L.start_off = c.take<uint16_t>(chunks);
+    L.exit_off = c.take<uint16_t>(chunks);
     L.bytes = c.bytes;
     return L;
 }

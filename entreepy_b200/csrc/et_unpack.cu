@@ -31,6 +31,7 @@
 // so the walkers are written for instruction count.
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 
 #include "et_device.cuh"
 #include "et_kernels.cuh"
@@ -329,7 +330,9 @@ struct WordReader {
 // symbols at out[o..) while o < max_symbols.
 // clut / wlut: the first-level tables to read - the global ones (a.clut, a.wlut) or a copy in shared memory where the
 // caller has one (a walk through L2-resident tables costs ~10x the latency per symbol).
-template <bool WRITE>
+// BATCH: the copy the batch kernels call.  A separate copy leaves what the compiler derives from the single-stream
+// kernels' calls (their shared tables) as it was, and with it their code.
+template <bool WRITE, bool BATCH = false>
 __device__ __noinline__ uint64_t walk_generic(const DecArgs &a, uint64_t pos, uint64_t own_end, uint64_t hard_end,
                                               uint32_t *count, uint64_t o, uint32_t *bad, const uint32_t *clut = nullptr,
                                               const uint32_t *wlut = nullptr) {
@@ -456,6 +459,7 @@ __device__ __forceinline__ uint32_t count_chunk_fast(const DecArgs &a, const Chu
 }
 
 // The count walk of chunk c from `start` (known: a proven boundary; else a guess, and the walk begins 128 bits early).
+template <bool BATCH = false>
 __device__ __forceinline__ void sync_chunk(const DecArgs &a, uint32_t c, uint32_t start, bool known, const uint32_t *clut_sh) {
     const Chunk k = chunk_of(a, c);
     uint32_t cnt = 0, entry = start, exit_bits = 0;
@@ -467,11 +471,11 @@ __device__ __forceinline__ void sync_chunk(const DecArgs &a, uint32_t c, uint32_
         uint64_t pos = k.begin + start;
         uint32_t bad = 0, dummy = 0;
         if (!known && k.begin >= a.byte_lo * 8 + 128) {  // same run-up as the fast path
-            pos = walk_generic<false>(a, k.begin - 128, k.begin, a.end_bit, &dummy, 0, &bad, clut_sh);
+            pos = walk_generic<false, BATCH>(a, k.begin - 128, k.begin, a.end_bit, &dummy, 0, &bad, clut_sh);
             if (pos < k.begin) pos = k.begin;
         }
         entry = (uint32_t)(pos - k.begin);
-        if (pos < k.end) pos = walk_generic<false>(a, pos, k.end, a.end_bit, &cnt, 0, &bad, clut_sh);
+        if (pos < k.end) pos = walk_generic<false, BATCH>(a, pos, k.end, a.end_bit, &cnt, 0, &bad, clut_sh);
         exit_bits = pos > k.end ? (uint32_t)(pos - k.end) : 0u;
     }
     a.start_off[c] = (uint16_t)entry;
@@ -761,10 +765,10 @@ __global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const Dec
 // The host parses the dictionary into a trie (a few hundred nodes, microseconds) and uploads only that; the lookup tables
 // every decoder kernel reads (clut, wlut, marker slots, second-level tables: layouts in et_internal.h) are derived from
 // it here, one thread per 12-bit window - without 80 KB of host table building and upload in front of every decode.
-__global__ void __launch_bounds__(256) build_tables_kernel(const uint32_t *__restrict__ nodes, uint32_t *__restrict__ clut,
-                                                           uint32_t *__restrict__ wlut, uint16_t *__restrict__ slots,
-                                                           uint32_t *__restrict__ slot_count, uint32_t *__restrict__ slot_window) {
-    const uint32_t w = blockIdx.x * 256 + threadIdx.x;
+// Window w of the first-level tables, and a slot for it when it is a proper prefix of longer codes.
+__device__ __forceinline__ void build_table_entry(uint32_t w, const uint32_t *__restrict__ nodes, uint32_t *__restrict__ clut,
+                                                  uint32_t *__restrict__ wlut, uint16_t *__restrict__ slots,
+                                                  uint32_t *__restrict__ slot_count, uint32_t *__restrict__ slot_window) {
     if (w >= (uint32_t)kLutSize) return;
     uint32_t node = 0, pos = 0, cnt = 0, len0 = 0, len01 = 0, sym0 = 0, sym1 = 0;
     bool dead = false;  // ran into a bit pattern that is no code
@@ -804,10 +808,15 @@ __global__ void __launch_bounds__(256) build_tables_kernel(const uint32_t *__res
     }
     slots[w] = slot;
 }
+__global__ void __launch_bounds__(256) build_tables_kernel(const uint32_t *__restrict__ nodes, uint32_t *__restrict__ clut,
+                                                           uint32_t *__restrict__ wlut, uint16_t *__restrict__ slots,
+                                                           uint32_t *__restrict__ slot_count, uint32_t *__restrict__ slot_window) {
+    build_table_entry(blockIdx.x * 256 + threadIdx.x, nodes, clut, wlut, slots, slot_count, slot_window);
+}
 // sub[slot][next 8 bits] = symbol | length << 8 for codes of 13..20 bits behind a marker window, 0 otherwise.
-__global__ void __launch_bounds__(256) build_sub_tables_kernel(const uint32_t *__restrict__ nodes, uint16_t *__restrict__ slots,
-                                                               const uint32_t *__restrict__ slot_count, const uint32_t *__restrict__ slot_window) {
-    const uint32_t slot = blockIdx.x, x = threadIdx.x;  // one block per slot, one thread per 8-bit continuation
+__device__ __forceinline__ void build_sub_table_entry(uint32_t slot, uint32_t x, const uint32_t *__restrict__ nodes,
+                                                      uint16_t *__restrict__ slots, const uint32_t *__restrict__ slot_count,
+                                                      const uint32_t *__restrict__ slot_window) {
     uint16_t entry = 0;
     if (slot < min(*slot_count, kMaxSubTables)) {
         uint32_t node = slot_window[slot] >> 16;
@@ -822,6 +831,177 @@ __global__ void __launch_bounds__(256) build_sub_tables_kernel(const uint32_t *_
         }
     }
     slots[kLutSize + (slot << kSubBits) + x] = entry;
+}
+__global__ void __launch_bounds__(256) build_sub_tables_kernel(const uint32_t *__restrict__ nodes, uint16_t *__restrict__ slots,
+                                                               const uint32_t *__restrict__ slot_count, const uint32_t *__restrict__ slot_window) {
+    build_sub_table_entry(blockIdx.x, threadIdx.x, nodes, slots, slot_count, slot_window);  // one block per slot, one thread per 8-bit continuation
+}
+
+// ------------------------------------------------------------------ batched decode: many streams per launch (et_batch.inc)
+// A CTA decodes one tile: kChunkThreads chunks of one stream (tiles never cross streams).  It copies that stream's DecArgs
+// into shared memory and runs the walks of the per-thread kernels above unchanged, with chunk indices local to the stream,
+// so chunk_of and every edge case (ragged ends, unaligned bodies, fixed_len entries) behave as for a single stream.
+__device__ __forceinline__ BatchTile load_tile(DecArgs &dst, const DecArgs *__restrict__ args, const BatchTile *__restrict__ tiles,
+                                               uint32_t t) {
+    static_assert(sizeof(DecArgs) % 8 == 0, "DecArgs is copied in 8-byte words");
+    const BatchTile tile = tiles[t];
+    const unsigned long long *src = reinterpret_cast<const unsigned long long *>(args + tile.item);
+    unsigned long long *d = reinterpret_cast<unsigned long long *>(&dst);
+    for (uint32_t i = threadIdx.x; i < sizeof(DecArgs) / 8; i += blockDim.x) d[i] = src[i];
+    __syncthreads();
+    return tile;
+}
+
+// chunk_sync_kernel over tiles; a walk of a later round raises the group's flag.  Five CTAs per SM (48 registers), where
+// chunk_sync_kernel has six: its arguments are constant-bank operands, these are loaded from shared memory into registers,
+// and at 40 registers the count walk spilled its sector pair to local memory.
+__global__ void __launch_bounds__(kChunkThreads, 5) batch_sync_kernel(const DecArgs *args, const BatchTile *tiles, int round,
+                                                                      uint32_t *batch_changed) {
+    __shared__ __align__(16) uint32_t clut_sh[kLutSize];
+    __shared__ __align__(16) DecArgs a;
+    const uint32_t c = load_tile(a, args, tiles, blockIdx.x).first + threadIdx.x;
+    uint32_t start = 0;
+    bool work = c < a.n_chunks;
+    if (work && round != 0) {
+        if (c == 0) {
+            work = false;
+        } else {
+            start = a.exit_off[c - 1];
+            work = start != a.start_off[c];
+        }
+    }
+    if (!__syncthreads_or(work)) return;  // later rounds touch only the chunks whose entry moved
+    for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) clut_sh[i] = a.clut[i];
+    __syncthreads();
+    if (!work) return;
+    if (round != 0) *batch_changed = 1u;
+    if (c == 0 && a.head_known) start = a.head_off;
+    bool known = round != 0 || (c == 0 && a.head_known);
+    if (a.fixed_len && round == 0) {  // entries in closed form (chunk_sync_kernel)
+        const uint64_t begin = chunk_of(a, c).begin, base = a.grid_bit + (a.head_known ? a.head_off : 0u);
+        if (begin > base) start = (uint32_t)((a.fixed_len - (begin - base) % a.fixed_len) % a.fixed_len);
+        known = true;
+    }
+    sync_chunk<true>(a, c, start, known, clut_sh);
+}
+
+// chunk_sum_kernel over tiles: the tile's symbols into its slot of the tile sums; a failed check raises the stream's
+// flag and the group's.
+__global__ void __launch_bounds__(kChunkThreads) batch_sum_kernel(const DecArgs *args, const BatchTile *tiles, uint32_t *batch_changed) {
+    __shared__ __align__(16) DecArgs a;
+    __shared__ uint32_t warp_sum[kChunkThreads / 32];
+    const BatchTile tile = load_tile(a, args, tiles, blockIdx.x);
+    const uint32_t c = tile.first + threadIdx.x;
+    uint32_t v = c < a.n_chunks ? a.count[c] : 0u;
+    if (c > 0 && c < a.n_chunks && a.start_off[c] != a.exit_off[c - 1]) {
+        *a.changed = 1u;
+        *batch_changed = 1u;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = v;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned long long s = 0;
+        for (int i = 0; i < kChunkThreads / 32; ++i) s += warp_sum[i];
+        a.block_prefix[tile.first / kChunkThreads] = s;
+    }
+}
+
+// chunk_write_kernel over tiles.  The tile sums of the whole group were scanned together: a stream's text starts at its
+// first tile's prefix, and its total is its share of the sums (written by its first tile).  Four CTAs per SM (56
+// registers): at five, as chunk_write_kernel, the arguments in registers pushed the walk into local memory.
+__global__ void __launch_bounds__(kChunkThreads, 4) batch_write_kernel(const DecArgs *args, const BatchTile *tiles) {
+    __shared__ __align__(16) uint32_t wlut_sh[kLutSize];
+    __shared__ __align__(16) uint32_t rings[(kChunkThreads / 32) * 16 * 32];  // per warp: 16 words x 32 lanes
+    __shared__ uint32_t warp_sum[kChunkThreads / 32];
+    __shared__ __align__(16) DecArgs a;
+    const BatchTile tile = load_tile(a, args, tiles, gridDim.x - 1u - blockIdx.x);  // last tiles first, as chunk_write_kernel
+    for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) wlut_sh[i] = a.wlut[i];
+
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t bid = tile.first / kChunkThreads;
+    const unsigned long long base = a.block_prefix[0];
+    if (bid == 0 && tid == 0) *a.total = a.block_prefix[(a.n_chunks + kChunkThreads - 1) / kChunkThreads] - base;
+    const uint32_t c = tile.first + tid;
+    const bool live = c < a.n_chunks;
+    const uint32_t cnt = live ? a.count[c] : 0u;
+    uint32_t incl = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t up = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= (uint32_t)d) incl += up;
+    }
+    if (lane == 31) warp_sum[warp] = incl;
+    __syncthreads();
+    uint32_t before = 0;
+    for (uint32_t q = 0; q < warp; ++q) before += warp_sum[q];
+    const unsigned long long o = a.block_prefix[bid] - base + before + (incl - cnt);
+    if (!live || cnt == 0 || o >= a.max_symbols) return;
+
+    const Chunk k = chunk_of(a, c);
+    const uint32_t start = a.start_off[c];
+    uint32_t bad = 0;
+    if ((k.interior || (k.walkable && start < 256u)) && o + cnt <= a.max_symbols) {
+        uint8_t *dst = a.out + o;
+        OutRing r;
+        r.ring_s = smem_addr(rings) + warp * 2048u + lane * 4u;
+        r.head_skip = (uint32_t)(reinterpret_cast<uintptr_t>(dst) & 31u);
+        r.gsector = dst - r.head_skip;
+        r.lo = r.hi = 0;
+        r.stored = 0;
+        const uint32_t head = r.head_skip;
+        uint32_t s = start | (head << 9);
+        const uint64_t pair0 = k.begin >> 8;
+        const uint32_t wlut_s = smem_addr(wlut_sh);
+        uint32_t w[5];
+        const uint32_t n_pieces = a.chunk_bytes >> 4;
+        Pair raw = load_pair_raw(a, pair0);
+        Pair cur = raw;
+#pragma unroll 1
+        for (uint32_t p = 0; p < n_pieces; ++p) {
+            if (!(p & 1u)) {
+                cur = swap_pair(raw);
+                if (p + 2 < n_pieces)
+                    raw = load_pair_raw(a, pair0 + (p >> 1) + 1);
+                else
+                    raw.a = __ldg(reinterpret_cast<const uint4 *>(a.body_aligned) + 2 * (pair0 + (p >> 1) + 1));
+                w[0] = cur.a.x; w[1] = cur.a.y; w[2] = cur.a.z; w[3] = cur.a.w; w[4] = cur.b.x;
+            } else {
+                w[0] = cur.b.x; w[1] = cur.b.y; w[2] = cur.b.z; w[3] = cur.b.w; w[4] = bswap32(raw.a.x);
+            }
+            s = write_piece(w, s, p + 1 == n_pieces, wlut_s, r, a.clut, a.wlut, a.nodes, &bad);
+        }
+        const uint32_t n_end = s >> 9;
+        if (n_end & 3u) sts_u32(ring_slot(r, n_end >> 2), r.hi >> (8u * (4u - (n_end & 3u))));
+        for (uint32_t kk = r.head_skip ? head : (n_end & ~31u); kk < n_end; ++kk)
+            r.gsector[kk & 31u] = (uint8_t)lds_u8(ring_slot(r, kk >> 2) + (kk & 3u));
+    } else {
+        uint32_t n = 0;
+        if (k.begin + start < k.end) walk_generic<true, true>(a, k.begin + start, k.end, a.end_bit, &n, o, &bad, nullptr, wlut_sh);
+    }
+    if (bad) atomicOr(a.error_flags, kErrInvalidCode);
+}
+
+// The tables of every stream of the group: blockIdx.y selects the stream.
+__global__ void __launch_bounds__(256) batch_tables_kernel(const DecArgs *__restrict__ args, uint32_t *__restrict__ work) {
+    const DecArgs &a = args[blockIdx.y];
+    uint32_t *wk = work + (size_t)blockIdx.y * kBatchWorkWords;
+    build_table_entry(blockIdx.x * 256 + threadIdx.x, a.nodes, const_cast<uint32_t *>(a.clut), const_cast<uint32_t *>(a.wlut),
+                      const_cast<uint16_t *>(a.slots), wk, wk + 2);
+}
+__global__ void __launch_bounds__(256) batch_sub_tables_kernel(const DecArgs *__restrict__ args, const uint32_t *__restrict__ work) {
+    const DecArgs &a = args[blockIdx.y];
+    const uint32_t *wk = work + (size_t)blockIdx.y * kBatchWorkWords;
+    build_sub_table_entry(blockIdx.x, threadIdx.x, a.nodes, const_cast<uint16_t *>(a.slots), wk, wk + 2);
+}
+
+// The front of every stream into one staging array, for one copy to the host (any alignment: byte loads).
+__global__ void __launch_bounds__(256) batch_heads_kernel(const BatchSource *__restrict__ sources, uint8_t *__restrict__ heads) {
+    const BatchSource src = sources[blockIdx.x];
+    const uint32_t n = (uint32_t)(src.n < kBatchHeadBytes ? src.n : kBatchHeadBytes);
+    uint8_t *dst = heads + (size_t)blockIdx.x * kBatchHeadBytes;
+    for (uint32_t i = threadIdx.x; i < n; i += 256) dst[i] = src.p[i];
 }
 
 #include "et_lanes.inc"
@@ -1082,6 +1262,28 @@ static cudaError_t launch_unpack_lanes(const DecArgs &a, uint32_t n_regions, con
     return cudaGetLastError();
 }
 
+// The fields of DecArgs that describe the stream; the others are zero.
+static DecArgs stream_args(const UnpackGeometry &g, uint32_t n, uint32_t chunk_bytes, uint32_t fixed_len) {
+    DecArgs a{};
+    a.body_aligned = g.body_aligned;
+    a.grid_bit = g.own_begin_bit / 256 * 256;  // chunks are whole 32-byte sectors
+    a.own_end_bit = g.own_end_bit;
+    a.end_bit = g.end_bit;
+    a.byte_lo = g.byte_lo;
+    a.byte_hi = g.byte_hi;
+    a.head_known = g.head_known ? 1u : 0u;
+    a.head_off = (uint32_t)(g.head_bit - a.grid_bit);
+    a.n_chunks = n;
+    a.chunk_bytes = chunk_bytes;
+    a.fixed_len = fixed_len;
+    return a;
+}
+
+// Whether the per-thread path decodes a stream of n chunks through transfer functions (tr_log2: decode_layout's).
+static bool takes_transfer(uint32_t tr_log2, uint32_t fixed_len, uint64_t n, const UnpackTuning &tune) {
+    return tr_log2 != 0 && !fixed_len && n > 1 && !tune.no_transfer;
+}
+
 cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const uint32_t *d_clut, const uint32_t *d_wlut,
                           const uint32_t *d_nodes, const uint16_t *d_slots, uint8_t *d_out, uint64_t max_symbols, void *scratch_base,
                           DecodeStatus *h_status, cudaStream_t stream, const UnpackTuning &tune, uint32_t fixed_len, uint32_t transfer_states,
@@ -1098,18 +1300,7 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
     }
     const uint32_t n = (uint32_t)n64;
     const uint32_t nb = (uint32_t)L.n_blocks;
-    DecArgs a;
-    a.body_aligned = g.body_aligned;
-    a.grid_bit = g.own_begin_bit / 256 * 256;  // chunks are whole 32-byte sectors
-    a.own_end_bit = g.own_end_bit;
-    a.end_bit = g.end_bit;
-    a.byte_lo = g.byte_lo;
-    a.byte_hi = g.byte_hi;
-    a.head_known = g.head_known ? 1u : 0u;
-    a.head_off = (uint32_t)(g.head_bit - a.grid_bit);
-    a.n_chunks = n;
-    a.chunk_bytes = chunk_bytes;
-    a.fixed_len = fixed_len;
+    DecArgs a = stream_args(g, n, chunk_bytes, fixed_len);
     a.clut = d_clut;
     a.wlut = d_wlut;
     a.nodes = d_nodes;
@@ -1147,7 +1338,7 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
     // chunk), the final check fused into the block sums, the write walk — and a single look at
     // the flag at the very end.  Only when that check failed (slowly synchronising codes) do
     // the fixpoint rounds run, and the sums and the write walk are repeated.
-    const bool transfer = L.tr_log2 != 0 && !fixed_len && n > 1 && !tune.no_transfer;
+    const bool transfer = takes_transfer(L.tr_log2, fixed_len, n, tune);
     uint32_t rounds = 2;
     if (transfer) {
         // slowly synchronising codes: the chunks' transfer functions and a scan instead of repair rounds
@@ -1213,6 +1404,103 @@ cudaError_t launch_unpack(const UnpackGeometry &g, uint32_t chunk_bytes, const u
         // the error flags the first write walk may have raised came from a wrong parse
         err = cudaMemsetAsync(a.error_flags, 0, 4, stream);
         if (err != cudaSuccess) return err;
+    }
+    if (rounds_out) *rounds_out = rounds;
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ batched decode (et_batch.inc)
+bool batch_takes(const UnpackGeometry &g, uint32_t chunk_bytes, uint32_t transfer_states, uint32_t fixed_len, const UnpackTuning &tune,
+                 uint32_t *n_chunks) {
+    const uint64_t n = chunk_count(g, chunk_bytes);
+    *n_chunks = (uint32_t)n;
+    return chunk_bytes != kLaneBytes && !takes_transfer(transfer_log2(transfer_states), fixed_len, n, tune);
+}
+
+size_t batch_args_bytes() { return sizeof(DecArgs); }
+
+void batch_fill_args(void *dst, const BatchLayout &L, uint32_t j, const BatchStream &s) {
+    DecArgs a = stream_args(s.g, s.n_chunks, s.chunk_bytes, s.fixed_len);
+    a.clut = L.lut + (size_t)j * 2 * kLutSize;
+    a.wlut = a.clut + kLutSize;
+    a.nodes = L.nodes + s.node_off;
+    a.slots = L.slots + (size_t)j * kBatchSlots;
+    a.error_flags = &L.item_status[j].error_flags;
+    a.total = &L.item_status[j].total;
+    a.changed = &L.item_status[j].changed;
+    a.block_prefix = L.tile_sums + s.first_tile;
+    a.count = L.count + s.first_chunk;
+    a.start_off = L.start_off + s.first_chunk;
+    a.exit_off = L.exit_off + s.first_chunk;
+    a.out = s.out;
+    a.max_symbols = s.max_symbols;
+    std::memcpy(dst, &a, sizeof a);
+}
+
+cudaError_t launch_batch_heads(const BatchLayout &L, uint32_t items, cudaStream_t stream, int *launches) {
+    batch_heads_kernel<<<items, 256, 0, stream>>>(L.sources, L.heads);
+    if (launches) *launches += 1;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_batch_tables(const BatchLayout &L, uint32_t items, cudaStream_t stream, int *launches) {
+    const DecArgs *args = reinterpret_cast<const DecArgs *>(L.args);
+    batch_tables_kernel<<<dim3(kLutSize / 256, items), 256, 0, stream>>>(args, L.work);
+    batch_sub_tables_kernel<<<dim3(kMaxSubTables, items), 1u << kSubBits, 0, stream>>>(args, L.work);
+    if (launches) *launches += 2;
+    return cudaGetLastError();
+}
+
+// launch_unpack's per-thread branch over the tiles of a group: sync 0 and 1, then sum, scan and write, and one look
+// at the status; fixpoint rounds only when an entry of some stream still moved.
+cudaError_t launch_unpack_batch(const BatchLayout &L, uint32_t items, uint32_t n_tiles, uint64_t n_chunks, bool settle_first,
+                                BatchStatus *h_status, cudaStream_t stream, int *launches, uint32_t *rounds_out) {
+    const DecArgs *args = reinterpret_cast<const DecArgs *>(L.args);
+    uint32_t *changed = &L.status->changed;
+    cudaError_t err;
+    if (rounds_out) *rounds_out = 0;
+    if (n_tiles == 0) {  // no stream has a chunk: the cleared status is the result
+        if ((err = cudaMemcpyAsync(h_status, L.status, L.status_bytes, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return err;
+        return cudaStreamSynchronize(stream);
+    }
+    batch_sync_kernel<<<n_tiles, kChunkThreads, 0, stream>>>(args, L.tiles, 0, changed);
+    batch_sync_kernel<<<n_tiles, kChunkThreads, 0, stream>>>(args, L.tiles, 1, changed);
+    if (launches) *launches += 2;
+    if ((err = cudaMemsetAsync(changed, 0, 4, stream)) != cudaSuccess) return err;
+    // the scan of the tile sums is chunk_scan_kernel's: the group's total lands behind the last tile
+    DecArgs scan{};
+    scan.total = L.tile_sums + n_tiles;
+    scan.entry_exit = L.status->entry_exit;
+    scan.start_off = L.start_off;
+    scan.exit_off = L.exit_off;
+    scan.n_chunks = (uint32_t)n_chunks;
+    uint32_t rounds = 2;
+    auto settle = [&]() -> cudaError_t {  // launch_unpack's fixpoint rounds, four per host visit
+        for (;;) {
+            for (int i = 0; i < 3; ++i) batch_sync_kernel<<<n_tiles, kChunkThreads, 0, stream>>>(args, L.tiles, (int)rounds + i, changed);
+            cudaError_t e = cudaMemsetAsync(changed, 0, 4, stream);
+            if (e != cudaSuccess) return e;
+            batch_sync_kernel<<<n_tiles, kChunkThreads, 0, stream>>>(args, L.tiles, (int)rounds + 3, changed);
+            rounds += 4;
+            if (launches) *launches += 4;
+            if ((e = cudaMemcpyAsync(&h_status->changed, changed, 4, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return e;
+            if ((e = cudaStreamSynchronize(stream)) != cudaSuccess) return e;
+            if (h_status->changed == 0) return cudaSuccess;
+            if (rounds > n_chunks + 8u) return cudaErrorUnknown;  // cannot happen: each round settles one more chunk
+        }
+    };
+    if (settle_first && (err = settle()) != cudaSuccess) return err;
+    for (;;) {
+        batch_sum_kernel<<<n_tiles, kChunkThreads, 0, stream>>>(args, L.tiles, changed);
+        chunk_scan_kernel<<<1, 1024, 0, stream>>>(scan, L.tile_sums, n_tiles);
+        batch_write_kernel<<<n_tiles, kChunkThreads, 0, stream>>>(args, L.tiles);
+        if (launches) *launches += 3;
+        if ((err = cudaMemcpyAsync(h_status, L.status, L.status_bytes, cudaMemcpyDeviceToHost, stream)) != cudaSuccess) return err;
+        if ((err = cudaStreamSynchronize(stream)) != cudaSuccess) return err;
+        if (h_status->changed == 0) break;
+        if ((err = settle()) != cudaSuccess) return err;
+        // the error flags (and check flags) of the first write walk came from a wrong parse
+        if ((err = cudaMemsetAsync(L.item_status, 0, (size_t)items * sizeof(BatchItemStatus), stream)) != cudaSuccess) return err;
     }
     if (rounds_out) *rounds_out = rounds;
     return cudaGetLastError();

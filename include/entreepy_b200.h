@@ -160,6 +160,27 @@ ET_API int et_encode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_out, s
 ET_API int et_decode_dev(et_ctx *ctx, const void *d_in_after_magic, size_t n, void *d_out, size_t cap, size_t *out_len,
                   uint32_t flags, void *stream);
 
+/* Batched device decode: many independent streams in one call, for workloads of many small .et objects, where a call
+ * per stream would spend its time on launches and host synchronisations.  Item i ends with the status, *out_len and
+ * d_out bytes that et_decode_dev(ctx, d_in, n, d_out, cap, &out_len, flags, stream) would give it, including every
+ * failure (corrupt dictionary or body, ET_FLAG_VALIDATE rejections, ET_ERR_NO_SPACE, truncated dictionaries, dry
+ * runs); a failing item does not affect the others.  Items may share d_in.  Returns ET_OK once every item has its
+ * status; fails only for invalid arguments (items == NULL with count > 0: ET_ERR_INVALID_ARG) or a CUDA error or
+ * allocation failure, whose status is then also written into every item not yet finished.  count == 0 is ET_OK.
+ * Streams that et_decode_dev decodes with the per-thread chunk kernels are decoded together, with a fixed number of
+ * launches per group of up to 512 streams; longer bodies (lane decoder) and slowly synchronising codes that take
+ * transfer functions are decoded one by one after them.  ET_FLAG_TIMING: et_ctx_last_stage_ms covers the whole call
+ * ([0] heads and parse, [1] tables, [2] decode kernels); et_ctx_last_decode_rounds is the largest over the batch. */
+typedef struct et_batch_item {
+    const void *d_in; /* file[4..] of one stream, device memory (any alignment) */
+    size_t n;
+    void *d_out;      /* device memory, any alignment */
+    size_t cap;
+    size_t out_len;   /* out */
+    int status;       /* out: et_status of this stream */
+} et_batch_item;
+ET_API int et_decode_batch_dev(et_ctx *ctx, et_batch_item *items, size_t count, uint32_t flags, void *stream);
+
 /* ------------------------------------------------------------------ sharded path (SURVEY §8e) */
 /* One .et stream across several GPUs: each rank owns a contiguous byte range of the text
  * (encode) or of the body (decode); the host exchanges only the 2 KiB histogram, one bit
