@@ -223,3 +223,68 @@ def test_launches_do_not_grow_with_the_batch(codec):
         assert codec.last_decode_rounds == 2
     # one group: 1 head gather, 2 table builds, sync 0 and 1, sum, scan, write
     assert counts == [8, 8], counts
+
+
+def _codes_3_to_7(rng, n):
+    """40 of 48 symbols equiprobable, 8 of them more frequent: code lengths 3..7, a spread too wide for transfer functions,
+    and still slow to synchronise (test_lane_decoder_repairs_wrong_guesses)."""
+    w = np.ones(48)
+    w[:8] = 9.0
+    return rng.choice(48, n, p=w / w.sum()).astype(np.uint8)
+
+
+def _batch_with_oracle(codec, inputs, rng):
+    """The oracle's streams of `inputs` at random offsets, none long enough for the lane decoder: the batch against single
+    calls, then every item against the oracle.  -> (streams, kernel launches of one more batch call, its rounds)."""
+    import torch
+
+    streams = [_stream(d) for d in inputs]
+    lane_min = torch.cuda.get_device_properties(0).multi_processor_count * 3 * 4224  # lane_path_min_bytes
+    for s in streams:
+        d = et.parse_header(s)
+        assert d.max_length - d.min_length <= 2 or len(s) - d.body_offset < lane_min
+    items = Items(streams, [d.size for d in inputs], [int(x) for x in rng.integers(0, 16, len(streams))],
+                  [int(x) for x in rng.integers(0, 16, len(streams))])
+    res, outs = _batch_matches_single(codec, items)
+    for k, data in enumerate(inputs):
+        assert res[k] == (_abi.OK, data.size) and items.text(outs, k, data.size) == data.tobytes(), k
+    again = items.outputs()
+    before = codec.kernel_launches
+    assert codec.decode_batch_dev(items.args(again)) == res
+    launches, rounds = codec.kernel_launches - before, codec.last_decode_rounds
+    torch.cuda.synchronize()
+    assert all(torch.equal(a, b) for a, b in zip(again, outs))
+    return streams, launches, rounds
+
+
+def test_batch_repair_rounds_of_slowly_synchronising_streams(codec):
+    # Streams whose guessed chunk entries are wrong and that stay in the batch: launch_unpack_batch runs its fixpoint
+    # rounds (settle) and a second write walk, and clears the item status before it.  With ET_TUNE_NO_TRANSFER, codes
+    # whose lengths are within 2 bits of each other (uniform bytes: 7 and 8 bits) are such streams; so may be a stream of
+    # 3..7-bit codes under any tuning.  A body long enough for 512-byte chunks settles before its first write walk
+    # (settle_first).  Launches per group: 8 (test_launches_do_not_grow_with_the_batch), 4 per host visit of the rounds,
+    # 3 for a second write walk.
+    import torch
+
+    rng = np.random.default_rng(41)
+    fixed = rng.permutation(np.repeat(rng.permutation(256)[:32].astype(np.uint8), 20_000))  # 5-bit codes: closed-form entries
+    d = et.parse_header(_stream(fixed))
+    assert d.min_length == d.max_length == 5
+    mixed = [_text(200_003, 7), _codes_3_to_7(rng, 1 << 20), _text(1_000_003, 8), fixed]
+    uniform = [rng.integers(1, 256, n, dtype=np.uint8) for n in (70_001, 300_007, 1_000_003, 4_000_037)]
+    big = rng.integers(1, 256, 48_000_017, dtype=np.uint8)
+    codec.set_tuning(_abi.TUNE_NO_TRANSFER, 1)
+    try:
+        # chunks of 256 bytes: a write walk, the rounds, a second write walk
+        _, launches, rounds = _batch_with_oracle(codec, uniform + mixed, rng)
+        assert rounds > 2 and launches > 11 and (launches - 11) % 4 == 0, (rounds, launches)
+        # unpack_chunk_bytes keeps 512-byte chunks once body / 512 x max_length >= SMs x 4096: the rounds, one write walk
+        streams, launches, rounds = _batch_with_oracle(codec, [big] + uniform[:2] + mixed, rng)
+        d = et.parse_header(streams[0])
+        assert (len(streams[0]) - d.body_offset) // 512 * d.max_length >= torch.cuda.get_device_properties(0).multi_processor_count * 4096
+        assert rounds > 2 and launches > 8 and (launches - 8) % 4 == 0, (rounds, launches)
+    finally:
+        codec.set_tuning(_abi.TUNE_NO_TRANSFER, 0)
+    # default tuning: the codes of 3..7 bits among streams that synchronise at once still need the rounds
+    _, launches, rounds = _batch_with_oracle(codec, mixed, rng)
+    assert rounds > 2 and launches > 11 and (launches - 11) % 4 == 0, (rounds, launches)

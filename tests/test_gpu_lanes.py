@@ -145,6 +145,71 @@ def test_lane_decoder_deepest_codes_anywhere(codec, lanes):
         assert m == text.size and out.tobytes() == text.tobytes(), depth
 
 
+def _marker_windows(lengths, codes):
+    """12-bit windows that are proper prefixes of longer codes.  The first kMaxSubTables (16) of them to ask get a
+    second-level table (build_table_entry); lookups behind the others walk the trie (code_slow, code_at_global)."""
+    return len({int(codes[s]) >> (int(lengths[s]) - 12) for s in range(256) if int(lengths[s]) > 12})
+
+
+def _many_windows_handmade(rng):
+    """A complete code of 252 symbols with 20 marker windows, behind which chains run to 21..32 bits: the prefixes 1, 01,
+    .., 0000001 (1..7 bits), then the 32 windows under 0000000: 12 of them are codes, 20 are markers."""
+    entries = [(k + 1, 1) for k in range(7)] + [(12, w) for w in range(20, 32)]
+    for w, depth in zip(range(20), [9] * 12 + [10, 10, 11, 12, 13, 14, 15, 20]):
+        entries += [(13 + j, (w << (j + 1)) | (((1 << j) - 1) << 1)) for j in range(depth)]  # j ones and a zero
+        entries.append((12 + depth, (w << depth) | ((1 << depth) - 1)))
+    assert sum(2.0 ** -length for length, _ in entries) == 1.0
+    lengths, codes = [0] * 256, [0] * 256
+    symbols = rng.permutation(256)[: len(entries)]
+    for s, (length, code) in zip(symbols, entries):
+        lengths[s], codes[s] = length, code
+    short = symbols[:7]
+    text = np.where(rng.random(1 << 21) < 0.8, short[np.minimum(rng.geometric(0.5, 1 << 21) - 1, 6)],
+                    rng.choice(symbols, 1 << 21)).astype(np.uint8)
+    return lengths, codes, text
+
+
+def test_lane_decoder_over_sixteen_marker_windows(codec, lanes):
+    # More marker windows than second-level tables: which windows get one follows atomicAdd order and may change from run
+    # to run; lookups behind the rest walk the trie, deep into it for the hand-made chains.  Every run, every path
+    # (lanes, default tuning, the batch call, shards) must read the oracle's text back.
+    import torch
+
+    from test_gpu_shards import _unpack_in_shards
+
+    rng = np.random.default_rng(16)
+    streams = []
+    for frequent, count in ((64, 16384), (16, 131072)):  # codes of 6..15 bits, 32 windows; 4..13 bits, 111 windows
+        counts = np.zeros(256, dtype=np.int64)
+        counts[:frequent], counts[frequent:255] = count, 16
+        data = np.repeat(np.arange(256, dtype=np.uint8), counts)
+        rng.shuffle(data)
+        codes, lengths = oracle.build_dictionary(counts.astype(np.uint64))
+        streams.append((_oracle_et(data)[4:], data, _marker_windows(lengths, codes)))
+    lengths, codes, text = _many_windows_handmade(rng)
+    stream = _handmade_stream(lengths, codes, text)
+    assert oracle.decode(stream, text.size).tobytes() == text.tobytes()
+    assert max(lengths) == 32 and min(length for length in lengths if length > 12) == 13
+    streams.append((stream, text, _marker_windows(lengths, codes)))
+    assert [(s[1].size, s[2]) for s in streams] == [(1_051_632, 32), (2_100_976, 111), (1 << 21, 20)]
+
+    for stream, data, _ in streams:
+        for run in range(3):
+            m, out = codec.decode(stream)
+            assert m == data.size and out.tobytes() == data.tobytes(), (data.size, run)
+    _unpack_in_shards(codec, streams[1][1], 3, expect_guess_right=False)
+    codec.set_tuning(et._abi.TUNE_LANE_MIN_BYTES, -1)
+    for stream, data, _ in streams:
+        m, out = codec.decode(stream)
+        assert m == data.size and out.tobytes() == data.tobytes(), data.size
+    ins = [torch.from_numpy(np.frombuffer(s, dtype=np.uint8).copy()).cuda() for s, _, _ in streams]
+    outs = [torch.zeros(d.size + 64, dtype=torch.uint8, device="cuda") for _, d, _ in streams]
+    res = codec.decode_batch_dev([(i.data_ptr(), i.numel(), o.data_ptr(), d.size) for i, o, (_, d, _) in zip(ins, outs, streams)])
+    for (_, data, _), o, r in zip(streams, outs, res):
+        assert r == (et._abi.OK, data.size), (data.size, r)
+        assert o[: data.size].cpu().numpy().tobytes() == data.tobytes() and int(o[data.size :].sum()) == 0, data.size
+
+
 def test_lane_decoder_repairs_wrong_guesses(codec, lanes):
     # 40 of 48 symbols equiprobable: most codes have 6 or 7 bits and a wrong parse survives for a long time, so
     # the run-up guesses are often wrong and the repair rounds have to settle the entries

@@ -96,20 +96,138 @@ def test_encode_text_sizes_and_alignments(codec, manifest):
         assert out[out_off : out_off + got].cpu().numpy().tobytes() == want, (off, n, out_off)
 
 
+def _chain_bytes(depth):
+    """Smallest text whose exact Fibonacci counts (synth.fibonacci_counts) make a chain of `depth`: one copy of each of
+    the two rarest symbols."""
+    f = [1, 1]
+    while len(f) < depth + 1:
+        f.append(f[-1] + f[-2])
+    return sum(f)
+
+
+def _encode_dev_counted(codec, d_in, n, d_out, cap):
+    """encode_dev -> (size, kernel launches it took)."""
+    before = codec.kernel_launches
+    size = codec.encode_dev(d_in, n, d_out, cap, _abi.FLAG_WRITE_OUTPUT | _abi.FLAG_NO_SCRATCH_LIMIT)
+    return size, codec.kernel_launches - before
+
+
+def _first_difference(got, want):
+    """None when the byte strings are equal, else (first differing index, len(got), len(want))."""
+    a, b = np.frombuffer(got, np.uint8), np.frombuffer(want, np.uint8)
+    if a.size == b.size and np.array_equal(a, b):
+        return None
+    m = min(a.size, b.size)
+    diff = np.flatnonzero(a[:m] != b[:m])
+    return (int(diff[0]) if diff.size else m, a.size, b.size)
+
+
+def _expected_size(counts, n):
+    cb = et.build_codebook(np.asarray(counts, dtype=np.uint64))
+    return len(et.write_header(cb, n)) + (cb.body_bits + 7) // 8
+
+
 def test_encode_wide_codes_fibonacci_depth_32_and_beyond(codec):
-    # depth 32 = deepest the reference represents faithfully (SURVEY §0.4); depth 34 exercises the
-    # truncated-code emission (encode.zig:311 shift is u5) which must still match bit for bit
-    rng = np.random.default_rng(9)
-    for depth in (27, 32, 34):
-        w = synth.fibonacci_weights(depth)
-        n = 1 << 22
-        data = synth.generate(n, synth.thresholds_from_weights(w), seed=depth)
-        # make sure every symbol occurs, rarest ones at least once, so the tree has full depth
-        data[: depth + 1] = np.arange(depth + 1, dtype=np.uint8)
+    # Exact Fibonacci counts make a chain whose longest code has `depth` bits (i.i.d. sampling from the same weights stops
+    # near 20 bits).  Depth 32 is the deepest code the narrow pack takes and the reference represents faithfully
+    # (SURVEY §0.4).  Past it pack_wide_kernel emits the reference's truncated codes (encode.zig:311 shifts by a u5),
+    # which must still match bit for bit.  Depth 38 is 166 MB: about 40 K tiles of look-back.
+    import torch
+
+    for depth in (32, 33, 34, 36, 38):
+        n = _chain_bytes(depth)
+        counts = synth.fibonacci_counts(n, depth)
+        assert int(oracle.build_dictionary(np.array(counts, dtype=np.uint64))[1].max()) == depth
+        dev = synth.shuffled_dev(counts, seed=depth)
+        size_want = _expected_size(counts, n)
+        out = torch.empty(size_want + 64, dtype=torch.uint8, device="cuda")
+        size, launches = _encode_dev_counted(codec, dev.data_ptr(), n, out.data_ptr(), out.numel())
+        # from launch_pack: histogram, pack_wide_kernel, seam_fixup_kernel | histogram, four narrow pack kernels, seam fix-up
+        assert launches == (3 if depth > 32 else 6), (depth, launches)
+        want = _oracle_et(dev.cpu().numpy())
+        assert size == size_want == len(want), (depth, size, size_want, len(want))
+        assert _first_difference(out[:size].cpu().numpy().tobytes(), want) is None, depth
+
+
+def test_encode_wide_codes_sizes_and_alignments(codec):
+    # Depth 33 on the wide path: the input at every 16-byte phase, last tiles of 1, 15, 16, 4095 and 4096 symbols, odd
+    # output offsets, guard bytes on both sides (zero, or stale bytes that must stay); then the host-buffer entry point,
+    # and the decoder, which refuses codes over 32 bits without writing anything.
+    import torch
+
+    n0 = _chain_bytes(33)
+    rng = np.random.default_rng(33)
+    core = np.repeat(np.arange(256, dtype=np.uint8), np.array(synth.fibonacci_counts(n0, 33), dtype=np.int64))
+    rng.shuffle(core)
+    # the pads only add copies of the two most frequent symbols (1- and 2-bit codes): a slice that holds the core keeps the chain
+    pad = 8192 + 32
+    top2 = np.array([32, 33], dtype=np.uint8)
+    host = np.concatenate([rng.choice(top2, pad), core, rng.choice(top2, pad)])
+    dev = torch.from_numpy(host).cuda()
+    assert dev.data_ptr() % 16 == 0
+    lasts, out_offs = (1, 15, 16, 4095, 4096), (0, 1, 3, 7, 9, 15, 16, 33)
+    for off in range(16):
+        last = lasts[off % len(lasts)]
+        n = pad + n0 + (last - off - (pad + n0)) % 4096  # the tiles cover bytes [0, off + n) of dev: the last holds `last`
+        assert (off + n - 1) % 4096 + 1 == last and off + n <= host.size
+        data = host[off : off + n]
         occ = oracle.histogram(data)
-        _, length = oracle.build_dictionary(occ)
-        n_out, out = codec.encode(data, _flags())
-        assert out.tobytes() == _oracle_et(data), (depth, int(length.max()))
+        assert int(oracle.build_dictionary(occ)[1].max()) == 33, off
+        want = _oracle_et(data)
+        assert len(want) == _expected_size(occ, n)
+        out_off, fill = out_offs[off % len(out_offs)], 0xA5 if off % 2 else 0
+        out = torch.full((out_off + len(want) + 64,), fill, dtype=torch.uint8, device="cuda")
+        size, launches = _encode_dev_counted(codec, dev.data_ptr() + off, n, out.data_ptr() + out_off, out.numel() - out_off)
+        assert size == len(want) and launches == 3, (off, n, size, launches)
+        got = out.cpu().numpy()
+        assert (got[:out_off] == fill).all() and (got[out_off + size :] == fill).all(), (off, n, out_off)
+        assert _first_difference(got[out_off : out_off + size].tobytes(), want) is None, (off, n, out_off)
+    # et_encode: host buffers, the input uploaded in slices
+    data = host[5 : 5 + pad + n0 + 4095]
+    assert int(oracle.build_dictionary(oracle.histogram(data))[1].max()) == 33
+    n_out, enc = codec.encode(data, _flags())
+    assert _first_difference(enc.tobytes(), _oracle_et(data)) is None
+    # et_decode_dev: the dictionary holds codes of 33 bits, which the reference's decoder cannot hold
+    src = torch.from_numpy(enc.copy()).cuda()
+    out = torch.full((data.size + 64,), 0xA5, dtype=torch.uint8, device="cuda")
+    with pytest.raises(et.EntreepyError) as e:
+        codec.decode_dev(src.data_ptr() + 4, n_out - 4, out.data_ptr(), data.size)
+    assert e.value.name == "Unsupported"
+    assert bool((out == 0xA5).all())
+
+
+def test_encode_wide_codes_dropped_symbol_zero_bit_tiles(codec):
+    # All 256 byte values: the most frequent one (symbol 33 of a depth-33 chain) gets no code (encode.zig:70).  A run of
+    # it longer than three tiles, starting inside an output byte, gives whole tiles of zero bits that begin and end in
+    # the same byte: seam_fixup_kernel merges the heads of a chain of tiles from the wide kernel's tile states.
+    import torch
+
+    counts = synth.fibonacci_counts(_chain_bytes(33), 33)[:34] + [200_000] * 222
+    assert sum(counts) == 59_330_351
+    base = synth.shuffled_dev(counts, seed=34).cpu().numpy()
+    _, length = oracle.build_dictionary(np.array(counts, dtype=np.uint64))
+    assert int(length.max()) == 33 and length[33] == 0
+    run, at = 20_000, 30_000_001
+    bit = int(length[base[:at]].sum(dtype=np.int64))
+    while at % 2 == 0 or bit % 8 == 0:  # an odd offset, and the run begins inside a byte of the body
+        bit += int(length[base[at]])
+        at += 1
+    host = np.concatenate([base[:at], np.full(run, 33, np.uint8), base[at:]])
+    occ = oracle.histogram(host)
+    _, length = oracle.build_dictionary(occ)
+    assert int((occ > 0).sum()) == 256 and int(length.max()) == 33 and length[33] == 0
+    in_off = 3
+    assert (in_off + at + run) // 4096 - (in_off + at + 4095) // 4096 >= 3  # whole tiles inside the run
+    buf = torch.zeros(host.size + 16, dtype=torch.uint8, device="cuda")
+    buf[in_off : in_off + host.size] = torch.from_numpy(host).cuda()
+    want = _oracle_et(host)
+    assert len(want) == _expected_size(occ, host.size)
+    out = torch.full((len(want) + 64,), 0xA5, dtype=torch.uint8, device="cuda")
+    size, launches = _encode_dev_counted(codec, buf.data_ptr() + in_off, host.size, out.data_ptr() + 1, out.numel() - 1)
+    assert size == len(want) and launches == 3, (size, launches)
+    got = out.cpu().numpy()
+    assert got[0] == 0xA5 and (got[1 + size :] == 0xA5).all()
+    assert _first_difference(got[1 : 1 + size].tobytes(), want) is None
 
 
 # ---------------------------------------------------------------- decode

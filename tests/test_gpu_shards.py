@@ -48,6 +48,44 @@ def _fib32():
     return data
 
 
+def _chain33():
+    """Exact Fibonacci counts at the smallest size for a chain of depth 33: two symbols with 33-bit codes, one copy each
+    (pack_wide_kernel)."""
+    counts = synth.fibonacci_counts(14_930_351, 33)
+    data = np.repeat(np.arange(256, dtype=np.uint8), counts)
+    np.random.default_rng(9).shuffle(data)
+    return data
+
+
+def _chain33_at_cuts(world):
+    """_chain33 with its 33-bit codes moved to the starts of ranks 1 and 2 of the sharded encoder: their heads cannot
+    price their first output byte (first_output_byte), so the ranks exchange the real bytes after the pack."""
+    data = _chain33()
+    _, length = oracle.build_dictionary(oracle.histogram(data))
+    starts = sharded.ShardPlan(data.size, world, 0).bounds[1:3]
+    for at, deep in zip(starts, np.flatnonzero(length[data] == 33)):
+        data[[at, deep]] = data[[deep, at]]
+    assert all(length[data[at]] == 33 for at in starts)
+    assert any(_boundaries(data)[at] % 8 for at in starts)  # a rank that starts inside a byte
+    return data
+
+
+def _dropped_run_at_cut(world):
+    """All 256 byte values, the most frequent (255) gets no code; a run of it crosses the start of rank 1, which falls
+    inside a byte of the body: rank 1's first eight symbols give no bits, so the ranks exchange the real first bytes
+    after the pack."""
+    text = np.random.default_rng(300 + world).integers(0, 256, 143_000, dtype=np.uint8)
+    at = sharded.ShardPlan(text.size, world, 0).bounds[1]
+    for lead in range(1000, 1008):  # the run's first bit, and so rank 1's, moves with the code before it
+        data = text.copy()
+        data[at - lead : at + 2000] = 255
+        if _boundaries(data)[at] % 8:
+            break
+    assert et.build_codebook(oracle.histogram(data)).code[255].length == 0
+    assert _boundaries(data)[at] % 8
+    return data
+
+
 def _pack_in_shards(codec, data, cuts):
     """Pack data[cuts[i]:cuts[i+1]] at its final bit offset with et_pack_shard_dev; -> (header, body, phases)."""
     import torch
@@ -117,6 +155,21 @@ def test_pack_shards_tiny_dropped_and_deep(codec):
     cuts = [0, 1_000_001, 1_000_002, 4_000_013, 9_000_000, data.size]
     header, body, _ = _pack_in_shards(codec, data, cuts)
     assert header + body == _oracle_et(data)
+    # codes of 33 bits (the wide kernel): shards at every bit phase, shards that begin or end with a 33-bit code, and one
+    # that holds nothing else
+    data = _chain33()
+    _, length = oracle.build_dictionary(oracle.histogram(data))
+    assert int(length.max()) == 33
+    bounds = _boundaries(data)
+    at_phase = [t + int(np.flatnonzero(bounds[t : t + 256] % 8 == ph)[0]) for ph, t in zip(range(8), range(1_000_003, 14_000_000, 1_600_000))]
+    d0, d1 = (int(x) for x in np.flatnonzero(length[data] == 33))
+    want = _oracle_et(data)
+    seen = set()
+    for cuts in ([0] + at_phase + [data.size], sorted({0, d0, d0 + 1, d1 - 5, d1 + 1, data.size})):
+        header, body, phases = _pack_in_shards(codec, data, cuts)
+        assert header + body == want, cuts
+        seen.update(phases)
+    assert seen == set(range(8)), seen
 
 
 def _boundaries(data):
@@ -229,7 +282,9 @@ class ThreadComm:
         return torch.cat(mine) if mine else torch.empty(0, dtype=torch.uint8, device=send.device)
 
 
-def _run_ranks(world, data, results, native=False):
+def _run_ranks(world, data, results, native=False, decode=True):
+    """results[rank] = (header, the rank's own body bytes, total bytes, all-gathers of the native encode (None when not
+    native)) + with decode: (text offset, text, rounds).  decode=False stops after the encode (codes over 32 bits)."""
     import torch
 
     shared = {"slots": [None] * world, "barrier": threading.Barrier(world)}
@@ -241,8 +296,14 @@ def _run_ranks(world, data, results, native=False):
             with et.Codec(0) as codec:
                 plan = sharded.ShardPlan(data.size, world, rank)
                 tcomm = ThreadComm(world, rank, shared)
+                gathers = [0]
+
+                def allgather(send):
+                    gathers[0] += 1
+                    return b"".join(tcomm._exchange(send))
+
                 if native:  # the protocol inside the library; its all-gathers come back to this process through a callback
-                    ncomm = codec.comm_callback(rank, world, lambda send: b"".join(tcomm._exchange(send)))
+                    ncomm = codec.comm_callback(rank, world, allgather)
                     coder = sharded.NativeShardedCodec(codec, plan, ncomm, tcomm)
                 else:
                     coder = sharded.ShardedCodec(sharded.GpuBackend(codec), plan, tcomm)
@@ -251,13 +312,19 @@ def _run_ranks(world, data, results, native=False):
                 torch.cuda.synchronize()
                 res = coder.encode(t_in, t_body)
                 mine = t_body[res.own_lo - res.first_byte : res.own_hi - res.first_byte].cpu().numpy().tobytes()
+                encoded = (res.header, mine, res.total_bytes, gathers[0] if native else None)
+                if not decode:
+                    results[rank] = encoded
+                    if native:
+                        codec.comm_destroy(ncomm)
+                    return
                 t_range = coder.scatter_body(res, t_body)
                 cuts, ranges = coder.decode_ranges(res.body_bytes)
                 s, t = ranges[rank]
                 t_out = torch.zeros(8 * max(t - s, 1) + 64, dtype=torch.uint8, device="cuda")
                 torch.cuda.synchronize()
                 dres = coder.decode(res.header[4:], res.body_bytes, t_range, t_out)
-                results[rank] = (res.header, mine, res.total_bytes, dres.offset, t_out[: dres.n_local].cpu().numpy().tobytes(), dres.rounds)
+                results[rank] = encoded + (dres.offset, t_out[: dres.n_local].cpu().numpy().tobytes(), dres.rounds)
                 if native:
                     codec.comm_destroy(ncomm)
         except BaseException as exc:  # noqa: BLE001 - reported by the test thread
@@ -273,21 +340,27 @@ def _run_ranks(world, data, results, native=False):
         raise errors[0][1]
 
 
-def _check_protocol(world, name, data, native=False):
+def _check_protocol(world, name, data, native=False, decode=True, encode_gathers=None):
+    """The sharded .et against the oracle's, then (decode) the text.  encode_gathers: the all-gathers every rank's native
+    encode must make.  -> the largest decode rounds count."""
     results = [None] * world
-    _run_ranks(world, data, results, native)
+    _run_ranks(world, data, results, native, decode)
     want = _oracle_et(data)
     header = results[0][0]
     assert header + b"".join(r[1] for r in results) == want, f"{name}: sharded .et differs from the oracle's (world {world})"
     assert all(r[2] == len(want) for r in results)
+    if encode_gathers is not None:
+        assert [r[3] for r in results] == [encode_gathers] * world, (name, world, [r[3] for r in results])
+    if not decode:
+        return None
     lossless = np.unique(data).size < 256  # the reference drops a symbol when all 256 occur (SURVEY §0.2)
     expect = data.tobytes() if lossless else oracle.decode(np.frombuffer(want, np.uint8)[4:], data.size).tobytes()
     full = bytearray(len(expect))
-    for _, _, _, off, chunk, _ in results:
+    for *_, off, chunk, _ in results:
         full[off : off + len(chunk)] = chunk
-    assert sum(len(r[4]) for r in results) == len(expect), name
+    assert sum(len(r[5]) for r in results) == len(expect), name
     assert bytes(full) == expect, f"{name}: sharded decode differs (world {world})"
-    return max(r[5] for r in results)
+    return max(r[6] for r in results)
 
 
 @pytest.mark.parametrize("world", [2, 3, 8])
@@ -310,11 +383,15 @@ def test_sharded_protocol_on_real_kernels(world):
 def test_sharded_protocol_inside_the_library(world):
     """et_encode_sharded_dev / et_decode_sharded_dev (exchanges through an et_comm) against the oracle."""
     rng = np.random.default_rng(200 + world)
-    assert _check_protocol(world, "text", _text(2_000_003, seed=10 + world), native=True) == 1
+    assert _check_protocol(world, "text", _text(2_000_003, seed=10 + world), native=True, encode_gathers=1) == 1
     rounds = _check_protocol(world, "uniform255", rng.integers(1, 256, 700_001, dtype=np.uint8), native=True)
     assert world == 2 or rounds >= 2
     _check_protocol(world, "all256", np.concatenate([rng.integers(0, 256, 90_000, dtype=np.uint8), np.full(3000, 255, np.uint8),
                                                      rng.integers(0, 256, 50_000, dtype=np.uint8)]), native=True)
+    # the second exchange of the encoder: rank 1 starts inside a byte with a run of the symbol that has no code
+    _check_protocol(world, "all256_run_at_cut", _dropped_run_at_cut(world), native=True, encode_gathers=2)
+    if world > 2:  # ... or with a code of 33 bits; the decoder refuses such codes (the reference's cannot hold them)
+        _check_protocol(world, "chain33", _chain33_at_cuts(world), native=True, decode=False, encode_gathers=2)
     _check_protocol(world, "tiny", _text(50 + world), native=True)
     for name, case in make_cases().items():
         if np.unique(case).size >= 2 and case.size >= 16 * world:

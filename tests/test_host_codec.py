@@ -80,6 +80,22 @@ def test_header_matches_oracle_on_cases():
         assert len(full) == len(hdr) + (cb.body_bits + 7) // 8, name
 
 
+def test_header_matches_oracle_for_codes_over_32_bits():
+    # exact Fibonacci counts at the chain's minimum size: the longest code has `depth` bits, and the header writes its
+    # bits as the reference does past 32 (encode.zig:311 shifts by a u5: emitted_bit); the text order does not matter
+    from entreepy_b200 import synth
+
+    for depth, n in ((33, 14_930_351), (34, 24_157_816), (36, 63_245_985)):
+        counts = np.array(synth.fibonacci_counts(n, depth), dtype=np.uint64)
+        assert int(counts.sum()) == n and int(oracle.build_dictionary(counts)[1].max()) == depth
+        cb = et.build_codebook(counts)
+        assert cb.max_length == depth
+        hdr = et.write_header(cb, n)
+        full = oracle.encode(np.repeat(np.arange(256, dtype=np.uint8), counts.astype(np.int64))).tobytes()
+        assert full.startswith(hdr), depth
+        assert len(full) == len(hdr) + (cb.body_bits + 7) // 8, depth
+
+
 def test_body_length_field_wraps_at_32_bits():
     cb = et.build_codebook(oracle.histogram(b"ab"))
     assert et.write_header(cb, 2**32 + 5)[5:9] == (5).to_bytes(4, "big")  # encode.zig:279
