@@ -19,7 +19,7 @@ SYMBOLS = [
     "et_abi_version", "et_strerror", "et_ctx_create", "et_ctx_destroy", "et_last_error", "et_ctx_set_output_fd",
     "et_ctx_kernel_launches", "et_ctx_last_stage_ms", "et_ctx_last_decode_rounds", "et_ctx_set_tuning", "et_alloc_pinned", "et_free_pinned", "et_build_codebook",
     "et_header_size", "et_write_header", "et_encode_bound", "et_parse_header", "et_histogram", "et_histogram_dev",
-    "et_encode", "et_decode", "et_encode_dev", "et_decode_dev", "et_decode_batch_dev", "et_pack_shard_dev", "et_shard_bits",
+    "et_encode", "et_decode", "et_encode_dev", "et_decode_dev", "et_decode_batch_dev", "et_encode_batch_dev", "et_pack_shard_dev", "et_shard_bits",
     "et_unpack_shard_dev", "et_synth_dev", "et_comm_unique_id", "et_comm_create_nccl", "et_comm_create_callback", "et_comm_destroy",
     "et_encode_sharded_dev", "et_decode_sharded_dev",
 ]
@@ -40,7 +40,8 @@ class ShardDecoded(ctypes.Structure):
 
 
 class BatchItem(ctypes.Structure):
-    """et_batch_item: one stream of et_decode_batch_dev (device pointers; out_len and status are written by the call)."""
+    """et_batch_item: one stream of et_decode_batch_dev or one text of et_encode_batch_dev (device pointers; out_len and status
+    are written by the call)."""
     _fields_ = [("d_in", ctypes.c_void_p), ("n", ctypes.c_size_t), ("d_out", ctypes.c_void_p), ("cap", ctypes.c_size_t),
                 ("out_len", ctypes.c_size_t), ("status", ctypes.c_int)]
 
@@ -115,6 +116,7 @@ def load():
         "et_encode_dev": (i, [vp, vp, sz, vp, sz, szp, u32, vp]),
         "et_decode_dev": (i, [vp, vp, sz, vp, sz, szp, u32, vp]),
         "et_decode_batch_dev": (i, [vp, ctypes.POINTER(BatchItem), sz, u32, vp]),
+        "et_encode_batch_dev": (i, [vp, ctypes.POINTER(BatchItem), sz, u32, vp]),
         "et_pack_shard_dev": (i, [vp, vp, sz, ctypes.POINTER(Codebook), u32, u64, vp, sz, szp, vp]),
         "et_shard_bits": (u64, [vp, ctypes.POINTER(Codebook)]),
         "et_unpack_shard_dev": (i, [vp, vp, sz, sz, sz, ctypes.POINTER(Dictionary), ctypes.c_int64, vp, sz,

@@ -775,3 +775,4 @@ extern "C" int et_synth_dev(et_ctx *ctx, void *d_out, size_t n, uint64_t seed, u
 
 #include "et_shard.inc"
 #include "et_batch.inc"
+#include "et_batch_encode.inc"

@@ -85,6 +85,44 @@ cudaError_t launch_histogram(const uint8_t *d_in, size_t n, unsigned long long *
     return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------- batched histogram (et_encode_batch_dev)
+namespace {
+constexpr int kBatchHistThreads = 256;
+
+// A CTA per tile of one stream: the same lane-column table as histogram_kernel, folded into the stream's counts.
+__global__ void __launch_bounds__(kBatchHistThreads) batch_histogram_kernel(const EncHistTile *__restrict__ tiles,
+                                                                            unsigned long long *__restrict__ counts) {
+    __shared__ __align__(16) uint32_t table[256 * 32];  // [bin][lane], 32 KiB
+    for (int i = threadIdx.x; i < 256 * 32; i += kBatchHistThreads) table[i] = 0;
+    const EncHistTile t = tiles[blockIdx.x];
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31;
+    uint8_t *table_lane = reinterpret_cast<uint8_t *>(table) + lane * 4;
+    for (uint32_t b0 = threadIdx.x * 16u; b0 < t.hi; b0 += kBatchHistThreads * 16u) {
+        if (b0 >= t.lo && b0 + 16u <= t.hi) {
+            const uint4 a = ld_stream_v4(reinterpret_cast<const uint4 *>(t.base + b0));
+            count_word(table_lane, a.x); count_word(table_lane, a.y); count_word(table_lane, a.z); count_word(table_lane, a.w);
+        } else {  // the ragged ends of the stream: only its own bytes
+            for (uint32_t k = max(b0, t.lo); k < min(b0 + 16u, t.hi); ++k) atomicAdd(&table[t.base[k] * 32 + lane], 1u);
+        }
+    }
+    __syncthreads();
+    const uint32_t bin = threadIdx.x;
+    unsigned long long sum = 0;
+#pragma unroll 8
+    for (uint32_t k = 0; k < 32; ++k) sum += table[bin * 32 + ((k + lane) & 31)];
+    if (sum) atomicAdd(&counts[(size_t)t.item * 256 + bin], sum);
+}
+static_assert(kBatchHistThreads == 256, "a thread per bin folds the table");
+}  // namespace
+
+cudaError_t launch_batch_histogram(const EncBatchLayout &L, uint32_t hist_tiles, cudaStream_t stream, int *launches) {
+    if (hist_tiles == 0) return cudaSuccess;
+    batch_histogram_kernel<<<hist_tiles, kBatchHistThreads, 0, stream>>>(L.hist_tiles, L.counts);
+    if (launches) *launches += 1;
+    return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------- synthetic input generator
 namespace {
 __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {

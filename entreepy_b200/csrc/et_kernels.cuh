@@ -35,7 +35,7 @@ size_t pack_scratch_bytes(const PackGeometry &g);
 cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, uint32_t max_len, uint8_t *d_out, uint32_t bit_phase,
                         void *scratch_base, int num_sms,
                         cudaStream_t stream, int *launches, int bits_ctas_per_sm = 0);
-// Once per context: lets the pack kernels use all of an SM's shared memory and reads how many CTAs of pass A fit an SM
+// Once per context: lets the pack kernels (the batched pass B too) use all of an SM's shared memory and reads how many CTAs of pass A fit an SM
 // (both used to be asked of the runtime at every call, a few microseconds each with the GPU waiting).
 cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm);
 
@@ -125,6 +125,28 @@ cudaError_t launch_batch_tables(const BatchLayout &L, uint32_t items, cudaStream
 // settle_first: a stream with long chunks synchronises slowly, so the entries are settled before the first write walk.
 cudaError_t launch_unpack_batch(const BatchLayout &L, uint32_t items, uint32_t n_tiles, uint64_t n_chunks, bool settle_first,
                                 BatchStatus *h_status, cudaStream_t stream, int *launches, uint32_t *rounds_out);
+
+// ---------------------------------------------------------------- batched encode (et_batch_encode.inc)
+// Adds every histogram tile's byte counts into L.counts[item * 256 ..) (cleared by the caller); one launch.
+cudaError_t launch_batch_histogram(const EncBatchLayout &L, uint32_t hist_tiles, cudaStream_t stream, int *launches);
+// One stream of the batched pack: its text, its place among the group's regions and where its file goes.
+struct BatchPackStream {
+    PackGeometry g;
+    uint64_t first_region;  // its regions in the group's arrays (EncBatchLayout L, device addresses)
+    uint32_t n_regions;
+    uint32_t table;         // its pack table: L.tables + 512 * table
+    uint64_t header_off;    // its header: L.headers + header_off, header_len bytes, to d_out[0, header_len)
+    uint32_t header_len;
+    uint8_t *d_out;
+};
+size_t batch_pack_args_bytes();
+// Writes the pack's arguments for a stream of the group to dst (host memory, batch_pack_args_bytes() bytes).
+void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStream &s);
+// Packs the group (args, tables, headers and tiles uploaded) as launch_pack's lane-run path packs one stream, and copies
+// every header in front of its body: pass A, region scan, group scan, pass B, seam fix-up with headers (5 launches).
+// max_len: the longest code of the group's streams (sizes the warps' bit images).  Does not synchronise.
+cudaError_t launch_pack_batch(const EncBatchLayout &L, uint32_t n_tiles, uint64_t n_regions, uint32_t max_len, cudaStream_t stream,
+                              int *launches);
 
 // ---------------------------------------------------------------- synthetic input generator
 cudaError_t launch_synth(uint8_t *d_out, size_t n, uint64_t seed, uint64_t first_index, const uint32_t *d_thresholds,

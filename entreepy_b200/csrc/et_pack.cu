@@ -31,6 +31,8 @@
 //
 // Algorithmic HBM bytes per symbol: 1 read + len/8 written (text: 1.586 B/symbol); pass A reads
 // the text a second time (not credited).
+#include <cstring>
+
 #include "et_device.cuh"
 #include "et_kernels.cuh"
 
@@ -201,6 +203,39 @@ __device__ __forceinline__ uint32_t table_length(uint32_t w, uint32_t len_lane_s
     return len;
 }
 
+// Pass A's work on one region r (a warp): the bits of its 32 runs and its total.  Interior regions take the four vectors of
+// the lane, loaded coalesced (load i of lane L is vector 32 i + L of the region, a quarter of run 8 i + L / 4).
+__device__ __forceinline__ void region_bits_interior(const PackArgs &a, uint32_t r, uint32_t lane, const uint4 (&v)[4], uint32_t len_lane_s,
+                                                     uint32_t r128) {
+    uint32_t total = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const uint32_t w[4] = {v[i].x, v[i].y, v[i].z, v[i].w};
+        uint32_t bits = 0;
+#pragma unroll
+        for (int q = 0; q < 4; ++q)
+            bits += table_length<0>(w[q], len_lane_s, r128) + table_length<1>(w[q], len_lane_s, r128) +
+                    table_length<2>(w[q], len_lane_s, r128) + table_length<3>(w[q], len_lane_s, r128);
+        bits += __shfl_xor_sync(0xffffffffu, bits, 1);
+        bits += __shfl_xor_sync(0xffffffffu, bits, 2);  // the run's bits, in its four lanes
+        if ((lane & 3u) == 0) a.run_bits[(size_t)r * 32 + 8 * i + (lane >> 2)] = (uint16_t)bits;
+        total += (lane & 3u) == 0 ? bits : 0u;
+    }
+    total = __reduce_add_sync(0xffffffffu, total);
+    if (lane == 0) a.tile_bits[r] = total;
+}
+__device__ __forceinline__ void region_bits_ragged(const PackArgs &a, uint32_t r, uint32_t lane, const uint32_t *len_sh) {
+    uint32_t bits = 0;
+    {  // ragged ends of the input: a lane takes its own run, only the symbols that exist
+        const uint64_t v0 = (uint64_t)r * kRegionSyms + (uint64_t)lane * kRunSyms;
+        for (uint32_t i = 0; i < (uint32_t)kRunSyms; ++i)
+            if (v0 + i >= a.misalign && v0 + i < a.v_end) bits += len_sh[(uint32_t)a.in_aligned[v0 + i] * 32];
+    }
+    a.run_bits[(size_t)r * 32 + lane] = (uint16_t)bits;
+    const uint32_t total = __reduce_add_sync(0xffffffffu, bits);
+    if (lane == 0) a.tile_bits[r] = total;
+}
+
 // Pass A, a warp per region: four coalesced 16-byte loads per lane, a run's bit count is the sum over the four lanes that
 // hold it (two shuffles), and nothing in the kernel waits for anything - no barrier, no running total carried by one
 // thread (round 1's slab form, 4096 symbols per CTA step with the group's running total kept
@@ -234,33 +269,10 @@ __global__ void __launch_bounds__(kPackThreads) region_bits_kernel(const PackArg
         if (have) {
             const uint4 v[4] = {nv[0], nv[1], nv[2], nv[3]};
             request(r + stride);
-            uint32_t total = 0;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const uint32_t w[4] = {v[i].x, v[i].y, v[i].z, v[i].w};
-                uint32_t bits = 0;
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-                    bits += table_length<0>(w[q], len_lane_s, r128) + table_length<1>(w[q], len_lane_s, r128) +
-                            table_length<2>(w[q], len_lane_s, r128) + table_length<3>(w[q], len_lane_s, r128);
-                bits += __shfl_xor_sync(0xffffffffu, bits, 1);
-                bits += __shfl_xor_sync(0xffffffffu, bits, 2);  // the run's bits, in its four lanes
-                if ((lane & 3u) == 0) a.run_bits[(size_t)r * 32 + 8 * i + (lane >> 2)] = (uint16_t)bits;
-                total += (lane & 3u) == 0 ? bits : 0u;
-            }
-            total = __reduce_add_sync(0xffffffffu, total);
-            if (lane == 0) a.tile_bits[r] = total;
+            region_bits_interior(a, r, lane, v, len_lane_s, r128);
             continue;
         }
-        uint32_t bits = 0;
-        {  // ragged ends of the input: a lane takes its own run, only the symbols that exist
-            const uint64_t v0 = (uint64_t)r * kRegionSyms + (uint64_t)lane * kRunSyms;
-            for (uint32_t i = 0; i < (uint32_t)kRunSyms; ++i)
-                if (v0 + i >= a.misalign && v0 + i < a.v_end) bits += len_sh[(uint32_t)a.in_aligned[v0 + i] * 32];
-        }
-        a.run_bits[(size_t)r * 32 + lane] = (uint16_t)bits;
-        const uint32_t total = __reduce_add_sync(0xffffffffu, bits);
-        if (lane == 0) a.tile_bits[r] = total;
+        region_bits_ragged(a, r, lane, len_sh);
         request(r + stride);
     }
 }
@@ -676,12 +688,9 @@ __global__ void __launch_bounds__(kPackThreads) pack_wide_kernel(const PackArgs 
 // One thread per tile: the byte a tile's last bits end in (when it also starts in that
 // tile) is the OR of that tile's tail and the heads of every following tile that starts
 // in the same byte.  Byte 0 of a shard that begins mid-byte has no owner; thread 0 adds it.
-__global__ void __launch_bounds__(256) seam_fixup_kernel(const unsigned long long *__restrict__ tile_state,
-                                                         const uint8_t *__restrict__ seam_head,
-                                                         const uint8_t *__restrict__ seam_tail, uint32_t num_tiles,
-                                                         uint32_t bit_phase, uint8_t *__restrict__ out) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= num_tiles) return;
+__device__ __forceinline__ void seam_fixup_tile(const unsigned long long *__restrict__ tile_state, const uint8_t *__restrict__ seam_head,
+                                                const uint8_t *__restrict__ seam_tail, uint32_t num_tiles, uint32_t bit_phase,
+                                                uint8_t *__restrict__ out, uint32_t i) {
     auto end_of = [&](uint32_t j) { return tile_state[j] & ~kStatusMask; };
     auto begin_of = [&](uint32_t j) { return j == 0 ? (unsigned long long)bit_phase : end_of(j - 1); };
     auto merge_from = [&](unsigned long long byte, uint32_t value, uint32_t j) {
@@ -696,6 +705,117 @@ __global__ void __launch_bounds__(256) seam_fixup_kernel(const unsigned long lon
     if ((e & 7) != 0 && ((e >> 3) << 3) >= b) merge_from(e >> 3, seam_tail[i], i + 1);
     if (i == 0 && bit_phase != 0) merge_from(0, 0, 0);
 }
+__global__ void __launch_bounds__(256) seam_fixup_kernel(const unsigned long long *__restrict__ tile_state,
+                                                         const uint8_t *__restrict__ seam_head,
+                                                         const uint8_t *__restrict__ seam_tail, uint32_t num_tiles,
+                                                         uint32_t bit_phase, uint8_t *__restrict__ out) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= num_tiles) return;
+    seam_fixup_tile(tile_state, seam_head, seam_tail, num_tiles, bit_phase, out, i);
+}
+
+// ------------------------------------------------------------------ batched pack (et_encode_batch_dev)
+// The lane-run pack of many streams at once.  Stream j owns the regions [R_j, R_j + n_regions) of the group; its PackArgs
+// hold its own geometry, table and output (out = its body, d_out + header_len), with run_bits, tile_bits, tile_state and the
+// seam arrays moved to its first region, so that the device functions above run on it with stream-local region numbers.
+// The scan runs over the regions of every stream: a region's body bit is prefix(R_j + r) - prefix(R_j).
+struct BatchPackArgs {
+    PackArgs a;
+    uint64_t first_region;         // R_j
+    const uint8_t *header;         // the stream's header in the group's scratch
+    uint32_t header_len;
+};
+static_assert(kEncPrefixGroup == kPrefixGroup, "the batched scan uses region_prefix_kernel's groups");
+
+__device__ __forceinline__ unsigned long long batch_region_prefix(const BatchPackArgs &b, uint32_t r) {
+    return b.a.group_prefix[(b.first_region + r) / kPrefixGroup] + b.a.tile_bits[r];
+}
+
+// Pass A over tiles of kEncTileRegions regions of one stream: the stream's table of lengths, then a warp per region.
+__global__ void __launch_bounds__(kPackThreads) batch_region_bits_kernel(const BatchPackArgs *__restrict__ args,
+                                                                         const BatchTile *__restrict__ tiles) {
+    __shared__ uint32_t len_sh[256 * 32];
+    const BatchTile tile = tiles[blockIdx.x];
+    const PackArgs &a = args[tile.item].a;
+    for (int i = threadIdx.x; i < 256 * 32; i += kPackThreads) len_sh[i] = static_cast<const uint2 *>(a.tables)[i >> 5].y;
+    __syncthreads();
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t len_lane_s = (uint32_t)__cvta_generic_to_shared(reinterpret_cast<const uint8_t *>(len_sh) + lane * 4);
+    const uint32_t r128 = opaque_128(a);
+    for (uint32_t r = tile.first + (threadIdx.x >> 5); r < min(tile.first + kEncTileRegions, a.n_regions); r += kWarps) {
+        if (region_is_interior(a, r)) {
+            const uint4 *src = reinterpret_cast<const uint4 *>(a.in_aligned + (uint64_t)r * kRegionSyms) + lane;
+            const uint4 v[4] = {ld_stream_v4(src), ld_stream_v4(src + 32), ld_stream_v4(src + 64), ld_stream_v4(src + 96)};
+            region_bits_interior(a, r, lane, v, len_lane_s, r128);
+        } else {
+            region_bits_ragged(a, r, lane, len_sh);
+        }
+    }
+}
+
+// Pass B over tiles of up to kEncTileRegions regions of one stream, a warp per region.  Dynamic shared memory as
+// pack_runs_kernel's: table | per warp: bit image | per warp: 32 edge bytes.
+__global__ void __launch_bounds__(kRunWarps * 32, 2) batch_pack_runs_kernel(const BatchPackArgs *__restrict__ args,
+                                                                            const BatchTile *__restrict__ tiles, uint32_t image_words) {
+    extern __shared__ __align__(16) uint8_t smem[];
+    uint8_t *table = smem;
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint32_t *stage = reinterpret_cast<uint32_t *>(smem + kTableBytes) + (size_t)warp * image_words;
+    uint8_t *edge = smem + kTableBytes + (size_t)kRunWarps * image_words * 4 + warp * 32;
+    const BatchTile tile = tiles[blockIdx.x];
+    const BatchPackArgs &b = args[tile.item];
+    const PackArgs &a = b.a;
+    {
+        const uint2 *src = static_cast<const uint2 *>(a.tables);
+        uint2 *dst = reinterpret_cast<uint2 *>(table);
+        for (int i = tid; i < 256 * kTableLanes; i += kRunWarps * 32) dst[i] = src[i / kTableLanes];
+        for (uint32_t i = lane; i < image_words; i += 32) stage[i] = 0;
+    }
+    __syncthreads();
+    const uint32_t r = tile.first + warp;
+    if (r >= a.n_regions) return;
+    const uint8_t *table_lane = table + (lane & (kTableLanes - 1)) * 8;
+    const uint32_t r128 = opaque_128(a);
+    const bool interior = region_is_interior(a, r);
+    uint4 raw[4];
+    unsigned long long valid = ~0ull;
+    load_run(a, r, lane, interior, raw, &valid);
+    const uint32_t my_bits = a.run_bits[(size_t)r * 32 + lane];
+    const unsigned long long bit_begin = batch_region_prefix(b, r) - batch_region_prefix(b, 0);
+    const uint32_t incl = warp_inclusive_scan(my_bits, lane);
+    const uint32_t region_bits = __shfl_sync(0xffffffffu, incl, 31);
+    const uint32_t my_off = incl - my_bits;
+    if (lane == 0) a.tile_state[r] = bit_begin + region_bits;  // for the seam fix-up
+    {  // assembled at the positions of the output frame, as in pack_runs_kernel
+        const uint32_t shift = region_frame_shift(a, bit_begin);
+        if (lane < 2) stage[kStageGuard + ((shift + region_bits) >> 5) + lane] = 0;
+        __syncwarp();
+        BitAcc acc;
+        open_acc(acc, (uint32_t)__cvta_generic_to_shared(stage + kStageGuard) * 8u + shift + my_off);
+        pack_run_symbols(acc, raw, valid, interior, table_lane, r128);
+        __syncwarp();  // every whole word is in place
+        if (acc.pos & 31u) atomicOr(stage + kStageGuard + ((shift + my_off + my_bits) >> 5), acc.lo << (32u - (acc.pos & 31u)));
+    }
+    __syncwarp();  // image complete
+    region_copy_out(a, r, stage, edge, bit_begin, region_bits, lane);
+}
+
+// The seam fix-up over the same tiles (a thread per region; the merge stops at the end of the stream), and the header of
+// every stream by the CTA of its first tile.  The body starts on a byte boundary and the regions store only the bytes they
+// own, so no byte holds both header and body.
+constexpr int kBatchSeamThreads = 64;
+__global__ void __launch_bounds__(kBatchSeamThreads) batch_seam_fixup_kernel(const BatchPackArgs *__restrict__ args,
+                                                                             const BatchTile *__restrict__ tiles) {
+    const BatchTile tile = tiles[blockIdx.x];
+    const BatchPackArgs &b = args[tile.item];
+    const PackArgs &a = b.a;
+    const uint32_t r = tile.first + threadIdx.x;
+    if (threadIdx.x < kEncTileRegions && r < a.n_regions)
+        seam_fixup_tile(a.tile_state, a.seam_head, a.seam_tail, a.n_regions, 0, a.out, r);
+    if (tile.first == 0)
+        for (uint32_t k = threadIdx.x; k < b.header_len; k += kBatchSeamThreads) a.out[(int64_t)k - (int64_t)b.header_len] = b.header[k];
+}
+static_assert(kEncTileRegions <= kBatchSeamThreads && kEncTileRegions == kRunWarps, "a tile is a region per warp of pass B");
 
 }  // namespace
 
@@ -713,6 +833,8 @@ size_t pack_scratch_bytes(const PackGeometry &g) { return pack_layout(nullptr, g
 
 cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm) {
     cudaError_t err = cudaFuncSetAttribute(pack_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+    if (err != cudaSuccess) return err;
+    err = cudaFuncSetAttribute(batch_pack_runs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
     if (err != cudaSuccess) return err;
     int per_sm = 0;
     err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, region_bits_kernel, kPackThreads, 0);
@@ -812,6 +934,62 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
     seam_fixup_kernel<<<(g.num_tiles + 255) / 256, 256, 0, stream>>>(s.tile_state, s.seam_head, s.seam_tail,
                                                                     g.num_tiles, bit_phase, d_out);
     if (launches) *launches += 1;
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ batched pack (et_batch_encode.inc)
+size_t batch_pack_args_bytes() { return sizeof(BatchPackArgs); }
+
+void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStream &s) {
+    BatchPackArgs b{};
+    PackArgs &a = b.a;
+    const PackGeometry &g = s.g;
+    a.in_aligned = g.in_aligned;
+    a.misalign = g.misalign;
+    a.v_end = g.v_end;
+    a.num_tiles = s.n_regions;
+    a.n_regions = s.n_regions;
+    a.tables = L.tables + (size_t)s.table * 512;
+    a.out = s.d_out + s.header_len;
+    a.bit_phase = 0;
+    a.tile_state = L.region_end + s.first_region;
+    a.seam_head = L.seam_head + s.first_region;
+    a.seam_tail = L.seam_tail + s.first_region;
+    a.tile_bits = L.region_bits + s.first_region;
+    a.run_bits = L.run_bits + s.first_region * 32;
+    a.group_prefix = L.group_prefix;  // indexed by the group's region numbers (batch_region_prefix)
+    a.group_tiles = kPrefixGroup;
+    a.group_shift = 10;
+    a.interior_lo = g.misalign ? 1u : 0u;
+    a.interior_hi = (uint32_t)(g.v_end / kRegionSyms);
+    if (a.interior_hi < a.interior_lo) a.interior_hi = a.interior_lo;
+    a.image_words = 1;  // read by opaque_128 only: batch_pack_runs_kernel takes the group's image size as a parameter
+    b.first_region = s.first_region;
+    b.header = L.headers + s.header_off;
+    b.header_len = s.header_len;
+    std::memcpy(dst, &b, sizeof b);
+}
+
+cudaError_t launch_pack_batch(const EncBatchLayout &L, uint32_t n_tiles, uint64_t n_regions, uint32_t max_len, cudaStream_t stream,
+                              int *launches) {
+    if (n_tiles == 0) return cudaSuccess;
+    const BatchPackArgs *args = reinterpret_cast<const BatchPackArgs *>(L.args);
+    // the scan over every region of the group, with the single-stream kernels
+    PackArgs s{};
+    s.tile_bits = L.region_bits;
+    s.group_prefix = L.group_prefix;
+    s.n_regions = (uint32_t)n_regions;
+    s.bit_phase = 0;
+    const uint32_t groups = (uint32_t)((n_regions + kPrefixGroup - 1) / kPrefixGroup);
+    batch_region_bits_kernel<<<n_tiles, kPackThreads, 0, stream>>>(args, L.tiles);
+    region_prefix_kernel<<<groups, kPrefixGroup, 0, stream>>>(s);
+    group_scan_kernel<<<1, 1024, 0, stream>>>(s, groups);
+    // the warps' images are sized by the group's longest code, as launch_pack sizes them by the stream's
+    const uint32_t image_words = (uint32_t)(kStageGuard + (kRegionSyms * max_len + 31) / 32 + 16 + 3) & ~3u;
+    const int smem = kTableBytes + kRunWarps * (int)image_words * 4 + kRunWarps * 32;
+    batch_pack_runs_kernel<<<n_tiles, kRunWarps * 32, smem, stream>>>(args, L.tiles, image_words);
+    batch_seam_fixup_kernel<<<n_tiles, kBatchSeamThreads, 0, stream>>>(args, L.tiles);
+    if (launches) *launches += 5;
     return cudaGetLastError();
 }
 

@@ -219,4 +219,67 @@ inline BatchLayout batch_layout(void *base, uint32_t items, size_t args_bytes, u
     return L;
 }
 
+// ---------------------------------------------------------------- batched encode (et_encode_batch_dev)
+// Groups follow the decode batch's rule (kBatchGroupItems streams, kBatchGroupBytes of text).  The histograms run over
+// tiles of kEncHistTileBytes of one stream; the pack numbers the regions of 2048 symbols of every stream of the group
+// one after another and runs over tiles of kEncTileRegions regions of one stream.
+constexpr uint32_t kEncHistTileBytes = 16384;  // text per CTA of the batched histogram (a multiple of 16)
+constexpr uint32_t kEncTileRegions = 16;       // regions per CTA of the batched pack (pass B: one per warp)
+constexpr uint32_t kEncPrefixGroup = 1024;     // regions per group of the scan (region_prefix_kernel)
+
+struct EncHistTile {  // bytes [lo, hi) of base[0, kEncHistTileBytes) belong to stream `item` (base 16-byte aligned)
+    const uint8_t *base;
+    uint32_t lo, hi;
+    uint32_t item, pad;
+};
+
+// The scratch of one encode group: `items` streams, `hist_tiles` histogram tiles; `packed` of them reach the batched pack
+// with `header_bytes` of headers, `tiles` pack tiles and `regions` regions in all.  Four runs: the counts (cleared, read
+// back), the histogram tiles (uploaded before the histogram), args .. tiles (uploaded with one copy before the pack),
+// device only.  A pinned host buffer of host_bytes carved the same way mirrors the first three.
+struct EncBatchLayout {
+    unsigned long long *counts = nullptr;        // [items * 256]
+    EncHistTile *hist_tiles = nullptr;           // [hist_tiles]
+    uint8_t *args = nullptr;                     // [packed * args_bytes] the pack's arguments per stream
+    uint32_t *tables = nullptr;                  // [packed * 512] narrow pack tables: 256 x {code, len}
+    uint8_t *headers = nullptr;                  // [header_bytes]
+    BatchTile *tiles = nullptr;                  // [tiles] kEncTileRegions regions of one stream, from its region `first`
+    uint16_t *run_bits = nullptr;                // [regions * 32] bits of every run of 64 symbols
+    uint32_t *region_bits = nullptr;             // [regions] a region's bits, then the bits before it inside its scan group
+    unsigned long long *group_prefix = nullptr;  // [(regions + kEncPrefixGroup - 1) / kEncPrefixGroup] bits before each scan group
+    unsigned long long *region_end = nullptr;    // [regions] last bit + 1 of each region, in its stream's body
+    uint8_t *seam_head = nullptr;                // [regions]
+    uint8_t *seam_tail = nullptr;                // [regions]
+    size_t counts_bytes = 0;                     // counts, from the start of the block
+    size_t hist_begin = 0, hist_end = 0;         // hist_tiles
+    size_t upload_begin = 0, upload_end = 0;     // args .. tiles
+    size_t host_bytes = 0;                       // counts .. tiles
+    size_t bytes = 0;
+};
+
+inline EncBatchLayout enc_batch_layout(void *base, uint32_t items, uint64_t hist_tiles, uint32_t packed, size_t args_bytes,
+                                       uint64_t header_bytes, uint64_t tiles, uint64_t regions) {
+    EncBatchLayout L;
+    Carve c{static_cast<uint8_t *>(base)};
+    L.counts = c.take<unsigned long long>((size_t)items * 256);
+    L.counts_bytes = c.bytes;
+    L.hist_tiles = c.take<EncHistTile>(hist_tiles);
+    L.hist_begin = c.bytes - hist_tiles * sizeof(EncHistTile);
+    L.hist_end = c.bytes;
+    L.args = c.take<uint8_t>((size_t)packed * args_bytes);
+    L.upload_begin = c.bytes - (size_t)packed * args_bytes;
+    L.tables = c.take<uint32_t>((size_t)packed * 512);
+    L.headers = c.take<uint8_t>(header_bytes);
+    L.tiles = c.take<BatchTile>(tiles);
+    L.upload_end = L.host_bytes = c.bytes;
+    L.run_bits = c.take<uint16_t>(regions * 32);
+    L.region_bits = c.take<uint32_t>(regions);
+    L.group_prefix = c.take<unsigned long long>((regions + kEncPrefixGroup - 1) / kEncPrefixGroup);
+    L.region_end = c.take<unsigned long long>(regions);
+    L.seam_head = c.take<uint8_t>(regions);
+    L.seam_tail = c.take<uint8_t>(regions);
+    L.bytes = c.bytes;
+    return L;
+}
+
 }  // namespace et

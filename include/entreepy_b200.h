@@ -172,14 +172,27 @@ ET_API int et_decode_dev(et_ctx *ctx, const void *d_in_after_magic, size_t n, vo
  * transfer functions are decoded one by one after them.  ET_FLAG_TIMING: et_ctx_last_stage_ms covers the whole call
  * ([0] heads and parse, [1] tables, [2] decode kernels); et_ctx_last_decode_rounds is the largest over the batch. */
 typedef struct et_batch_item {
-    const void *d_in; /* file[4..] of one stream, device memory (any alignment) */
+    const void *d_in; /* device memory, any alignment: file[4..] of one stream (decode) | one text (encode) */
     size_t n;
-    void *d_out;      /* device memory, any alignment */
+    void *d_out;      /* device memory, any alignment: the text (decode) | the whole .et file (encode) */
     size_t cap;
-    size_t out_len;   /* out */
-    int status;       /* out: et_status of this stream */
+    size_t out_len;   /* out: bytes written (decode) | the file size, also on a dry run (encode) */
+    int status;       /* out: et_status of this item */
 } et_batch_item;
 ET_API int et_decode_batch_dev(et_ctx *ctx, et_batch_item *items, size_t count, uint32_t flags, void *stream);
+
+/* Batched device encode: many independent texts in one call, the other direction of et_decode_batch_dev.  Item i ends
+ * with the status, *out_len and d_out bytes that et_encode_dev(ctx, d_in, n, d_out, cap, &out_len, flags, stream) would
+ * give it, including every failure (d_in == NULL with n > 0 or ET_FLAG_WRITE_OUTPUT with d_out == NULL:
+ * ET_ERR_INVALID_ARG; n == 0: ET_ERR_QUEUE_EMPTY; n > 2^32-1: ET_ERR_TOO_LARGE, before any byte is read;
+ * ET_ERR_NO_SPACE) and dry runs (*out_len = the file size, nothing written); a failing item does not affect the others.
+ * Items may share d_in.  Call-level behaviour as et_decode_batch_dev's.  Texts are handled in groups of up to 512 texts
+ * and 256 MiB: per group one histogram launch, one synchronise, the codebooks and headers on the host, one upload and a
+ * fixed number of pack launches.  Texts whose codes are longer than 32 bits, and texts of at least 256 MiB, are
+ * encoded one by one after their group, as et_encode_dev encodes them.  ET_FLAG_TIMING or ET_FLAG_DEBUG:
+ * et_ctx_last_stage_ms covers the whole call ([0] histograms and counts read-back, [1] host codebooks, headers and
+ * upload, [2] pack kernels); nothing is printed. */
+ET_API int et_encode_batch_dev(et_ctx *ctx, et_batch_item *items, size_t count, uint32_t flags, void *stream);
 
 /* ------------------------------------------------------------------ sharded path (SURVEY §8e) */
 /* One .et stream across several GPUs: each rank owns a contiguous byte range of the text
