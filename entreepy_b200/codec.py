@@ -225,20 +225,19 @@ class Codec:
         """et_decode_batch_dev: items = [(d_in_after_magic, n, d_out, cap)] -> [(status, out_len)], one per item, each what
         decode_dev would have given that item (a failing item carries its status and does not raise).  Raises only when
         the call itself fails (a CUDA error or allocation failure)."""
-        arr = (_abi.BatchItem * max(len(items), 1))()
-        for k, (d_in, n, d_out, cap) in enumerate(items):
-            arr[k] = _abi.BatchItem(d_in, n, d_out, cap, 0, 0)
-        self._check(self._lib.et_decode_batch_dev(self._ctx, arr, len(items), flags, stream))
-        return [(int(arr[k].status), int(arr[k].out_len)) for k in range(len(items))]
+        return self._batch(self._lib.et_decode_batch_dev, items, flags, stream)
 
     def encode_batch_dev(self, items, flags=_abi.FLAG_WRITE_OUTPUT, stream=None):
         """et_encode_batch_dev: items = [(d_in, n, d_out, cap)] -> [(status, out_len)], one per item, each what encode_dev
         would have given that item (a failing item carries its status and does not raise; out_len is the file size, also
         on a dry run).  Raises only when the call itself fails (a CUDA error or allocation failure)."""
+        return self._batch(self._lib.et_encode_batch_dev, items, flags, stream)
+
+    def _batch(self, entry, items, flags, stream):
         arr = (_abi.BatchItem * max(len(items), 1))()
         for k, (d_in, n, d_out, cap) in enumerate(items):
             arr[k] = _abi.BatchItem(d_in, n, d_out, cap, 0, 0)
-        self._check(self._lib.et_encode_batch_dev(self._ctx, arr, len(items), flags, stream))
+        self._check(entry(self._ctx, arr, len(items), flags, stream))
         return [(int(arr[k].status), int(arr[k].out_len)) for k in range(len(items))]
 
     def shard_bits(self, counts, cb):

@@ -155,6 +155,19 @@ struct StageTimer {
         if (!on) return;
         for (int i = 0; i + 1 < n_marks && i < 4; ++i) cudaEventElapsedTime(&ctx->stage_ms[i], ctx->ev[i], ctx->ev[i + 1]);
     }
+    // The end of a batch group's stages (marks 0..2 made): adds the times between the marks to ms[0..2].
+    cudaError_t add_group(float *ms) {
+        if (!on) return cudaSuccess;
+        mark(3);
+        const cudaError_t e = cudaEventSynchronize(ctx->ev[3]);
+        if (e != cudaSuccess) return e;
+        for (int k = 0; k < 3; ++k) {
+            float t = 0.f;
+            cudaEventElapsedTime(&t, ctx->ev[k], ctx->ev[k + 1]);
+            ms[k] += t;
+        }
+        return cudaSuccess;
+    }
 };
 
 // Histogram of a device buffer into host counts (blocks until the counts are on the host).
@@ -208,6 +221,22 @@ struct EncodePlan {
     et_codebook cb;
     size_t header_len = 0, total = 0;
 };
+
+// The file of `plan` to d_out: the header through the pinned staging, then the body behind it (pack_dev); returns once
+// the stream has finished (the staging is free again).  tm (or null): marks 2 and 3 around the pack.
+int write_encoded_dev(et_ctx *ctx, const void *d_in, size_t n, const EncodePlan &plan, uint8_t *d_out, cudaStream_t s, StageTimer *tm) {
+    uint8_t *h_header = ctx->h_small->header;
+    size_t hl = 0;
+    int rc = et_write_header(&plan.cb, n, h_header, kMaxHeaderBytes, &hl);  // E5
+    if (rc != ET_OK) return fail(ctx, rc, "header");
+    ET_CUDA(ctx, cudaMemcpyAsync(d_out, h_header, hl, cudaMemcpyHostToDevice, s));
+    if (tm) tm->mark(2);
+    rc = pack_dev(ctx, d_in, n, plan.cb, 0, d_out + hl, s);  // E6
+    if (rc != ET_OK) return rc;
+    if (tm) tm->mark(3);
+    ET_CUDA(ctx, cudaStreamSynchronize(s));
+    return ET_OK;
+}
 
 // Everything between the histogram and the pack: codebook, sizes, capacity checks.
 int plan_encode(et_ctx *ctx, const uint64_t counts[256], size_t n, size_t cap, uint32_t flags, EncodePlan *p) {
@@ -386,17 +415,8 @@ extern "C" int et_encode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_ou
     if (rc != ET_OK) return rc;
     if (flags & ET_FLAG_DEBUG) print_dictionary(ctx->out_fd, plan.cb);
     if (write_out) {
-        uint8_t *h_header = ctx->h_small->header;
-        size_t hl = 0;
-        rc = et_write_header(&plan.cb, n, h_header, kMaxHeaderBytes, &hl);  // E5
-        if (rc != ET_OK) return fail(ctx, rc, "header");
-        uint8_t *out = static_cast<uint8_t *>(d_out);
-        ET_CUDA(ctx, cudaMemcpyAsync(out, h_header, hl, cudaMemcpyHostToDevice, s));
-        tm.mark(2);
-        rc = pack_dev(ctx, d_in, n, plan.cb, 0, out + hl, s);  // E6
+        rc = write_encoded_dev(ctx, d_in, n, plan, static_cast<uint8_t *>(d_out), s, &tm);
         if (rc != ET_OK) return rc;
-        tm.mark(3);
-        ET_CUDA(ctx, cudaStreamSynchronize(s));
         tm.finish(4);
     }
     *out_len = plan.total;  // returned even on a dry run (encode.zig:336)
@@ -572,6 +592,16 @@ int check_stream(et_ctx *ctx, const et_dictionary &dict, size_t n, uint32_t flag
     return ET_OK;
 }
 
+// et_decode_dev's result for a stream in which the decoder found `total` symbols: *out_len, or NoSpaceLeft when the text
+// did not fit `cap`.
+int decode_result(et_ctx *ctx, const et_dictionary &dict, size_t cap, uint64_t total, size_t *out_len) {
+    const uint64_t want = std::min<uint64_t>(dict.body_len, cap);
+    const uint64_t produced = std::min<uint64_t>(total, want);
+    if (produced == cap && dict.body_len > cap) return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %u symbols, capacity %zu", dict.body_len, cap);
+    *out_len = (size_t)produced;
+    return ET_OK;
+}
+
 }  // namespace
 
 extern "C" int et_decode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_out, size_t cap, size_t *out_len,
@@ -601,12 +631,10 @@ extern "C" int et_decode_dev(et_ctx *ctx, const void *d_in, size_t n, void *d_ou
     rc = unpack_dev(ctx, unpack_geometry(static_cast<const uint8_t *>(d_in) + dict.body_offset, n - dict.body_offset), dict,
                     static_cast<uint8_t *>(d_out), want, s, &st, &tm, false, (flags & ET_FLAG_VALIDATE) != 0);  // D3
     if (rc != ET_OK) return rc;
-    const uint64_t produced = std::min<uint64_t>(st.total, want);
     tm.mark(3);
     ET_CUDA(ctx, cudaEventSynchronize(ctx->ev[3]));
     tm.finish(4);
-    if (produced == cap && dict.body_len > cap) return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %u symbols, capacity %zu", dict.body_len, cap);
-    *out_len = (size_t)produced;
+    if ((rc = decode_result(ctx, dict, cap, st.total, out_len)) != ET_OK) return rc;
     if (flags & ET_FLAG_DEBUG) {
         const auto us = std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t0).count();
         fd_printf(ctx->out_fd, "time taken: %lldμs\n", (long long)us);  // decode.zig:16
@@ -651,8 +679,8 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
             if (rc != ET_OK) return rc;
             produced = std::min<uint64_t>(st.total, want);
             if (write_out) {
-                if (produced == cap && dict.body_len > cap)
-                    return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %u symbols, capacity %zu", dict.body_len, cap);
+                size_t fits = 0;  // *out_len is set once the text is home
+                if ((rc = decode_result(ctx, dict, cap, produced, &fits)) != ET_OK) return rc;
                 if (produced) ET_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, produced, cudaMemcpyDeviceToHost, s));
                 ET_CUDA(ctx, cudaStreamSynchronize(s));
             }
@@ -700,8 +728,8 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
             const cudaError_t e = cudaStreamSynchronize(ctx->copy_stream2);
             cleanup();
             if (e != cudaSuccess) return fail(ctx, ET_ERR_CUDA, "download: %s", cudaGetErrorString(e));
-            if (write_out && produced == cap && dict.body_len > cap)
-                return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %u symbols, capacity %zu", dict.body_len, cap);
+            size_t fits = 0;
+            if (write_out && (rc = decode_result(ctx, dict, cap, produced, &fits)) != ET_OK) return rc;
         }
         if (print_out && produced) {  // decode.zig:189 prints every symbol to std_out
             std::vector<uint8_t> text(produced);

@@ -140,8 +140,9 @@ struct BatchPackStream {
     uint8_t *d_out;
 };
 size_t batch_pack_args_bytes();
-// Writes the pack's arguments for a stream of the group to dst (host memory, batch_pack_args_bytes() bytes).
-void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStream &s);
+// Writes the pack's arguments for a stream of the group to dst (host memory, batch_pack_args_bytes() bytes).  max_len: the
+// longest code of the group's streams, as passed to launch_pack_batch.
+void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStream &s, uint32_t max_len);
 // Packs the group (args, tables, headers and tiles uploaded) as launch_pack's lane-run path packs one stream, and copies
 // every header in front of its body: pass A, region scan, group scan, pass B, seam fix-up with headers (5 launches).
 // max_len: the longest code of the group's streams (sizes the warps' bit images).  Does not synchronise.

@@ -241,10 +241,14 @@ __device__ __forceinline__ void region_bits_ragged(const PackArgs &a, uint32_t r
 // thread (round 1's slab form, 4096 symbols per CTA step with the group's running total kept
 // by thread 0, spent a third of its issue slots on those: 288 us per GiB against ~190 us here).  It writes the
 // run totals and every region's total; region_prefix_kernel turns the totals into prefixes inside groups of 1024.
-__global__ void __launch_bounds__(kPackThreads) region_bits_kernel(const PackArgs a) {
-    __shared__ uint32_t len_sh[256 * 32];  // [sym][lane]: a warp-wide lookup never has a bank conflict
-    for (int i = threadIdx.x; i < 256 * 32; i += kPackThreads) len_sh[i] = static_cast<const uint2 *>(a.tables)[i >> 5].y;
+// Pass A's table of lengths, [sym][lane]: a warp-wide lookup never has a bank conflict.
+__device__ __forceinline__ void load_len_table(uint32_t *len_sh, const PackArgs &a, uint32_t tid) {
+    for (int i = tid; i < 256 * 32; i += kPackThreads) len_sh[i] = static_cast<const uint2 *>(a.tables)[i >> 5].y;
     __syncthreads();
+}
+__global__ void __launch_bounds__(kPackThreads) region_bits_kernel(const PackArgs a) {
+    __shared__ uint32_t len_sh[256 * 32];
+    load_len_table(len_sh, a, threadIdx.x);
     const uint32_t lane = threadIdx.x & 31;
     const uint8_t *len_lane = reinterpret_cast<const uint8_t *>(len_sh) + lane * 4;
     const uint32_t len_lane_s = (uint32_t)__cvta_generic_to_shared(len_lane), r128 = opaque_128(a);
@@ -430,6 +434,47 @@ __device__ __forceinline__ void region_copy_out(const PackArgs &a, uint32_t r, c
     __syncwarp();  // the slots are free again
 }
 
+// Pass B's shared memory: the table, replicated for kTableLanes lanes, and the warp's bit image cleared.
+__device__ __forceinline__ void load_run_table(uint8_t *table, const PackArgs &a, uint32_t *stage, uint32_t tid) {
+    const uint32_t lane = tid & 31;
+    const uint2 *src = static_cast<const uint2 *>(a.tables);
+    uint2 *dst = reinterpret_cast<uint2 *>(table);
+    for (int i = tid; i < 256 * kTableLanes; i += kRunWarps * 32) dst[i] = src[i / kTableLanes];
+    for (uint32_t i = lane; i < a.image_words; i += 32) stage[i] = 0;
+    __syncthreads();
+}
+
+// Pass B's work on region r once a lane holds its run (raw, valid): the run offsets, the region's end for the seam
+// fix-up, the image assembled at the positions of the output frame, and the copy-out.  bit_begin: the region's first
+// bit in the stream's body.
+__device__ __forceinline__ void pack_region(const PackArgs &a, uint32_t r, uint32_t lane, const uint4 (&raw)[4], unsigned long long valid,
+                                            bool interior, uint32_t my_bits, unsigned long long bit_begin, uint32_t *stage, uint8_t *edge,
+                                            const uint8_t *table_lane, uint32_t r128) {
+    const uint32_t incl = warp_inclusive_scan(my_bits, lane);
+    const uint32_t region_bits = __shfl_sync(0xffffffffu, incl, 31);
+    const uint32_t my_off = incl - my_bits;
+    const unsigned long long bit_end = bit_begin + region_bits;
+    if (lane == 0) a.tile_state[r] = bit_end;  // for the seam fix-up
+
+    // ---- assemble at region-relative positions (words hold stream bits MSB-first)
+    {
+        // the word in which the region ends is only ever ORed into (or not touched at all), and the byte in which
+        // it ends may reach into the word after it: both start from zero
+        // (the image is assembled at the positions of the output frame - region bit 0 at bit `shift` - so that the
+        // copy-out has nothing to shift; what lies before the region's first bit in its first block is never stored)
+        const uint32_t shift = region_frame_shift(a, bit_begin);
+        if (lane < 2) stage[kStageGuard + ((shift + region_bits) >> 5) + lane] = 0;
+        __syncwarp();
+        BitAcc acc;
+        open_acc(acc, (uint32_t)__cvta_generic_to_shared(stage + kStageGuard) * 8u + shift + my_off);
+        pack_run_symbols(acc, raw, valid, interior, table_lane, r128);
+        __syncwarp();  // every whole word is in place
+        if (acc.pos & 31u) atomicOr(stage + kStageGuard + ((shift + my_off + my_bits) >> 5), acc.lo << (32u - (acc.pos & 31u)));
+    }
+    __syncwarp();  // image complete
+    region_copy_out(a, r, stage, edge, bit_begin, region_bits, lane);
+}
+
 // Pass B.  Dynamic shared memory: table (32 KiB, 16-lane replicated) | per warp: bit image | per warp: 32 edge bytes.
 __global__ void __launch_bounds__(kRunWarps * 32, 2) pack_runs_kernel(const PackArgs a) {
     extern __shared__ __align__(16) uint8_t smem[];
@@ -437,13 +482,7 @@ __global__ void __launch_bounds__(kRunWarps * 32, 2) pack_runs_kernel(const Pack
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     uint32_t *stage = reinterpret_cast<uint32_t *>(smem + kTableBytes) + (size_t)warp * a.image_words;
     uint8_t *edge = smem + kTableBytes + (size_t)kRunWarps * a.image_words * 4 + warp * 32;
-    {
-        const uint2 *src = static_cast<const uint2 *>(a.tables);
-        uint2 *dst = reinterpret_cast<uint2 *>(table);
-        for (int i = tid; i < 256 * kTableLanes; i += kRunWarps * 32) dst[i] = src[i / kTableLanes];
-        for (uint32_t i = lane; i < a.image_words; i += 32) stage[i] = 0;
-    }
-    __syncthreads();
+    load_run_table(table, a, stage, tid);
     const uint8_t *table_lane = table + (lane & (kTableLanes - 1)) * 8;
     const uint32_t r128 = opaque_128(a);
     const uint32_t stride = gridDim.x * kRunWarps;
@@ -489,29 +528,7 @@ __global__ void __launch_bounds__(kRunWarps * 32, 2) pack_runs_kernel(const Pack
                                           : reinterpret_cast<const uint8_t *>(a.run_bits + (size_t)r_next * 32);
             if (lane <= 16) asm volatile("prefetch.global.L2 [%0];" ::"l"(nx));
         }
-        const uint32_t incl = warp_inclusive_scan(my_bits, lane);
-        const uint32_t region_bits = __shfl_sync(0xffffffffu, incl, 31);
-        const uint32_t my_off = incl - my_bits;
-        const unsigned long long bit_end = bit_begin + region_bits;
-        if (lane == 0) a.tile_state[r] = bit_end;  // for the seam fix-up
-
-        // ---- assemble at region-relative positions (words hold stream bits MSB-first)
-        {
-            // the word in which the region ends is only ever ORed into (or not touched at all), and the byte in which
-            // it ends may reach into the word after it: both start from zero
-            // (the image is assembled at the positions of the output frame - region bit 0 at bit `shift` - so that the
-            // copy-out has nothing to shift; what lies before the region's first bit in its first block is never stored)
-            const uint32_t shift = region_frame_shift(a, bit_begin);
-            if (lane < 2) stage[kStageGuard + ((shift + region_bits) >> 5) + lane] = 0;
-            __syncwarp();
-            BitAcc acc;
-            open_acc(acc, (uint32_t)__cvta_generic_to_shared(stage + kStageGuard) * 8u + shift + my_off);
-            pack_run_symbols(acc, raw, valid, interior, table_lane, r128);
-            __syncwarp();  // every whole word is in place
-            if (acc.pos & 31u) atomicOr(stage + kStageGuard + ((shift + my_off + my_bits) >> 5), acc.lo << (32u - (acc.pos & 31u)));
-        }
-        __syncwarp();  // image complete
-        region_copy_out(a, r, stage, edge, bit_begin, region_bits, lane);
+        pack_region(a, r, lane, raw, valid, interior, my_bits, bit_begin, stage, edge, table_lane, r128);
         __syncwarp();  // everyone has read the image
         if (r_next >= a.n_regions) break;
         r = r_next;
@@ -737,8 +754,7 @@ __global__ void __launch_bounds__(kPackThreads) batch_region_bits_kernel(const B
     __shared__ uint32_t len_sh[256 * 32];
     const BatchTile tile = tiles[blockIdx.x];
     const PackArgs &a = args[tile.item].a;
-    for (int i = threadIdx.x; i < 256 * 32; i += kPackThreads) len_sh[i] = static_cast<const uint2 *>(a.tables)[i >> 5].y;
-    __syncthreads();
+    load_len_table(len_sh, a, threadIdx.x);
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t len_lane_s = (uint32_t)__cvta_generic_to_shared(reinterpret_cast<const uint8_t *>(len_sh) + lane * 4);
     const uint32_t r128 = opaque_128(a);
@@ -754,24 +770,19 @@ __global__ void __launch_bounds__(kPackThreads) batch_region_bits_kernel(const B
 }
 
 // Pass B over tiles of up to kEncTileRegions regions of one stream, a warp per region.  Dynamic shared memory as
-// pack_runs_kernel's: table | per warp: bit image | per warp: 32 edge bytes.
+// pack_runs_kernel's: table | per warp: bit image | per warp: 32 edge bytes (every stream of the group has the group's
+// image_words).
 __global__ void __launch_bounds__(kRunWarps * 32, 2) batch_pack_runs_kernel(const BatchPackArgs *__restrict__ args,
-                                                                            const BatchTile *__restrict__ tiles, uint32_t image_words) {
+                                                                            const BatchTile *__restrict__ tiles) {
     extern __shared__ __align__(16) uint8_t smem[];
     uint8_t *table = smem;
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    uint32_t *stage = reinterpret_cast<uint32_t *>(smem + kTableBytes) + (size_t)warp * image_words;
-    uint8_t *edge = smem + kTableBytes + (size_t)kRunWarps * image_words * 4 + warp * 32;
     const BatchTile tile = tiles[blockIdx.x];
     const BatchPackArgs &b = args[tile.item];
     const PackArgs &a = b.a;
-    {
-        const uint2 *src = static_cast<const uint2 *>(a.tables);
-        uint2 *dst = reinterpret_cast<uint2 *>(table);
-        for (int i = tid; i < 256 * kTableLanes; i += kRunWarps * 32) dst[i] = src[i / kTableLanes];
-        for (uint32_t i = lane; i < image_words; i += 32) stage[i] = 0;
-    }
-    __syncthreads();
+    uint32_t *stage = reinterpret_cast<uint32_t *>(smem + kTableBytes) + (size_t)warp * a.image_words;
+    uint8_t *edge = smem + kTableBytes + (size_t)kRunWarps * a.image_words * 4 + warp * 32;
+    load_run_table(table, a, stage, tid);
     const uint32_t r = tile.first + warp;
     if (r >= a.n_regions) return;
     const uint8_t *table_lane = table + (lane & (kTableLanes - 1)) * 8;
@@ -782,22 +793,7 @@ __global__ void __launch_bounds__(kRunWarps * 32, 2) batch_pack_runs_kernel(cons
     load_run(a, r, lane, interior, raw, &valid);
     const uint32_t my_bits = a.run_bits[(size_t)r * 32 + lane];
     const unsigned long long bit_begin = batch_region_prefix(b, r) - batch_region_prefix(b, 0);
-    const uint32_t incl = warp_inclusive_scan(my_bits, lane);
-    const uint32_t region_bits = __shfl_sync(0xffffffffu, incl, 31);
-    const uint32_t my_off = incl - my_bits;
-    if (lane == 0) a.tile_state[r] = bit_begin + region_bits;  // for the seam fix-up
-    {  // assembled at the positions of the output frame, as in pack_runs_kernel
-        const uint32_t shift = region_frame_shift(a, bit_begin);
-        if (lane < 2) stage[kStageGuard + ((shift + region_bits) >> 5) + lane] = 0;
-        __syncwarp();
-        BitAcc acc;
-        open_acc(acc, (uint32_t)__cvta_generic_to_shared(stage + kStageGuard) * 8u + shift + my_off);
-        pack_run_symbols(acc, raw, valid, interior, table_lane, r128);
-        __syncwarp();  // every whole word is in place
-        if (acc.pos & 31u) atomicOr(stage + kStageGuard + ((shift + my_off + my_bits) >> 5), acc.lo << (32u - (acc.pos & 31u)));
-    }
-    __syncwarp();  // image complete
-    region_copy_out(a, r, stage, edge, bit_begin, region_bits, lane);
+    pack_region(a, r, lane, raw, valid, interior, my_bits, bit_begin, stage, edge, table_lane, r128);
 }
 
 // The seam fix-up over the same tiles (a thread per region; the merge stops at the end of the stream), and the header of
@@ -841,6 +837,21 @@ cudaError_t pack_init_device(int max_smem, int *bits_ctas_per_sm) {
     if (err != cudaSuccess) return err;
     *bits_ctas_per_sm = per_sm < 1 ? 1 : per_sm;
     return cudaSuccess;
+}
+
+// Words of a warp's bit image in pass B: a region at max_len bits a symbol, the frame's slack and the guard, in whole
+// 16-byte blocks.
+static uint32_t run_image_words(uint32_t max_len) { return (uint32_t)(kStageGuard + (kRegionSyms * max_len + 31) / 32 + 16 + 3) & ~3u; }
+
+// The lane-run fields of a stream's PackArgs: its interior regions, the groups of the region scan and the bit image.
+static void set_lane_runs(PackArgs &a, const PackGeometry &g, uint32_t max_len) {
+    a.interior_lo = g.misalign ? 1u : 0u;
+    a.interior_hi = (uint32_t)(g.v_end / kRegionSyms);
+    if (a.interior_hi < a.interior_lo) a.interior_hi = a.interior_lo;
+    a.image_words = run_image_words(max_len);
+    // (a region holds at most 2048 x 32 bits, a group 2^26: the prefix inside a group fits 32 bits)
+    a.group_tiles = kPrefixGroup;
+    a.group_shift = 10;
 }
 
 cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, uint32_t max_len, uint8_t *d_out, uint32_t bit_phase,
@@ -888,15 +899,9 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
         a.run_bits = s.run_bits;
         a.n_regions = n_regions;
         a.num_tiles = n_regions;
-        a.interior_lo = g.misalign ? 1u : 0u;
-        a.interior_hi = (uint32_t)(g.v_end / kRegionSyms);
-        if (a.interior_hi < a.interior_lo) a.interior_hi = a.interior_lo;
-        a.image_words = (uint32_t)(kStageGuard + (kRegionSyms * max_len + 31) / 32 + 16 + 3) & ~3u;
+        set_lane_runs(a, g, max_len);
         if (a.image_words < kStageGuard + kRegionSyms / 4) a.image_words = kStageGuard + kRegionSyms / 4;  // the image also stages the region's text
         // pass A: run and region totals (a warp per region), prefixes inside groups of 1024 regions, prefixes of the groups
-        // (a region holds at most 2048 x 32 bits, a group 2^26: the prefix inside a group fits 32 bits)
-        a.group_tiles = kPrefixGroup;
-        a.group_shift = 10;
         const uint32_t groups = (n_regions + kPrefixGroup - 1) / kPrefixGroup;
         {
             int per_sm = bits_ctas_per_sm;  // CTAs of 8 warps that fit an SM (32 KB table each, 48 registers per thread: five)
@@ -940,7 +945,7 @@ cudaError_t launch_pack(const PackGeometry &g, const void *d_tables, bool wide, 
 // ------------------------------------------------------------------ batched pack (et_batch_encode.inc)
 size_t batch_pack_args_bytes() { return sizeof(BatchPackArgs); }
 
-void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStream &s) {
+void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStream &s, uint32_t max_len) {
     BatchPackArgs b{};
     PackArgs &a = b.a;
     const PackGeometry &g = s.g;
@@ -958,12 +963,7 @@ void batch_fill_pack_args(void *dst, const EncBatchLayout &L, const BatchPackStr
     a.tile_bits = L.region_bits + s.first_region;
     a.run_bits = L.run_bits + s.first_region * 32;
     a.group_prefix = L.group_prefix;  // indexed by the group's region numbers (batch_region_prefix)
-    a.group_tiles = kPrefixGroup;
-    a.group_shift = 10;
-    a.interior_lo = g.misalign ? 1u : 0u;
-    a.interior_hi = (uint32_t)(g.v_end / kRegionSyms);
-    if (a.interior_hi < a.interior_lo) a.interior_hi = a.interior_lo;
-    a.image_words = 1;  // read by opaque_128 only: batch_pack_runs_kernel takes the group's image size as a parameter
+    set_lane_runs(a, g, max_len);
     b.first_region = s.first_region;
     b.header = L.headers + s.header_off;
     b.header_len = s.header_len;
@@ -985,9 +985,8 @@ cudaError_t launch_pack_batch(const EncBatchLayout &L, uint32_t n_tiles, uint64_
     region_prefix_kernel<<<groups, kPrefixGroup, 0, stream>>>(s);
     group_scan_kernel<<<1, 1024, 0, stream>>>(s, groups);
     // the warps' images are sized by the group's longest code, as launch_pack sizes them by the stream's
-    const uint32_t image_words = (uint32_t)(kStageGuard + (kRegionSyms * max_len + 31) / 32 + 16 + 3) & ~3u;
-    const int smem = kTableBytes + kRunWarps * (int)image_words * 4 + kRunWarps * 32;
-    batch_pack_runs_kernel<<<n_tiles, kRunWarps * 32, smem, stream>>>(args, L.tiles, image_words);
+    const int smem = kTableBytes + kRunWarps * (int)run_image_words(max_len) * 4 + kRunWarps * 32;
+    batch_pack_runs_kernel<<<n_tiles, kRunWarps * 32, smem, stream>>>(args, L.tiles);
     batch_seam_fixup_kernel<<<n_tiles, kBatchSeamThreads, 0, stream>>>(args, L.tiles);
     if (launches) *launches += 5;
     return cudaGetLastError();

@@ -483,9 +483,11 @@ __device__ __forceinline__ void sync_chunk(const DecArgs &a, uint32_t c, uint32_
     a.count[c] = cnt;
 }
 
-__global__ void __launch_bounds__(kChunkThreads, 6) chunk_sync_kernel(const DecArgs a, int round) {
-    __shared__ __align__(16) uint32_t clut_sh[kLutSize];
-    const uint32_t c = blockIdx.x * kChunkThreads + threadIdx.x;
+// A round of the count walks over the block's chunks (c: thread tid's): a chunk's entry, then its walk.  Round 0 walks
+// every chunk from a guess (or from the head, or in closed form); a later round walks only the chunks whose entry moved,
+// and raises *changed.  (The kernels pass threadIdx.x in: read there, it carries their __launch_bounds__.)
+template <bool BATCH = false>
+__device__ __forceinline__ void sync_round(const DecArgs &a, uint32_t c, uint32_t tid, int round, uint32_t *clut_sh, uint32_t *changed) {
     uint32_t start = 0;
     bool work = c < a.n_chunks;
     if (work && round != 0) {
@@ -497,12 +499,13 @@ __global__ void __launch_bounds__(kChunkThreads, 6) chunk_sync_kernel(const DecA
         }
     }
     if (!__syncthreads_or(work)) return;  // later rounds touch only the chunks whose entry moved
-    for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) clut_sh[i] = a.clut[i];
+    for (int i = tid; i < kLutSize; i += kChunkThreads) clut_sh[i] = a.clut[i];
     __syncthreads();
     if (!work) return;
-    if (round != 0) *a.changed = 1u;
-    if (c == 0 && a.head_known) start = a.head_off;
-    bool known = round != 0 || (c == 0 && a.head_known);
+    if (round != 0) *changed = 1u;
+    const bool head_known = a.head_known;  // read before the tests: they then need no branch
+    if (c == 0 && head_known) start = a.head_off;
+    bool known = round != 0 || (c == 0 && head_known);
     if (a.fixed_len && round == 0) {
         // Codes of one length never re-synchronise (a wrong phase stays wrong for ever), but they need not: every
         // boundary is a whole number of codes past the first one.  Without a known head the first entry is a guess
@@ -511,7 +514,12 @@ __global__ void __launch_bounds__(kChunkThreads, 6) chunk_sync_kernel(const DecA
         if (begin > base) start = (uint32_t)((a.fixed_len - (begin - base) % a.fixed_len) % a.fixed_len);
         known = true;
     }
-    sync_chunk(a, c, start, known, clut_sh);
+    sync_chunk<BATCH>(a, c, start, known, clut_sh);
+}
+
+__global__ void __launch_bounds__(kChunkThreads, 6) chunk_sync_kernel(const DecArgs a, int round) {
+    __shared__ __align__(16) uint32_t clut_sh[kLutSize];
+    sync_round(a, blockIdx.x * kChunkThreads + threadIdx.x, threadIdx.x, round, clut_sh, a.changed);
 }
 
 // ------------------------------------------------------------------ transfer functions (slowly synchronising codes)
@@ -640,21 +648,30 @@ __global__ void __launch_bounds__(kSegThreads) compose_apply_kernel(const DecArg
 }
 
 // ------------------------------------------------------------------ scan
-__global__ void __launch_bounds__(kChunkThreads) chunk_sum_kernel(const DecArgs a) {
-    __shared__ uint32_t warp_sum[kChunkThreads / 32];
-    const uint32_t c = blockIdx.x * kChunkThreads + threadIdx.x;
+// The symbols of the block's chunks (c: thread tid's) into block_prefix[slot].  The check of the guessed entries rides
+// along: a chunk that does not start where its left neighbour ended raises both flags (the stream's and the group's; a
+// single stream passes its own twice).
+__device__ __forceinline__ void sum_block(const DecArgs &a, uint32_t c, uint32_t tid, uint32_t slot, uint32_t *stream_changed,
+                                          uint32_t *group_changed, uint32_t *warp_sum) {
     uint32_t v = c < a.n_chunks ? a.count[c] : 0u;
-    // the check of the guessed entries rides along: does every chunk start where its left neighbour ended?
-    if (c > 0 && c < a.n_chunks && a.start_off[c] != a.exit_off[c - 1]) *a.changed = 1u;
+    if (c > 0 && c < a.n_chunks && a.start_off[c] != a.exit_off[c - 1]) {
+        *stream_changed = 1u;
+        *group_changed = 1u;
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = v;
+    if ((tid & 31) == 0) warp_sum[tid >> 5] = v;
     __syncthreads();
-    if (threadIdx.x == 0) {
+    if (tid == 0) {
         unsigned long long s = 0;
         for (int i = 0; i < kChunkThreads / 32; ++i) s += warp_sum[i];
-        a.block_prefix[blockIdx.x] = s;
+        a.block_prefix[slot] = s;
     }
+}
+__global__ void __launch_bounds__(kChunkThreads) chunk_sum_kernel(const DecArgs a) {
+    __shared__ uint32_t warp_sum[kChunkThreads / 32];
+    const uint32_t tid = threadIdx.x;
+    sum_block(a, blockIdx.x * kChunkThreads + tid, tid, blockIdx.x, a.changed, a.changed, warp_sum);
 }
 
 // One block: in-place exclusive scan of `arr` (block sums, or the sums of groups of 1024 regions); total and the
@@ -688,18 +705,9 @@ __global__ void __launch_bounds__(1024) chunk_scan_kernel(const DecArgs a, unsig
 }
 
 // ------------------------------------------------------------------ write
-__global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const DecArgs a) {
-    __shared__ __align__(16) uint32_t wlut_sh[kLutSize];
-    __shared__ __align__(16) uint32_t rings[(kChunkThreads / 32) * 16 * 32];  // per warp: 16 words x 32 lanes
-    __shared__ uint32_t warp_sum[kChunkThreads / 32];
-    for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) wlut_sh[i] = a.wlut[i];
-
-    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t bid = gridDim.x - 1u - blockIdx.x;  // last chunks first: the stream's ragged end (walked with every check) is the slow one
-    const uint32_t c = bid * kChunkThreads + tid;
-    const bool live = c < a.n_chunks;
-    const uint32_t cnt = live ? a.count[c] : 0u;
-    // where this chunk's text goes: block prefix + exclusive scan inside the block
+// Where the text of this thread's chunk (cnt symbols) goes, from the start of its block's text: an exclusive scan inside
+// the block.
+__device__ __forceinline__ unsigned long long text_in_block(uint32_t cnt, uint32_t lane, uint32_t warp, uint32_t *warp_sum) {
     uint32_t incl = cnt;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) {
@@ -710,9 +718,13 @@ __global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const Dec
     __syncthreads();
     uint32_t before = 0;
     for (uint32_t q = 0; q < warp; ++q) before += warp_sum[q];
-    const unsigned long long o = a.block_prefix[bid] + before + (incl - cnt);
-    if (!live || cnt == 0 || o >= a.max_symbols) return;
+    return (unsigned long long)before + (incl - cnt);
+}
 
+// The write walk of chunk c: its cnt symbols to out[o..).  wlut_sh: the block's copy of wlut; rings: the block's rings.
+template <bool BATCH = false>
+__device__ __forceinline__ void write_chunk(const DecArgs &a, uint32_t c, uint32_t cnt, unsigned long long o, uint32_t *wlut_sh,
+                                            uint32_t *rings, uint32_t lane, uint32_t warp) {
     const Chunk k = chunk_of(a, c);
     const uint32_t start = a.start_off[c];
     uint32_t bad = 0;
@@ -727,12 +739,10 @@ __global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const Dec
         const uint32_t head = r.head_skip;
         uint32_t s = start | (head << 9);
         const uint64_t pair0 = k.begin >> 8;
-        const uint32_t n_pairs = a.chunk_bytes >> 5;
         const uint32_t wlut_s = smem_addr(wlut_sh);
         // (no L2 prefetch of the whole chunk here: with the text also streaming out, lines fetched that early are evicted before use)
         uint32_t w[5];
         const uint32_t n_pieces = a.chunk_bytes >> 4;
-        (void)n_pairs;
         Pair raw = load_pair_raw(a, pair0);
         Pair cur = raw;
 #pragma unroll 1
@@ -756,9 +766,26 @@ __global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const Dec
             r.gsector[kk & 31u] = (uint8_t)lds_u8(ring_slot(r, kk >> 2) + (kk & 3u));
     } else {
         uint32_t n = 0;
-        if (k.begin + start < k.end) walk_generic<true>(a, k.begin + start, k.end, a.end_bit, &n, o, &bad, nullptr, wlut_sh);
+        if (k.begin + start < k.end) walk_generic<true, BATCH>(a, k.begin + start, k.end, a.end_bit, &n, o, &bad, nullptr, wlut_sh);
     }
     if (bad) atomicOr(a.error_flags, kErrInvalidCode);
+}
+
+__global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const DecArgs a) {
+    __shared__ __align__(16) uint32_t wlut_sh[kLutSize];
+    __shared__ __align__(16) uint32_t rings[(kChunkThreads / 32) * 16 * 32];  // per warp: 16 words x 32 lanes
+    __shared__ uint32_t warp_sum[kChunkThreads / 32];
+    for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) wlut_sh[i] = a.wlut[i];
+
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t bid = gridDim.x - 1u - blockIdx.x;  // last chunks first: the stream's ragged end (walked with every check) is the slow one
+    const uint32_t c = bid * kChunkThreads + tid;
+    const bool live = c < a.n_chunks;
+    const uint32_t cnt = live ? a.count[c] : 0u;
+    const unsigned long long in_block = text_in_block(cnt, lane, warp, warp_sum);
+    const unsigned long long o = a.block_prefix[bid] + in_block;
+    if (!live || cnt == 0 || o >= a.max_symbols) return;
+    write_chunk(a, c, cnt, o, wlut_sh, rings, lane, warp);
 }
 
 // ------------------------------------------------------------------ first-level tables from the trie, on the device
@@ -839,8 +866,9 @@ __global__ void __launch_bounds__(256) build_sub_tables_kernel(const uint32_t *_
 
 // ------------------------------------------------------------------ batched decode: many streams per launch (et_batch.inc)
 // A CTA decodes one tile: kChunkThreads chunks of one stream (tiles never cross streams).  It copies that stream's DecArgs
-// into shared memory and runs the walks of the per-thread kernels above unchanged, with chunk indices local to the stream,
-// so chunk_of and every edge case (ragged ends, unaligned bodies, fixed_len entries) behave as for a single stream.
+// into shared memory and calls the per-thread kernels' device functions (sync_round, sum_block, text_in_block,
+// write_chunk) with chunk indices local to the stream, so chunk_of and every edge case (ragged ends, unaligned bodies,
+// fixed_len entries) behave as for a single stream.
 __device__ __forceinline__ BatchTile load_tile(DecArgs &dst, const DecArgs *__restrict__ args, const BatchTile *__restrict__ tiles,
                                                uint32_t t) {
     static_assert(sizeof(DecArgs) % 8 == 0, "DecArgs is copied in 8-byte words");
@@ -859,30 +887,8 @@ __global__ void __launch_bounds__(kChunkThreads, 5) batch_sync_kernel(const DecA
                                                                       uint32_t *batch_changed) {
     __shared__ __align__(16) uint32_t clut_sh[kLutSize];
     __shared__ __align__(16) DecArgs a;
-    const uint32_t c = load_tile(a, args, tiles, blockIdx.x).first + threadIdx.x;
-    uint32_t start = 0;
-    bool work = c < a.n_chunks;
-    if (work && round != 0) {
-        if (c == 0) {
-            work = false;
-        } else {
-            start = a.exit_off[c - 1];
-            work = start != a.start_off[c];
-        }
-    }
-    if (!__syncthreads_or(work)) return;  // later rounds touch only the chunks whose entry moved
-    for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) clut_sh[i] = a.clut[i];
-    __syncthreads();
-    if (!work) return;
-    if (round != 0) *batch_changed = 1u;
-    if (c == 0 && a.head_known) start = a.head_off;
-    bool known = round != 0 || (c == 0 && a.head_known);
-    if (a.fixed_len && round == 0) {  // entries in closed form (chunk_sync_kernel)
-        const uint64_t begin = chunk_of(a, c).begin, base = a.grid_bit + (a.head_known ? a.head_off : 0u);
-        if (begin > base) start = (uint32_t)((a.fixed_len - (begin - base) % a.fixed_len) % a.fixed_len);
-        known = true;
-    }
-    sync_chunk<true>(a, c, start, known, clut_sh);
+    const uint32_t tid = threadIdx.x;
+    sync_round<true>(a, load_tile(a, args, tiles, blockIdx.x).first + tid, tid, round, clut_sh, batch_changed);
 }
 
 // chunk_sum_kernel over tiles: the tile's symbols into its slot of the tile sums; a failed check raises the stream's
@@ -891,21 +897,8 @@ __global__ void __launch_bounds__(kChunkThreads) batch_sum_kernel(const DecArgs 
     __shared__ __align__(16) DecArgs a;
     __shared__ uint32_t warp_sum[kChunkThreads / 32];
     const BatchTile tile = load_tile(a, args, tiles, blockIdx.x);
-    const uint32_t c = tile.first + threadIdx.x;
-    uint32_t v = c < a.n_chunks ? a.count[c] : 0u;
-    if (c > 0 && c < a.n_chunks && a.start_off[c] != a.exit_off[c - 1]) {
-        *a.changed = 1u;
-        *batch_changed = 1u;
-    }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if ((threadIdx.x & 31) == 0) warp_sum[threadIdx.x >> 5] = v;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        unsigned long long s = 0;
-        for (int i = 0; i < kChunkThreads / 32; ++i) s += warp_sum[i];
-        a.block_prefix[tile.first / kChunkThreads] = s;
-    }
+    const uint32_t tid = threadIdx.x;
+    sum_block(a, tile.first + tid, tid, tile.first / kChunkThreads, a.changed, batch_changed, warp_sum);
 }
 
 // chunk_write_kernel over tiles.  The tile sums of the whole group were scanned together: a stream's text starts at its
@@ -926,61 +919,10 @@ __global__ void __launch_bounds__(kChunkThreads, 4) batch_write_kernel(const Dec
     const uint32_t c = tile.first + tid;
     const bool live = c < a.n_chunks;
     const uint32_t cnt = live ? a.count[c] : 0u;
-    uint32_t incl = cnt;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint32_t up = __shfl_up_sync(0xffffffffu, incl, d);
-        if (lane >= (uint32_t)d) incl += up;
-    }
-    if (lane == 31) warp_sum[warp] = incl;
-    __syncthreads();
-    uint32_t before = 0;
-    for (uint32_t q = 0; q < warp; ++q) before += warp_sum[q];
-    const unsigned long long o = a.block_prefix[bid] - base + before + (incl - cnt);
+    const unsigned long long in_block = text_in_block(cnt, lane, warp, warp_sum);
+    const unsigned long long o = a.block_prefix[bid] - base + in_block;
     if (!live || cnt == 0 || o >= a.max_symbols) return;
-
-    const Chunk k = chunk_of(a, c);
-    const uint32_t start = a.start_off[c];
-    uint32_t bad = 0;
-    if ((k.interior || (k.walkable && start < 256u)) && o + cnt <= a.max_symbols) {
-        uint8_t *dst = a.out + o;
-        OutRing r;
-        r.ring_s = smem_addr(rings) + warp * 2048u + lane * 4u;
-        r.head_skip = (uint32_t)(reinterpret_cast<uintptr_t>(dst) & 31u);
-        r.gsector = dst - r.head_skip;
-        r.lo = r.hi = 0;
-        r.stored = 0;
-        const uint32_t head = r.head_skip;
-        uint32_t s = start | (head << 9);
-        const uint64_t pair0 = k.begin >> 8;
-        const uint32_t wlut_s = smem_addr(wlut_sh);
-        uint32_t w[5];
-        const uint32_t n_pieces = a.chunk_bytes >> 4;
-        Pair raw = load_pair_raw(a, pair0);
-        Pair cur = raw;
-#pragma unroll 1
-        for (uint32_t p = 0; p < n_pieces; ++p) {
-            if (!(p & 1u)) {
-                cur = swap_pair(raw);
-                if (p + 2 < n_pieces)
-                    raw = load_pair_raw(a, pair0 + (p >> 1) + 1);
-                else
-                    raw.a = __ldg(reinterpret_cast<const uint4 *>(a.body_aligned) + 2 * (pair0 + (p >> 1) + 1));
-                w[0] = cur.a.x; w[1] = cur.a.y; w[2] = cur.a.z; w[3] = cur.a.w; w[4] = cur.b.x;
-            } else {
-                w[0] = cur.b.x; w[1] = cur.b.y; w[2] = cur.b.z; w[3] = cur.b.w; w[4] = bswap32(raw.a.x);
-            }
-            s = write_piece(w, s, p + 1 == n_pieces, wlut_s, r, a.clut, a.wlut, a.nodes, &bad);
-        }
-        const uint32_t n_end = s >> 9;
-        if (n_end & 3u) sts_u32(ring_slot(r, n_end >> 2), r.hi >> (8u * (4u - (n_end & 3u))));
-        for (uint32_t kk = r.head_skip ? head : (n_end & ~31u); kk < n_end; ++kk)
-            r.gsector[kk & 31u] = (uint8_t)lds_u8(ring_slot(r, kk >> 2) + (kk & 3u));
-    } else {
-        uint32_t n = 0;
-        if (k.begin + start < k.end) walk_generic<true, true>(a, k.begin + start, k.end, a.end_bit, &n, o, &bad, nullptr, wlut_sh);
-    }
-    if (bad) atomicOr(a.error_flags, kErrInvalidCode);
+    write_chunk<true>(a, c, cnt, o, wlut_sh, rings, lane, warp);
 }
 
 // The tables of every stream of the group: blockIdx.y selects the stream.
