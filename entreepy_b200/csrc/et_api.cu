@@ -592,13 +592,13 @@ int check_stream(et_ctx *ctx, const et_dictionary &dict, size_t n, uint32_t flag
     return ET_OK;
 }
 
-// et_decode_dev's result for a stream in which the decoder found `total` symbols: *out_len, or NoSpaceLeft when the text
-// did not fit `cap`.
+// et_decode_dev's result for a stream in which the decoder found `total` symbols (not clipped to `cap`): *out_len, or
+// NoSpaceLeft when the text, min(total, body_len) symbols, does not fit `cap`.  A text of exactly `cap` symbols fits,
+// whatever body_len claims: the reference's writer only fails on a byte it cannot store.
 int decode_result(et_ctx *ctx, const et_dictionary &dict, size_t cap, uint64_t total, size_t *out_len) {
-    const uint64_t want = std::min<uint64_t>(dict.body_len, cap);
-    const uint64_t produced = std::min<uint64_t>(total, want);
-    if (produced == cap && dict.body_len > cap) return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %u symbols, capacity %zu", dict.body_len, cap);
-    *out_len = (size_t)produced;
+    const uint64_t text = std::min<uint64_t>(total, dict.body_len);
+    if (text > cap) return fail(ctx, ET_ERR_NO_SPACE, "NoSpaceLeft: %llu symbols, capacity %zu", (unsigned long long)text, cap);
+    *out_len = (size_t)text;
     return ET_OK;
 }
 
@@ -678,11 +678,11 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
             rc = unpack_dev(ctx, unpack_geometry(ctx->d_in, body_bytes), dict, ctx->d_out, want, s, &st, nullptr, false, validate);
             if (rc != ET_OK) return rc;
             produced = std::min<uint64_t>(st.total, want);
-            if (write_out) {
-                size_t fits = 0;  // *out_len is set once the text is home
-                if ((rc = decode_result(ctx, dict, cap, produced, &fits)) != ET_OK) return rc;
+            if (write_out) {  // the first cap bytes go home even when the text does not fit, as from et_decode_dev
                 if (produced) ET_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_out, produced, cudaMemcpyDeviceToHost, s));
                 ET_CUDA(ctx, cudaStreamSynchronize(s));
+                size_t fits = 0;  // *out_len is set below
+                if ((rc = decode_result(ctx, dict, cap, st.total, &fits)) != ET_OK) return rc;
             }
         } else {
             rc = upload_unpack_tables(ctx, dict, s, validate);  // before the bulk uploads: copies in one direction run in issue order
@@ -704,7 +704,10 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
                 }
             }
             uint64_t head_bit = 0;  // first codeword of the next slice, bits from the start of the body
-            for (size_t k = 0; k < n_slices && produced < want; ++k) {
+            // symbols found so far; decoding stops at body_len, or once one symbol more than fits `cap` has been found
+            uint64_t found = 0;
+            const uint64_t enough = write_out ? std::min<uint64_t>(dict.body_len, (uint64_t)cap + 1) : dict.body_len;
+            for (size_t k = 0; k < n_slices && found < enough; ++k) {
                 const bool last = k + 1 == n_slices;
                 // slice k owns body bytes [k*kSlice - 64, (k+1)*kSlice - 64): what it needs to look ahead is uploaded
                 const size_t own_lo = k ? k * kSlice - 64 : 0, own_hi = last ? body_bytes : (k + 1) * kSlice - 64;
@@ -723,13 +726,14 @@ extern "C" int et_decode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out,
                 if (write_out && got)  // unpack_dev returned after its kernels finished: the text is ready to go down
                     cudaMemcpyAsync(out + produced, ctx->d_out + produced, got, cudaMemcpyDeviceToHost, ctx->copy_stream2);
                 produced += got;
+                found += st.total;
             }
             cudaStreamSynchronize(ctx->copy_stream);
             const cudaError_t e = cudaStreamSynchronize(ctx->copy_stream2);
             cleanup();
             if (e != cudaSuccess) return fail(ctx, ET_ERR_CUDA, "download: %s", cudaGetErrorString(e));
             size_t fits = 0;
-            if (write_out && (rc = decode_result(ctx, dict, cap, produced, &fits)) != ET_OK) return rc;
+            if (write_out && (rc = decode_result(ctx, dict, cap, found, &fits)) != ET_OK) return rc;
         }
         if (print_out && produced) {  // decode.zig:189 prints every symbol to std_out
             std::vector<uint8_t> text(produced);

@@ -771,10 +771,13 @@ __device__ __forceinline__ void write_chunk(const DecArgs &a, uint32_t c, uint32
     if (bad) atomicOr(a.error_flags, kErrInvalidCode);
 }
 
+// Writes nothing when the entry check of the sums failed: the walk would start from wrong entries, and its text could reach
+// past the true end of the text (up to max_symbols) where the walk after the rounds would not overwrite it.
 __global__ void __launch_bounds__(kChunkThreads, 5) chunk_write_kernel(const DecArgs a) {
     __shared__ __align__(16) uint32_t wlut_sh[kLutSize];
     __shared__ __align__(16) uint32_t rings[(kChunkThreads / 32) * 16 * 32];  // per warp: 16 words x 32 lanes
     __shared__ uint32_t warp_sum[kChunkThreads / 32];
+    if (*a.changed) return;
     for (int i = threadIdx.x; i < kLutSize; i += kChunkThreads) wlut_sh[i] = a.wlut[i];
 
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -916,6 +919,7 @@ __global__ void __launch_bounds__(kChunkThreads, 4) batch_write_kernel(const Dec
     const uint32_t bid = tile.first / kChunkThreads;
     const unsigned long long base = a.block_prefix[0];
     if (bid == 0 && tid == 0) *a.total = a.block_prefix[(a.n_chunks + kChunkThreads - 1) / kChunkThreads] - base;
+    if (*a.changed) return;  // the stream's entries are wrong: as chunk_write_kernel
     const uint32_t c = tile.first + tid;
     const bool live = c < a.n_chunks;
     const uint32_t cnt = live ? a.count[c] : 0u;

@@ -151,7 +151,9 @@ ET_API int et_histogram_dev(et_ctx *ctx, const void *d_in, size_t n, uint64_t co
  * (encode.zig:319,336). */
 ET_API int et_encode(et_ctx *ctx, const uint8_t *in, size_t n, uint8_t *out, size_t cap, size_t *out_len, uint32_t flags);
 /* decode.zig:13.  `in` is file[4..] exactly as main.zig:204 / test.zig:26 pass it.
- * *out_len = bytes written (0 on a dry run, decode.zig:187,219). */
+ * *out_len = bytes written (0 on a dry run, decode.zig:187,219).  The text is min(body_len, symbols the body holds)
+ * symbols; when that is more than `cap`, the decoders (this one, et_decode_dev and the batch) return ET_ERR_NO_SPACE
+ * with *out_len = 0 and the first `cap` bytes of the text written to out. */
 ET_API int et_decode(et_ctx *ctx, const uint8_t *in_after_magic, size_t n, uint8_t *out, size_t cap, size_t *out_len,
               uint32_t flags);
 /* Same, input and output resident in device memory (no PCIe bulk copies). */
